@@ -5,6 +5,7 @@ Metric (BASELINE.json): vehicle crops/s through warp + VUNet at N GPUs, plus the
 the dominant kernel, next to the reference algorithm's CPU path timed on this box's host cores.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (one rank per GPU under torchrun)
+  python bench.py ... --dump-outputs DIR                         also write the last timed step's outputs to DIR/*.npy
   python bench.py --impl reference ...                           CPU arm: the oracle port of the reference path
 
 One "step" = one pass of the hot path over one batch of synthetic crops (BASELINE config 2: 64 crops
@@ -343,7 +344,7 @@ def run_ours(args):
         # several streams are in flight: bracket with device events and cross-check with the host clock
         ms = reduce_max(max(e0.elapsed_time(e1), wall if (n * M >= 20 or not resident) else 0.0))
         barrier()
-        return ms
+        return ms, last_t
 
     # ---- device-resident loop: inputs and noise already in HBM, graph replays only ----------------
     # The public batched API: NovelViewPipeline (CUDA-graph replay of the launches of a micro-batch, two in flight).
@@ -355,8 +356,10 @@ def run_ours(args):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(pipe, args.steps, True, host_u8, pipe.slots[pipe.n % pipe.depth].stream, lambda t: pipe.slots[t % pipe.depth].stream)
+    ms_total, last_ticket = timed(pipe, args.steps, True, host_u8, pipe.slots[pipe.n % pipe.depth].stream, lambda t: pipe.slots[t % pipe.depth].stream)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pipe, last_ticket, min(M, pipe.depth))
     launches = launches_per_mb * M * args.steps
     ms_per_step = ms_total / args.steps
     value = world * CPR / (ms_per_step * 1e-3)
@@ -366,13 +369,13 @@ def run_ours(args):
     # noise on the CPU generator (reference semantics), and lands its completed crops + flags in host memory, inside
     # the timed region.  One compute stream shared by the slots: with host copies in the loop, graphs that overlap only
     # partially slow each other down (measured 11.8 vs 14.2 ms/step, scripts/e2e_probe.py).
-    e2e_steps = max(4, args.steps)
+    e2e_steps = args.steps
 
     def e2e_run(host, **kw):
         pp = NovelViewPipeline(model, depth=3, shared_stream=True, gather_fn=gather, micro_batches_per_step=M, **kw)
         lt = run_steps(pp, max(2, (5 + M - 1) // M), resident=False, host=host)
         d2h = M * pp.d2h_bytes(lt)
-        ms = timed(pp, e2e_steps, False, host, pp.copy_stream, lambda t: pp.out_stream)
+        ms, _ = timed(pp, e2e_steps, False, host, pp.copy_stream, lambda t: pp.out_stream)
         return world * CPR / (ms / e2e_steps * 1e-3), ms / e2e_steps, d2h
     e2e_value, e2e_ms_step, d2h_bytes = e2e_run(host_u8)
     extra = {}
@@ -541,6 +544,34 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, pipe, last_ticket, n_tickets):
+    """Writes what the timed loop computed in its last step -- the device outputs of its last `n_tickets` submits (all a
+    pipeline of that depth still holds), crop axis first, concatenated in submit order -- as <out_dir>/<name>.npy, float32
+    (float64 where float32 would not be exact).  Together they stay under DUMP_BYTES: smallest first, an array larger than
+    an equal share of what is left keeps only a sample of its crops, the first k of a permutation seeded with 0, in crop
+    order -- the same crops on every run, so two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    outs = [pipe.device_outputs(t) for t in range(last_ticket - n_tickets + 1, last_ticket + 1)]
+    arrays = {}
+    for k, v in outs[-1].items():
+        v = v if k == "crops_all" else torch.cat([o[k] for o in outs])      # crops_all: the whole step, all ranks
+        wide = v.dtype in (torch.float64, torch.int32, torch.int64)
+        arrays[k] = v.to(torch.float64 if wide else torch.float32).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES - 4096 * len(arrays)                                    # room for the .npy headers
+    for i, (k, a) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].nbytes)):
+        share = left // (len(arrays) - i)
+        if a.nbytes > share:
+            keep = max(1, share // (a.nbytes // a.shape[0]))
+            a = a[np.sort(np.random.default_rng(0).permutation(a.shape[0])[:keep])]
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+        left -= a.nbytes
+
+
 def icn_info(torch, synth, B, dev):
     """Informational, outside every timed region of the headline metric: the ICN generator G_Resnet (SURVEY.md 8f-1, the consumer of
     the warped planes in the reference's data flow) on the same batch size -- crops/s and FLOP-weighted tensor throughput."""
@@ -578,7 +609,13 @@ def main():
     ap.add_argument("--headline-only", action="store_true", help="skip the informational extra keys (e2e_fp32, ICN)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-icn", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl ours)")
     # stdout carries exactly one JSON line: libraries that write to fd 1 on their own (NCCL prints its version there
     # whatever NCCL_DEBUG_FILE says) are pointed at stderr for the whole run, and print() gets the real stdout back
     sys.stdout.flush()

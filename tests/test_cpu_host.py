@@ -11,6 +11,8 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# a checkout of the original Python project (alexj94/future_urban_scene_generation), if one is at hand
+REFERENCE = os.environ.get("FUSG_REFERENCE_DIR", "")
 
 
 def test_library_exports_every_declared_symbol():
@@ -212,7 +214,7 @@ def test_import_shim_serves_reference_import_sites():
     import subprocess
     import sys
     shim = os.path.join(ROOT, "future_urban_scene_generation_b200", "shim")
-    ref = "/root/reference"
+    ref = REFERENCE
     code = (
         "import sys, warnings; warnings.filterwarnings('ignore');"
         f"sys.path[:0] = [{ROOT!r}, {shim!r}];"
@@ -227,7 +229,7 @@ def test_import_shim_serves_reference_import_sites():
         + "from warp_learn.models import get_icn_inputs;"
         "assert get_icn_inputs.__module__.startswith('future_urban_scene_generation_b200');"
         + ("from warp_learn.models import get_icn_inputs_reference, G_Resnet_reference, GANLoss; import warp_learn.models as wm;"
-           "assert get_icn_inputs_reference.__code__.co_filename.startswith('/root/reference');"
+           f"assert get_icn_inputs_reference.__code__.co_filename.startswith({ref!r});"
            "assert wm.planes_to_torch.__module__.startswith('future_urban_scene_generation_b200');" if os.path.isdir(ref) else "")
         + "print('ok')")
     env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
@@ -236,17 +238,16 @@ def test_import_shim_serves_reference_import_sites():
 
 
 def test_reference_orchestrator_imports_through_the_shim():
-    """The reference's own orchestrator module (`trajectory_inference.py`, unedited, build container only) imports with the
-    shim first on sys.path: every hot-path name it binds -- get_icn_inputs, pascal_texture_planes, to_image,
-    warp_unwarp_planes, and through the reference's own vehicle_utils: compute_visibility, get_planes, get_rendered (the
-    Open3D window) -- resolves to the B200 modules.  open3d / matplotlib / skimage are not installed: they are stubbed.
-    (Running traj_test itself needs a GPU AND the reference tree on one machine, which this environment never has: the
-    tree stays in the build container, the GPU box only receives this repository.)"""
+    """The reference's own orchestrator module (`trajectory_inference.py`, unedited, from the checkout FUSG_REFERENCE_DIR
+    names; skipped without one) imports with the shim first on sys.path: every hot-path name it binds -- get_icn_inputs,
+    pascal_texture_planes, to_image, warp_unwarp_planes, and through the reference's own vehicle_utils:
+    compute_visibility, get_planes, get_rendered (the Open3D window) -- resolves to the B200 modules.  open3d /
+    matplotlib / skimage are stubbed.  (Running traj_test itself needs a GPU as well as the checkout.)"""
     import subprocess
     import sys
-    ref = "/root/reference"
+    ref = REFERENCE
     if not os.path.isdir(ref):
-        pytest.skip("reference checkout not present (GPU box)")
+        pytest.skip("needs a checkout of the original project: set FUSG_REFERENCE_DIR")
     shim = os.path.join(ROOT, "future_urban_scene_generation_b200", "shim")
     code = r"""
 import sys, types, warnings
