@@ -26,7 +26,6 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
-#include <cstdlib>
 #include "../../include/fusg.h"
 #include "fusg_common.h"
 
@@ -529,12 +528,10 @@ __device__ __forceinline__ void unpair_chunk(float *out, const float *s_bias, in
 // ------------------------------------------------------------------------------------------------
 // k_conv_tc
 // ------------------------------------------------------------------------------------------------
-#ifndef FUSG_TC_EPI_WARPS
-#define FUSG_TC_EPI_WARPS 8
-#endif
-constexpr int TC_EPI_WARPS = FUSG_TC_EPI_WARPS;          // 8 or 16: warps 2.. ; warp 0 TMA, warp 1 MMA
+constexpr int TC_EPI_WARPS = 8;                         // warps 2..9; warp 0 TMA, warp 1 MMA
 constexpr int TC_THREADS = 64 + 32 * TC_EPI_WARPS;
-constexpr int TC_STAGE_BYTES = 32768 / TC_EPI_WARPS;     // per-warp staging block of the staged epilogue
+constexpr int TC_STAGING_BYTES = 32768;                  // shared memory of the staged epilogue
+constexpr int TC_STAGE_BYTES = TC_STAGING_BYTES / TC_EPI_WARPS;     // per-warp staging block
 constexpr int TC_BLOCK_M = 128;
 constexpr int TC_HALO_ROWS_MAX = TC_BLOCK_M + 6;                   // pixels of one halo A buffer: 128 + ksize - 1, ksize <= 7
 constexpr int TC_HALO_BYTES = ((TC_HALO_ROWS_MAX * 128 + 1023) / 1024) * 1024;   // 128-byte rows (kc = 64), 1024-aligned
@@ -563,7 +560,8 @@ struct alignas(64) ConvTcParams {
     int hks;                        // halo mode: kernel size (3; 5 or 7 for the bordered ICN layers) -- hks horizontal taps per loaded row segment
     uint32_t halo_skip;             // halo mode: bit (ky * chunks + chunk) set = all three taps of that stage have zero weights -> skipped
     int pair;                       // halo mode on CTA pairs (cta_group::2): M = 256 per MMA, each CTA holds half of the weight rows
-    int pdl;                        // launched with programmatic stream serialization (griddepcontrol in the kernel)
+    int epi_smem;                   // bytes past the bias: the staged epilogue's staging blocks (reserved whenever the plan wanted
+                                    // it, even if the lean epilogue was then refused) or the split-K receive buffer
     unsigned long long w_prefetch_bytes;   // > 0: bytes of the weight matrix the grid pulls into L2 before the dependency wait
     int ksplit;                     // > 1: thread-block cluster of `ksplit` CTAs per tile, each reducing 1/ksplit of K (few-tile layers)
     int kb_local;                   // k-blocks per CTA = num_kblocks / ksplit
@@ -572,6 +570,22 @@ struct alignas(64) ConvTcParams {
     FastEpi fe;
 };
 
+// Shared-memory layout of k_conv_tc, in bytes from the kernel's 1024-aligned base: barriers (first KB) | A pipeline |
+// B region | bias | staging / split-K receive buffer.  `total` is the launch's dynamic shared-memory size, alignment
+// slack included.
+struct TcSmem { size_t b, bias, stage, total; };
+__host__ __device__ __forceinline__ TcSmem tc_smem(const ConvTcParams &p) {
+    const size_t pipe_a = p.halo ? (size_t)p.stages * 2 * TC_HALO_BYTES : (size_t)p.stages * p.group * p.a_bytes;
+    // B k-blocks: [stages][hks] in halo mode, [stages][group] streamed, or [num_kblocks] resident
+    const size_t pipe_b = p.w_resident ? (size_t)p.num_kblocks * p.b_bytes
+                                       : (p.halo ? (size_t)p.stages * p.hks * p.b_bytes : (size_t)p.stages * p.group * p.b_bytes);
+    TcSmem s;
+    s.b = 1024 + pipe_a;
+    s.bias = s.b + ((pipe_b + 15) & ~(size_t)15);              // cout_pad floats, 16-byte aligned (float4 reads)
+    s.stage = s.bias + (size_t)p.d.cout_pad * 4;
+    s.total = 1024 /*alignment slack*/ + s.b + pipe_b + 16 /*bias alignment*/ + (size_t)p.d.cout_pad * 4 + (size_t)p.epi_smem;
+    return s;
+}
 
 // MMA-issuer role of k_conv_tc.  Everything the loop needs is hoisted into registers and the
 // (sub-tile, k-step) MMAs of a k-block are fully unrolled: the single issuing thread must stay well
@@ -717,18 +731,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_conv_tc(const __grid_constant
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     // 1024-byte aligned base (swizzle atoms)
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    // barriers (first KB: mbar_wait finds the CTA's wait-failure counter from a barrier's address, so the block must sit on a
-    // 1024-byte boundary) | [stages][group] A k-blocks | B k-blocks ([stages][group] streamed, or [num_kblocks] resident) | bias
+    // barriers first: mbar_wait finds the CTA's wait-failure counter from a barrier's address, so the block must sit on a
+    // 1024-byte boundary (tc_smem)
+    const TcSmem lay = tc_smem(p);
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem);
     uint8_t *sA = smem + 1024;
-    uint8_t *sB = sA + (p.halo ? (size_t)p.stages * 2 * TC_HALO_BYTES : (size_t)p.stages * p.group * p.a_bytes);
-    const size_t b_region = p.w_resident ? (size_t)p.num_kblocks * p.b_bytes
-                                         : (p.halo ? (size_t)p.stages * p.hks * p.b_bytes : (size_t)p.stages * p.group * p.b_bytes);
+    uint8_t *sB = smem + lay.b;
     uint64_t *full_bar = bars, *empty_bar = bars + TC_MAX_STAGES, *tfull_bar = bars + 2 * TC_MAX_STAGES, *tempty_bar = tfull_bar + 2;
     uint64_t *w_bar = tempty_bar + 2;
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(w_bar + 1);
-    float *s_bias = reinterpret_cast<float *>(sB + ((b_region + 15) & ~(size_t)15));        // cout_pad floats, 16-byte aligned (float4 reads)
-    uint8_t *s_stage = reinterpret_cast<uint8_t *>(s_bias + p.d.cout_pad);   // fast_epi == 2: 32 KB of per-warp staging blocks
+    float *s_bias = reinterpret_cast<float *>(smem + lay.bias);
+    // lay.stage, fast_epi == 2: 32 KB of per-warp staging blocks.  Taken from s_bias because the same address written as
+    // smem + lay.stage makes k_conv_tc<true> spill registers
+    uint8_t *s_stage = reinterpret_cast<uint8_t *>(s_bias + p.d.cout_pad);
     float *s_recv = reinterpret_cast<float *>(s_stage);                      // ksplit > 1: block_n x 128 fp32 receive buffer (no staging then)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -755,23 +770,21 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_conv_tc(const __grid_constant
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     // programmatic dependent launch: everything above (barriers, TMEM, tensor-map prefetch, bias) touched nothing the
-    // previous kernel of the stream produces; wait for it here, then let the next kernel start its own prologue
-    if (p.pdl) {
-        // few-CTA layers (the coarse scales and the auto-regressive tail) are bound by how fast a handful of SMs can pull their
-        // weight slabs (K up to 4608) from HBM: the weights do not depend on the previous kernel, so the grid pulls the whole
-        // matrix into L2 NOW, underneath that kernel's tail -- each CTA an equal share, as bulk prefetches
-        if (p.w_prefetch_bytes && threadIdx.x == 32) {
-            const unsigned long long total = p.w_prefetch_bytes, per = ((total / gridDim.x) + 15ull) & ~15ull;
-            unsigned long long lo = per * blockIdx.x, hi = lo + per < total ? lo + per : total;
-            const char *wb = reinterpret_cast<const char *>(d.weight);
-            for (; lo < hi; lo += 32768ull) {
-                const unsigned n = (unsigned)(hi - lo < 32768ull ? hi - lo : 32768ull) & ~15u;
-                if (n) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(wb + lo), "r"(n) : "memory");
-            }
+    // previous kernel of the stream produces; wait for it here, then let the next kernel start its own prologue.
+    // Few-CTA layers (the coarse scales and the auto-regressive tail) are bound by how fast a handful of SMs can pull their
+    // weight slabs (K up to 4608) from HBM: the weights do not depend on the previous kernel, so the grid pulls the whole
+    // matrix into L2 NOW, underneath that kernel's tail -- each CTA an equal share, as bulk prefetches
+    if (p.w_prefetch_bytes && threadIdx.x == 32) {
+        const unsigned long long total = p.w_prefetch_bytes, per = ((total / gridDim.x) + 15ull) & ~15ull;
+        unsigned long long lo = per * blockIdx.x, hi = lo + per < total ? lo + per : total;
+        const char *wb = reinterpret_cast<const char *>(d.weight);
+        for (; lo < hi; lo += 32768ull) {
+            const unsigned n = (unsigned)(hi - lo < 32768ull ? hi - lo : 32768ull) & ~15u;
+            if (n) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(wb + lo), "r"(n) : "memory");
         }
-        asm volatile("griddepcontrol.wait;" ::: "memory");
-        asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     }
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     // split-K: every CTA of the cluster must be running before a peer writes into its shared memory; arrive now,
     // wait just before the first remote store
     if (p.ksplit > 1) asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory");
@@ -900,7 +913,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_conv_tc(const __grid_constant
         int nparts = TC_EPI_WARPS / 4;
         while (nparts > 1 && p.block_n % (16 * nparts)) nparts >>= 1;
         // narrow layers (one 16-column chunk): the two warps of a lane quadrant split the two sub-tiles instead of the columns
-        const bool sub_split = TC_EPI_WARPS == 8 && nparts == 1 && p.msub == 2 && p.ksplit == 1;
+        const bool sub_split = nparts == 1 && p.msub == 2 && p.ksplit == 1;
         const int ncols = sub_split ? p.block_n : (part < nparts ? p.block_n / nparts : 0);
         const int c_begin = sub_split ? 0 : part * ncols;
         int acc = 0;
@@ -1321,7 +1334,7 @@ static bool tc_supported(const fusg_conv_desc &d, int Ho, int Wo) {
 }
 
 // SMs the persistent conv grids leave free for kernels of other streams (fusg_conv2d_set_sm_reserve)
-static int g_sm_reserve = getenv("FUSG_SM_RESERVE") ? atoi(getenv("FUSG_SM_RESERVE")) : 0;
+static int g_sm_reserve = 0;
 
 extern "C" int fusg_conv2d_set_sm_reserve(int n) {
     const int prev = g_sm_reserve;
@@ -1336,25 +1349,25 @@ extern "C" void fusg_conv2d_last_plan(int32_t *plan8) {
     for (int i = 0; i < 8; ++i) plan8[i] = g_last_plan[i];
 }
 
-static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
-    ConvTcParams p;
+// Tiling policy of k_conv_tc: fills every field of p except the three tensor maps, the grid size and the dynamic
+// shared-memory size.  Reads nothing but its arguments and g_sm_reserve.
+static int plan_tc(const fusg_conv_desc &d, int Ho, int Wo, int num_sms, ConvTcParams &p, int &grid, size_t &smem) {
     memset(&p, 0, sizeof(p));
     p.d = d;
     p.Ho = Ho; p.Wo = Wo;
     p.block_n = d.cout_pad < 128 ? d.cout_pad : 128;
     p.n_tiles = d.cout_pad / p.block_n;
-    const int num_sms = fusg_num_sms();
     // 256-row CTA tiles (two 128-row MMA sub-tiles sharing each weight k-block) once there is enough work for
     // at least ~4 tiles per SM; halves the weight traffic per output pixel
-    static const int msub_max = getenv("FUSG_MSUB1") ? 1 : 2;
     const long long rows = (long long)d.B * Ho * Wo;
     // (1x1 layers too: half as many barrier round trips per output row -- 0.51 -> 0.46 ms on the 6->128 NiN)
-    p.msub = (msub_max == 2 && rows / 256 * p.n_tiles >= 4LL * num_sms && rows % 256 == 0) ? 2 : 1;
+    p.msub = (rows / 256 * p.n_tiles >= 4LL * num_sms && rows % 256 == 0) ? 2 : 1;
     const int trows = TC_BLOCK_M * p.msub;
     p.Wt = Wo < 128 ? Wo : 128;
     p.Ht = (trows / p.Wt) < Ho ? (trows / p.Wt) : Ho;
     p.Bt = trows / (p.Wt * p.Ht);
     p.tiles_x = Wo / p.Wt; p.tiles_y = Ho / p.Ht; p.tiles_b = (d.B + p.Bt - 1) / p.Bt;
+    const int total_tiles = p.tiles_x * p.tiles_y * p.tiles_b * p.n_tiles;
     auto ilog2 = [](int v) { int sh = 0; while ((1 << sh) < v) ++sh; return sh; };
     p.wt_shift = ilog2(p.Wt); p.ht_shift = ilog2(p.Ht); p.txs = ilog2(p.tiles_x); p.tys = ilog2(p.tiles_y);
     const bool k64 = (d.c0 % 64 == 0) && (!d.in1 || d.c1 % 64 == 0);
@@ -1368,29 +1381,22 @@ static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
     // B k-blocks must start 1024-aligned too (swizzle atom): round the size up
     p.b_bytes = (p.b_bytes + 1023) & ~1023;
     // few-tile layers (the coarse scales and the auto-regressive tail): a cluster of `ksplit` CTAs per tile, each
-    // streaming 1/ksplit of the K range, then a DSMEM reduce-scatter -- a single SM pulls ~50-80 GB/s through TMA,
-    // so a 128 x 4608 weight slab per CTA costs ~45 us however few tiles there are
-    static const int ksplit_max = getenv("FUSG_KSPLIT_MAX") ? atoi(getenv("FUSG_KSPLIT_MAX")) : 8;
-    static const int ksplit_min_kb = getenv("FUSG_KSPLIT_MIN_KB") ? atoi(getenv("FUSG_KSPLIT_MIN_KB")) : 36;
+    // streaming 1/ksplit of the K range (at least 36 k-blocks in all), then a DSMEM reduce-scatter -- a single SM pulls
+    // ~50-80 GB/s through TMA, so a 128 x 4608 weight slab per CTA costs ~45 us however few tiles there are
     p.ksplit = 1;
-    {
-        const int tiles = p.tiles_x * p.tiles_y * p.tiles_b * p.n_tiles;
-        if (p.msub == 1 && p.block_n % 16 == 0) {
-            for (int sk = 8; sk >= 2; sk >>= 1) {
-                if (sk > ksplit_max || tiles * sk > 128) continue;
-                if (p.num_kblocks % sk || p.num_kblocks < ksplit_min_kb) continue;
-                if ((p.block_n / 16) % sk) continue;
-                p.ksplit = sk;
-                break;
-            }
+    if (p.msub == 1 && p.block_n % 16 == 0) {
+        for (int sk = 8; sk >= 2; sk >>= 1) {
+            if (total_tiles * sk > 128) continue;
+            if (p.num_kblocks % sk || p.num_kblocks < 36) continue;
+            if ((p.block_n / 16) % sk) continue;
+            p.ksplit = sk;
+            break;
         }
     }
     p.kb_local = p.num_kblocks / p.ksplit;
     // warp-staged epilogue for the big layers (needs 32 KB): applies to the lean-epilogue case with Wt >= 32
-    static const int staged_on = getenv("FUSG_EPI_DIRECT") ? 0 : 1;
     // (1x1 layers too: their direct epilogue touches 32 lines per store instruction -- 64 % LSU wavefronts, 236 -> 169 us on the 32->32 skip NiN at 256^2)
-    static const int staged_1x1 = getenv("FUSG_STAGED_1X1") ? atoi(getenv("FUSG_STAGED_1X1")) : 1;
-    bool want_staged = p.ksplit == 1 && staged_on && (d.ksize >= 3 || p.block_n == 128 || staged_1x1) && p.Wt >= 32 && p.block_n >= 32 && is_pow2(p.block_n) && d.noise == nullptr && d.cout % 16 == 0;
+    bool want_staged = p.ksplit == 1 && p.Wt >= 32 && p.block_n >= 32 && is_pow2(p.block_n) && d.noise == nullptr && d.cout % 16 == 0;
     const int smem_budget = (want_staged ? 168 : 200) * 1024 - (p.ksplit > 1 ? p.block_n * TC_BLOCK_M * 4 : 0);
     // weights resident when the whole (single) N tile fits next to a useful pipeline
     p.w_resident = (p.ksplit == 1 && p.n_tiles == 1 && p.num_kblocks * p.b_bytes <= 72 * 1024) ? 1 : 0;
@@ -1410,30 +1416,22 @@ static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
     if (stages < 2) stages = 2;
     p.stages = stages;
     // sliding-window (halo) A tiles for the wide-frame 3x3 layers: one row-segment load serves the three horizontal taps
-    static const int halo_on = getenv("FUSG_NO_HALO") ? 0 : 1;
-    static const int halo_nmax = getenv("FUSG_HALO_NMAX") ? atoi(getenv("FUSG_HALO_NMAX")) : 128;
-    p.halo = 0;
     p.hks = d.ksize;
     const bool halo_ks = d.pad_mode ? (d.ksize == 3 || d.ksize == 5 || d.ksize == 7) : d.ksize == 3;
-    if (halo_on && p.ksplit == 1 && halo_ks && d.stride == 1 && p.kc == 64 && p.msub == 2 && p.Wt == 128 && p.Ht == 2 && p.Bt == 1 &&
-        p.block_n <= halo_nmax) {
+    if (p.ksplit == 1 && halo_ks && d.stride == 1 && p.kc == 64 && p.msub == 2 && p.Wt == 128 && p.Ht == 2 && p.Bt == 1) {
         // CTA pairs (cta_group::2) for the 128-wide layers: each CTA keeps half of the weight rows, which makes room for
         // a third pipeline stage, and every MMA reads a quarter less shared memory
-        static const int pair_on = getenv("FUSG_NO_PAIR2") ? 0 : 1;
-        const int tiles_all = p.tiles_x * p.tiles_y * p.tiles_b * p.n_tiles;
-        p.pair = (pair_on && d.ksize == 3 && p.block_n == 128 && p.n_tiles == 1 && !p.w_resident && tiles_all % 2 == 0 && tiles_all >= 4 * num_sms) ? 1 : 0;
+        p.pair = (d.ksize == 3 && p.block_n == 128 && p.n_tiles == 1 && !p.w_resident && total_tiles % 2 == 0 && total_tiles >= 4 * num_sms) ? 1 : 0;
         if (p.pair) p.b_bytes = (p.block_n / 2) * p.kc * 2;                 // half of the weight rows per CTA and k-block
         const int stage_bytes = 2 * TC_HALO_BYTES + (p.w_resident ? 0 : d.ksize * p.b_bytes);
         // wide kernels (5x5 / 7x7): a third pipeline stage is worth more than the staged epilogue's 32 KB
-        static const int deep_pipe = getenv("FUSG_HALO_KEEP_STAGED") ? 0 : 1;
-        if (deep_pipe && d.ksize > 3 && want_staged && (192 * 1024) / stage_bytes < 3 && (222 * 1024) / stage_bytes >= 3) want_staged = false;
+        if (d.ksize > 3 && want_staged && (192 * 1024) / stage_bytes < 3 && (222 * 1024) / stage_bytes >= 3) want_staged = false;
         const int budget = (want_staged ? 192 : 222) * 1024 - (p.w_resident ? p.num_kblocks * p.b_bytes : 0);
         int st = budget / stage_bytes;
         if (st > TC_MAX_STAGES) st = TC_MAX_STAGES;
         if (st >= 2) { p.halo = 1; p.stages = st; p.group = 1; }
         else if (p.pair) return FUSG_ERR_UNSUPPORTED;
     }
-    p.halo_skip = 0;
     if (p.halo && d.zero_kblocks && d.ksize == 3) {
         const int cpt = p.chunks0 + p.chunks1;
         for (int ky = 0; ky < 3 && 9 * cpt <= 64; ++ky)
@@ -1446,6 +1444,7 @@ static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
     }
     int cols = 2 * p.msub * p.block_n;
     p.tmem_cols = cols < 32 ? 32 : cols;
+    p.epi_smem = want_staged ? TC_STAGING_BYTES : (p.ksplit > 1 ? p.block_n * TC_BLOCK_M * 4 : 0);
 
     // lean epilogue: no noise, only NHWC bf16 outputs (<= one raw, <= one ELU) with one addressing mode
     {
@@ -1492,6 +1491,24 @@ static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
         }
         p.fe = fe;
     }
+    const unsigned long long wbytes = (unsigned long long)d.cout_pad * taps * (d.c0 + d.c1) * 2ull;
+    p.w_prefetch_bytes = (total_tiles * p.ksplit <= 64 && wbytes >= 65536ull && (reinterpret_cast<uintptr_t>(d.weight) & 15) == 0) ? wbytes : 0ull;
+    // persistent CTAs own a STATIC share of the tiles, and one CTA fills an SM: if a co-tenant (the solver warps of the warp
+    // stage that runs next to the VUNet in a pipeline step) holds even one SM, the CTA meant for it starts only when another
+    // CTA has finished its whole share -- the layer takes twice as long.  g_sm_reserve SMs are therefore left to co-tenants.
+    const int usable = num_sms - g_sm_reserve > 8 ? num_sms - g_sm_reserve : num_sms;
+    grid = p.ksplit > 1 ? total_tiles * p.ksplit /* one cluster per tile */ : (total_tiles < usable ? total_tiles : usable);
+    if (p.pair) grid &= ~1;                                                  // whole CTA pairs
+    smem = tc_smem(p).total;
+    return FUSG_OK;
+}
+
+static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
+    ConvTcParams p;
+    int grid;
+    size_t smem;
+    const int rc = plan_tc(d, Ho, Wo, fusg_num_sms(), p, grid, smem);
+    if (rc != FUSG_OK) return rc;
     PFN_encodeTiled enc = get_encode();
     const CUtensorMapSwizzle sw = p.kc == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
     // c = channels the tensor really holds: a k-block box that reaches beyond them is zero-filled by TMA
@@ -1509,7 +1526,7 @@ static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
     if (!encodeA(&p.tmA0, d.in0, d.cphys0 ? d.cphys0 : d.c0, d.pitch0)) return FUSG_ERR_UNSUPPORTED;
     if (d.in1 && !encodeA(&p.tmA1, d.in1, d.cphys1 ? d.cphys1 : d.c1, d.pitch1)) return FUSG_ERR_UNSUPPORTED;
     {
-        const int ktot = taps * (d.c0 + d.c1);
+        const int ktot = d.ksize * d.ksize * (d.c0 + d.c1);
         cuuint64_t dims[2] = {(cuuint64_t)ktot, (cuuint64_t)d.cout_pad};
         cuuint64_t strides[1] = {(cuuint64_t)ktot * 2};
         cuuint32_t box[2] = {(cuuint32_t)p.kc, (cuuint32_t)(p.pair ? p.block_n / 2 : p.block_n)};
@@ -1518,10 +1535,6 @@ static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
                 CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return FUSG_ERR_UNSUPPORTED;
     }
-    const size_t pipe_a = p.halo ? (size_t)p.stages * 2 * TC_HALO_BYTES : (size_t)p.stages * p.group * p.a_bytes;
-    const size_t pipe_b = p.w_resident ? (size_t)p.num_kblocks * p.b_bytes : (p.halo ? (size_t)p.stages * d.ksize * p.b_bytes : (size_t)p.stages * p.group * p.b_bytes);
-    const size_t smem = pipe_a + pipe_b +
-                        1024 /*align slack*/ + 1024 /*barriers, first KB*/ + 16 + (size_t)d.cout_pad * 4 /*bias*/ + (want_staged ? 32768 : 0) /*epilogue staging*/ + (p.ksplit > 1 ? (size_t)p.block_n * TC_BLOCK_M * 4 : 0) /*split-K receive buffer*/;
     if (fusg_once_per_device(0, 0, [] {
             cudaError_t e = cudaFuncSetAttribute(k_conv_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
             return e != cudaSuccess ? e : cudaFuncSetAttribute(k_conv_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
@@ -1529,38 +1542,22 @@ static int launch_tc(const fusg_conv_desc &d, int Ho, int Wo, cudaStream_t st) {
         return fusg_check_launch();
     g_last_plan[0] = p.msub; g_last_plan[1] = p.pair; g_last_plan[2] = p.halo; g_last_plan[3] = p.ksplit;
     g_last_plan[4] = p.stages; g_last_plan[5] = p.group; g_last_plan[6] = p.w_resident; g_last_plan[7] = p.fast_epi;
-    const int total_tiles = p.tiles_x * p.tiles_y * p.tiles_b * p.n_tiles;
-    static const int pdl_on = getenv("FUSG_NO_PDL") ? 0 : 1;
-    p.pdl = pdl_on;
-    {
-        static const int wpf_on = getenv("FUSG_NO_WPREFETCH") ? 0 : 1;
-        const unsigned long long wbytes = (unsigned long long)d.cout_pad * taps * (d.c0 + d.c1) * 2ull;
-        p.w_prefetch_bytes = (wpf_on && pdl_on && total_tiles * p.ksplit <= 64 && wbytes >= 65536ull && (reinterpret_cast<uintptr_t>(d.weight) & 15) == 0) ? wbytes : 0ull;
-    }
-    // persistent CTAs own a STATIC share of the tiles, and one CTA fills an SM: if a co-tenant (the solver warps of the warp
-    // stage that runs next to the VUNet in a pipeline step) holds even one SM, the CTA meant for it starts only when another
-    // CTA has finished its whole share -- the layer takes twice as long.  g_sm_reserve SMs are therefore left to co-tenants.
-    const int usable = num_sms - g_sm_reserve > 8 ? num_sms - g_sm_reserve : num_sms;
-    int grid = p.ksplit > 1 ? total_tiles * p.ksplit /* one cluster per tile */ : (total_tiles < usable ? total_tiles : usable);
-    if (p.pair) grid &= ~1;                                                  // whole CTA pairs
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3((unsigned)grid, 1, 1);
     cfg.blockDim = dim3(TC_THREADS, 1, 1);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
+    // programmatic stream serialization: the kernel's prologue overlaps the previous kernel (griddepcontrol in k_conv_tc)
     cudaLaunchAttribute attr[2];
-    int na = 0;
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    int na = 1;
     if (p.ksplit > 1 || p.pair) {
         attr[na].id = cudaLaunchAttributeClusterDimension;
         attr[na].val.clusterDim.x = p.pair ? 2u : (unsigned)p.ksplit;
         attr[na].val.clusterDim.y = 1;
         attr[na].val.clusterDim.z = 1;
-        ++na;
-    }
-    if (p.pdl) {
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
         ++na;
     }
     cfg.attrs = attr;

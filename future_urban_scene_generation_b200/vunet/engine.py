@@ -10,7 +10,6 @@ dtype 'bf16' is the product path (tcgen05 kernels); dtype 'fp32' is the verifica
 (north_star: <=1e-4), which runs the same program on the CUDA-core direct kernel.
 """
 import ctypes as C
-import os
 
 from .. import _lib
 
@@ -77,14 +76,10 @@ class VunetEngine:
         self._w = {}
         self._wp = {}                  # pixel-pair packed weights of the narrow stride-1 layers
         self._wfused = {}              # combined weights of fused layer pairs (see prepare_weights)
-        self.fuse_first_nin = os.environ.get("FUSG_NO_NIN_FUSE") is None   # fold app_encoder_1.nin into residual_0 (bf16 path)
-        self.pair_narrow = os.environ.get("FUSG_NO_PAIR") is None   # run 32-channel stride-1 layers on pixel pairs (fusg_fold_weightnorm_paired)
         self.launches = 0
         self.profile = None            # list -> per-launch (path, impl, flops, start, end) CUDA-event records
         self.noise_provider = None     # callable(B,C,H,W) -> NHWC fp32 device tensor; None = CPU torch.randn (reference semantics)
         self.raw_skips = True          # also keep raw copies of NiN skips (needed by the sub-forward API)
-        # the 6- / 3-channel network inputs are stored 16 channels wide; TMA zero-fills the rest of their 64- / 32-channel K block
-        self.input_cphys = None if os.environ.get("FUSG_NO_CPHYS") else 16
 
     # ------------------------------------------------------------------ plumbing
     @property
@@ -135,7 +130,7 @@ class VunetEngine:
             for path, conv in self.m.convs.items():
                 cout, cin, k = conv.cout, conv.cin, conv.k
                 cin_pad = 32 if cin < 16 else cin            # the two RGB-ish first layers are padded to one 64B swizzle span
-                if path == FUSED_NIN[0] and self.fuse_first_nin and self.dtype == "bf16":
+                if path == FUSED_NIN[0] and self.dtype == "bf16":
                     cin_pad = 64                             # its input doubles as a 64-channel operand of the fused residual
                 cout_pad = _pad16(cout)
                 w = torch.empty((cout_pad, k * k, cin_pad), dtype=self.tdtype, device=dev)
@@ -163,7 +158,7 @@ class VunetEngine:
             # centre tap and zero elsewhere -- the tensor core adds the residual, so x0 itself is never written or read
             # (2.1 GB of HBM traffic per 64-crop forward); the kernel skips the all-zero k-blocks (zero_kblocks hint)
             self._wfused = {}
-            if self.fuse_first_nin and self.dtype == "bf16":
+            if self.dtype == "bf16":
                 nin_p, res_p = FUSED_NIN
                 wn, bn, cout, cout_pad, cinp_n, _ = self._w[nin_p]
                 wr, br, _, _, cinp_r, k = self._w[res_p]
@@ -190,7 +185,7 @@ class VunetEngine:
             w, bias, cout, cout_pad, cin_pad, k = self._w[path]
         a0, which0 = srcs[0]
         # pixel-pair packing: [B,H,W,32] viewed as [B,H,W/2,64] (same bytes) for narrow stride-1 layers
-        pair = (not fused and self.pair_narrow and path in self._wp and stride == 1 and noise is None and a0.W >= 64 and a0.W % 2 == 0
+        pair = (not fused and path in self._wp and stride == 1 and noise is None and a0.W >= 64 and a0.W % 2 == 0
                 and all(a.C == 32 and a.pitch == 32 and a.off == 0 for a, _ in srcs) and all(o.mode == PLAIN for o in outs))
         if pair:
             w, bias, cout, cout_pad, cin_pad, k = self._wp[path]
@@ -446,7 +441,8 @@ class VunetEngine:
     def enc_up(self, x_nchw):
         """models.py:333-353 -> (outputs [Act,Act], skips [Act,Act])."""
         B = x_nchw.shape[0]
-        xin = self.from_nchw(x_nchw, elu_only=True, cpad=self._w["app_encoder_1.nin.layers.1"][4], cphys=self.input_cphys)
+        # the 6- / 3-channel network inputs are stored 16 channels wide; TMA zero-fills the rest of their 64- / 32-channel K block
+        xin = self.from_nchw(x_nchw, elu_only=True, cpad=self._w["app_encoder_1.nin.layers.1"][4], cphys=16)
         x, _ = self.init_block("app_encoder_1", xin, B)
         for name in ("app_encoder_1_a", "app_encoder_1_b", "app_encoder_1_c", "app_encoder_2"):
             x, _ = self.down_block(name, x, B)
@@ -476,7 +472,7 @@ class VunetEngine:
     def dec_up(self, y_nchw):
         """models.py:355-388 -> (outputs [Act], skips [14 Acts])."""
         B = y_nchw.shape[0]
-        yin = self.from_nchw(y_nchw, elu_only=True, cpad=32, cphys=self.input_cphys)
+        yin = self.from_nchw(y_nchw, elu_only=True, cpad=32, cphys=16)
         rs = self.raw_skips
         skips = []
         x, sl = self.init_block("shape_encoder_1", yin, B, last_elu=True)

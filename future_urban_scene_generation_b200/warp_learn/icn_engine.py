@@ -18,7 +18,6 @@ floor of ~1.1e-2 under it (tests/test_icn_gpu.py; same tensor-core rate).  dtype
 bf16; dtype 'fp32' runs it on the CUDA-core direct kernel (verification build, <= 1e-4).
 """
 import ctypes as C
-import os
 
 from .. import _lib
 from ..vunet.engine import ConvDesc, DT_BF16, DT_F32, IMPL_AUTO, IMPL_TC, IMPL_DIRECT
@@ -106,7 +105,7 @@ class IcnEngine:
             # K of a narrow-input layer is widened to 64 (TMA zero-fills beyond the 32 stored channels, fusg_conv_desc.cphys0):
             # twice the tensor work, but a 64-channel k-block is what the sliding-window A tiles need -- one row-segment load
             # per (tile, ky) instead of a load per tap (49 for the 7x7 first layer)
-            kwide = 64 if (cin_pad == 32 and k >= 5 and os.environ.get("FUSG_ICN_NO_KWIDE") is None) else cin_pad
+            kwide = 64 if cin_pad == 32 and k >= 5 else cin_pad
             cout_pad = _pad16(cout)
             wp = torch.zeros((cout_pad, k * k, kwide), dtype=torch.float32, device=dev)
             wp[:cout, :, :cin] = w.permute(0, 2, 3, 1).reshape(cout, k * k, cin)

@@ -20,19 +20,6 @@
  * Faults: device-side mbarrier waits are bounded (seconds); a TMA-descriptor or pipeline bug makes the
  * kernel trap (the next call returns FUSG_ERR_CUDA, fusg_last_error names the launch failure) instead
  * of hanging the GPU.
- *
- * Environment switches (read once per process; DEBUG / A-B measurement only, never needed for correctness,
- * every setting gives results within the same tolerances):
- *   FUSG_MSUB1=1            conv: 128-row CTA tiles only (no 256-row tiles)
- *   FUSG_NO_HALO=1          conv: no sliding-window A tiles for wide 3x3/5x5/7x7 layers
- *   FUSG_HALO_NMAX=<n>      conv: widest N tile that may use the sliding window (default 128)
- *   FUSG_HALO_KEEP_STAGED=1 conv: keep the staged epilogue instead of a third pipeline stage on 5x5/7x7
- *   FUSG_NO_PAIR2=1         conv: no cta_group::2 CTA pairs
- *   FUSG_KSPLIT_MAX=<n>     conv: largest split-K cluster (default 8); FUSG_KSPLIT_MIN_KB=<n> smallest K (in
- *                           k-blocks) that is split (default 36)
- *   FUSG_EPI_DIRECT=1       conv: no warp-staged epilogue; FUSG_STAGED_1X1=0: not for the 1x1 layers
- *   FUSG_NO_PDL=1           conv: no programmatic dependent launch; FUSG_NO_WPREFETCH=1: no L2 weight prefetch ahead of the wait
- *   FUSG_SM_RESERVE=<n>     conv: initial value of fusg_conv2d_set_sm_reserve (default 0)
  */
 #ifndef FUSG_H_
 #define FUSG_H_
