@@ -32,6 +32,7 @@ def _load():
         "fusg_warp_workspace_bytes_hw": ([i, i, i], sz),
         "fusg_warp_fused": ([vp] * 11 + [vp, sz, i, i, i, vp], i),
         "fusg_warp_fused_traj": ([vp] * 12 + [vp, sz, i, i, i, vp], i),
+        "fusg_warp_fused_idx": ([vp, vp, i] + [vp] * 11 + [vp, sz, i, i, i, vp], i),
         "fusg_step_keypoints": ([vp] * 10 + [i, i, i, vp], i),
         "fusg_visibility": ([vp] * 6 + [i, i, i, vp], i),
         "fusg_get_planes": ([vp] * 3 + [i, i, i, vp], i),
@@ -57,6 +58,9 @@ def _load():
         "fusg_paste_workspace_bytes": ([i, i, i], sz),
         "fusg_paste_back": ([vp] * 7 + [sz, i, i, i, i, i, i, vp], i),
         "fusg_u8_to_vunet_inputs": ([vp] * 5 + [i, i, vp], i),
+        "fusg_u8_to_vunet_y": ([vp, vp, i, i, vp], i),
+        "fusg_gather_rows": ([vp, i, vp, i, vp], i),
+        "fusg_sizeof_gather_seg": ([], sz),
         "fusg_mask_bbox": ([vp] * 4 + [i, i, vp], i),
         "fusg_pack_icn_inputs": ([vp] * 8 + [i, vp, vp, i, i, i, i, vp], i),
         "fusg_pack_vunet_inputs": ([vp] * 10 + [i, i, i, i, vp], i),

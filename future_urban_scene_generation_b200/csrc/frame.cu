@@ -264,6 +264,42 @@ __global__ void __launch_bounds__(256) k_u8_to_inputs(const uint8_t *__restrict_
     }
 }
 
+// y alone (the trajectory step: the appearance image x is encoded once per vehicle, not per item) -- the same arithmetic
+__global__ void __launch_bounds__(256) k_u8_to_y(const uint8_t *__restrict__ nd, float *__restrict__ y, int res) {
+    const int b = blockIdx.y;
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= res * res) return;
+    const size_t plane = (size_t)res * res, q = ((size_t)b * plane + p) * 3;
+    float *yb = y + (size_t)b * 3 * plane + p;
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) yb[ch * plane] = to_tensor1(nd[q + 2 - ch]);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Per-item gather of per-vehicle rows: dst row b of every segment = src row index[b] (zeros for an index out of range).  The
+// segment table travels in the kernel's parameter space, so a captured graph holds it by value.  grid (segment, item, split):
+// a CTA copies a 1/split share of one row with 16-byte vectors.
+// ---------------------------------------------------------------------------------------------------------------
+struct GatherTable { fusg_gather_seg s[FUSG_GATHER_MAX_SEGS]; };
+
+constexpr int GATHER_THREADS = 256;
+
+__global__ void __launch_bounds__(GATHER_THREADS) k_gather_rows(const GatherTable tab, const int32_t *__restrict__ index) {
+    const fusg_gather_seg &sg = tab.s[blockIdx.x];
+    const int b = blockIdx.y;
+    const long long n16 = sg.row_bytes / 16;
+    const long long per = (n16 + gridDim.z - 1) / gridDim.z, k0 = per * blockIdx.z, k1 = min(n16, k0 + per);
+    if (k0 >= n16) return;
+    const int r = index[b];
+    int4 *d = reinterpret_cast<int4 *>(static_cast<uint8_t *>(sg.dst) + (size_t)b * sg.row_bytes);
+    if (r < 0 || r >= sg.n_src) {
+        for (long long k = k0 + threadIdx.x; k < k1; k += GATHER_THREADS) d[k] = make_int4(0, 0, 0, 0);
+        return;
+    }
+    const int4 *s4 = reinterpret_cast<const int4 *>(static_cast<const uint8_t *>(sg.src) + (size_t)r * sg.row_bytes);
+    for (long long k = k0 + threadIdx.x; k < k1; k += GATHER_THREADS) d[k] = __ldg(s4 + k);
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // ICN input packing (warp_learn/models.py:323-366 get_icn_inputs): square crop (bbox of the sketch mask) + cv2.resize of the
 // destination normal sketch and of the five warped planes, cv2's 8-bit RGB/BGR -> Lab, ToTensor + Normalize(0.5, 0.5),
@@ -389,6 +425,36 @@ extern "C" int fusg_u8_to_vunet_inputs(const uint8_t *mask_bbox, const uint8_t *
     if (!mask_bbox || !normal_src || !normal_dst || !x || !y || B <= 0 || res <= 0) return FUSG_ERR_ARG;
     if (B > 65535 || res > 4096) return FUSG_ERR_UNSUPPORTED;
     k_u8_to_inputs<<<dim3((res * res + 255) / 256, B), 256, 0, (cudaStream_t)stream>>>(mask_bbox, normal_src, normal_dst, x, y, res);
+    fusg_count_launch(1);
+    return fusg_check_launch();
+}
+
+extern "C" int fusg_u8_to_vunet_y(const uint8_t *normal_dst, float *y, int B, int res, void *stream) {
+    if (!normal_dst || !y || B <= 0 || res <= 0) return FUSG_ERR_ARG;
+    if (B > 65535 || res > 4096) return FUSG_ERR_UNSUPPORTED;
+    k_u8_to_y<<<dim3((res * res + 255) / 256, B), 256, 0, (cudaStream_t)stream>>>(normal_dst, y, res);
+    fusg_count_launch(1);
+    return fusg_check_launch();
+}
+
+extern "C" size_t fusg_sizeof_gather_seg(void) { return sizeof(fusg_gather_seg); }
+
+extern "C" int fusg_gather_rows(const fusg_gather_seg *segs, int nseg, const int32_t *index, int B, void *stream) {
+    if (!segs || nseg <= 0 || nseg > FUSG_GATHER_MAX_SEGS || !index || B <= 0) return FUSG_ERR_ARG;
+    GatherTable tab = {};
+    long long max16 = 0;
+    for (int i = 0; i < nseg; ++i) {
+        const fusg_gather_seg &sg = segs[i];
+        if (!sg.src || !sg.dst || sg.n_src <= 0 || sg.row_bytes <= 0 || sg.row_bytes % 16 != 0) return FUSG_ERR_ARG;
+        if ((reinterpret_cast<uintptr_t>(sg.src) | reinterpret_cast<uintptr_t>(sg.dst)) & 15) return FUSG_ERR_ARG;
+        tab.s[i] = sg;
+        max16 = sg.row_bytes / 16 > max16 ? sg.row_bytes / 16 : max16;
+    }
+    if (B > 65535) return FUSG_ERR_UNSUPPORTED;
+    // a CTA moves at least 4 vectors per thread; rows of a few KB (the cached appearance tensors) take one CTA each
+    long long split = (max16 + 4 * GATHER_THREADS - 1) / (4 * GATHER_THREADS);
+    if (split > 1024) split = 1024;
+    k_gather_rows<<<dim3(nseg, B, (unsigned)split), GATHER_THREADS, 0, (cudaStream_t)stream>>>(tab, index);
     fusg_count_launch(1);
     return fusg_check_launch();
 }

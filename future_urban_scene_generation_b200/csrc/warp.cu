@@ -171,12 +171,14 @@ struct PlaneRec {
 __global__ void __launch_bounds__(256) k_plane_gate(const int32_t *__restrict__ src_kp, const int32_t *__restrict__ dst_kp,
                                                     const uint8_t *__restrict__ vis, int8_t *__restrict__ plane_j, double *__restrict__ H12,
                                                     double *__restrict__ Minv, int *__restrict__ counters, int *__restrict__ list6,
-                                                    int *__restrict__ list4, int B, int H, int W) {
+                                                    int *__restrict__ list4, const int32_t *__restrict__ src_index, int n_src,
+                                                    int B, int H, int W) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= B * N_TEX) return;
     const int b = t / N_TEX, i = t % N_TEX;
     const uint8_t *sv = vis + 2 * N_VIS * b, *dv = sv + N_VIS;
     bool bad = sv[0] == 0xff || dv[0] == 0xff;
+    if (src_index && (src_index[b] < 0 || src_index[b] >= n_src)) bad = true;     // no source image: refused like an absurd vertex
     const int32_t *sk = src_kp + 2 * N_KP * b, *dk = dst_kp + 2 * N_KP * b;
     for (int k = 0; k < 2 * N_KP && !bad; ++k)
         if (abs(sk[k]) > POLY_COORD_MAX || abs(dk[k]) > POLY_COORD_MAX) bad = true;
@@ -507,9 +509,11 @@ __device__ __forceinline__ void row_polygon_span(const float *fx, const float *f
 
 // WIN = rows of the source window.  First launch: a persistent grid strides over the crops; oversize crops are appended to big_list.
 // Second launch (big_list != nullptr as INPUT, `from_list`): a fixed grid strides over the queued crops.
+// src_index (may be NULL): crop b reads source image src_index[b] (k_plane_gate has refused every crop whose index is out of
+// range, so such a crop selects no plane and never reaches the source read).
 template <int WIN>
 __global__ void __launch_bounds__(WARP_THREADS, WIN == WIN_SMALL ? 2 : 1)
-k_warp_rows(const uint8_t *__restrict__ src, const int32_t *__restrict__ src_kp, const int8_t *__restrict__ plane_j,
+k_warp_rows(const uint8_t *__restrict__ src, const int32_t *__restrict__ src_index, const int32_t *__restrict__ src_kp, const int8_t *__restrict__ plane_j,
             const double *__restrict__ Minv, const PlaneRec *__restrict__ recs, uint8_t *__restrict__ warped, int H, int W, int *__restrict__ big_count,
             int *__restrict__ big_list, int from_list, int n_crops, int zero_ahead) {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -550,7 +554,6 @@ k_warp_rows(const uint8_t *__restrict__ src, const int32_t *__restrict__ src_kp,
     const int n_items = from_list ? *big_count : n_crops;
     for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
         const int b = from_list ? big_list[item] : item;
-        const uint8_t *gsrc = src + (size_t)b * crop_bytes;
         uint8_t *gout = warped + (size_t)b * N_TEX * crop_bytes;
         __syncthreads();                                      // previous item done with the header / window
         // (filler lanes) this lane's blocks of the crop `zero_ahead` crops on are issued a block at a time between the rows of
@@ -618,7 +621,7 @@ k_warp_rows(const uint8_t *__restrict__ src, const int32_t *__restrict__ src_kp,
             continue;
         }
         const int win_rows = win_hi - win_lo + 1;
-        const uint8_t *gwin = gsrc + (size_t)win_lo * row_bytes;
+        const uint8_t *gwin = src + (size_t)(src_index ? src_index[b] : b) * crop_bytes + (size_t)win_lo * row_bytes;
         const uint32_t win_bytes = (uint32_t)win_rows * row_bytes;
         const bool use_tma = (win_bytes % 16 == 0) && ((reinterpret_cast<uintptr_t>(gwin) & 15) == 0);
         if (use_tma) {
@@ -829,7 +832,8 @@ __global__ void __launch_bounds__(32 * PM_ROWS) k_plane_masks(const int32_t *__r
 
 constexpr int WF_ROWS = 8;        // output rows per CTA of k_warp_frame: one per warp
 
-__global__ void __launch_bounds__(32 * WF_ROWS) k_warp_frame(const uint8_t *__restrict__ src, const int32_t *__restrict__ src_kp,
+__global__ void __launch_bounds__(32 * WF_ROWS) k_warp_frame(const uint8_t *__restrict__ src, const int32_t *__restrict__ src_index,
+                                                            const int32_t *__restrict__ src_kp,
                                                             const int8_t *__restrict__ plane_j, const double *__restrict__ Minv,
                                                             const uint32_t *__restrict__ masks, uint8_t *__restrict__ warped, int H, int W, int words,
                                                             int row_smem) {
@@ -874,7 +878,7 @@ __global__ void __launch_bounds__(32 * WF_ROWS) k_warp_frame(const uint8_t *__re
         return;
     }
     uint8_t *s_row = s_rows + (size_t)warp * row_smem;
-    const uint8_t *simg = src + (size_t)b * H * W * 3;
+    const uint8_t *simg = src + (size_t)(src_index ? src_index[b] : b) * H * W * 3;     // a refused index selects no plane (i < 0 above)
     const uint32_t *mk = masks + ((size_t)b * N_TEX + i) * H * words;
     const int bw = warp_block_w(H, W);
     for (int x = lane; x < W; x += 32) {
@@ -977,12 +981,14 @@ extern "C" int fusg_warp_perspective(const uint8_t *img, const double *Hm, uint8
     return fusg_check_launch();
 }
 
-static int warp_fused_impl(const uint8_t *src, const int32_t *src_kp, const int32_t *dst_kp, const double *K,
+// src_index == nullptr: crop b reads src[b].  Otherwise src holds n_src images and crop b reads src[src_index[b]].
+static int warp_fused_impl(const uint8_t *src, const int32_t *src_index, int n_src, const int32_t *src_kp, const int32_t *dst_kp, const double *K,
                            const double *E_src, const double *E_dst, const double *kp3d, const double *kp3d_dst, uint8_t *warped, uint8_t *vis,
                            int8_t *plane_j, double *H12, void *workspace, size_t workspace_bytes, int B, int H, int W,
                            void *stream) {
     if (!src || !src_kp || !dst_kp || !K || !E_src || !E_dst || !kp3d || !warped || !vis || !plane_j || !workspace) return FUSG_ERR_ARG;
     if (B <= 0) return FUSG_ERR_ARG;
+    if (src_index && n_src <= 0) return FUSG_ERR_ARG;
     if (H < 8 || W < 8 || H > 65535 || B > 65535) return FUSG_ERR_UNSUPPORTED;
     const bool frame_path = H > MAX_HW || W > MAX_HW;
     if (workspace_bytes < fusg_warp_workspace_bytes_hw(B, H, W)) return FUSG_ERR_WORKSPACE;
@@ -1000,7 +1006,7 @@ static int warp_fused_impl(const uint8_t *src, const int32_t *src_kp, const int3
     }
     k_visibility<<<(2 * B + VIS_WARPS - 1) / VIS_WARPS, VIS_WARPS * 32, 0, st>>>(K, E_src, E_dst, kp3d, kp3d_dst, vis, nullptr, nullptr, 2 * B, H, W);
     if (fusg_record_cuda(cudaMemsetAsync(counters, 0, 4 * sizeof(int), st)) != FUSG_OK) return FUSG_ERR_CUDA;
-    k_plane_gate<<<(B * N_TEX + 255) / 256, 256, 0, st>>>(src_kp, dst_kp, vis, plane_j, H12, Minv, counters, list6, list4, B, H, W);
+    k_plane_gate<<<(B * N_TEX + 255) / 256, 256, 0, st>>>(src_kp, dst_kp, vis, plane_j, H12, Minv, counters, list6, list4, src_index, n_src, B, H, W);
     fusg_count_launch(2);
     // The zero fill of the five planes (97 % of the output bytes stay zero) rides inside k_warp_rows as TMA bulk stores issued
     // two crops ahead of the gather (see the kernel); only outputs that are not 16-byte granular are cleared by a memset.
@@ -1026,10 +1032,10 @@ static int warp_fused_impl(const uint8_t *src, const int32_t *src_kp, const int3
     if (!frame_path) {
         // persistent: two CTAs per SM stride over the crops
         const int grid = B < 2 * fusg_num_sms() ? B : 2 * fusg_num_sms();
-        k_warp_rows<WIN_SMALL><<<grid, WARP_THREADS, warp_smem_bytes(WIN_SMALL), st>>>(src, src_kp, plane_j, Minv, recs, warped, H, W, counters + 2, big_list, 0, B, bulk_zero ? ZERO_AHEAD : 0);
+        k_warp_rows<WIN_SMALL><<<grid, WARP_THREADS, warp_smem_bytes(WIN_SMALL), st>>>(src, src_index, src_kp, plane_j, Minv, recs, warped, H, W, counters + 2, big_list, 0, B, bulk_zero ? ZERO_AHEAD : 0);
         // crops whose polygons span more than WIN_SMALL source rows (a vehicle filling the crop): full-height window
         const int bgrid = B < fusg_num_sms() ? B : fusg_num_sms();
-        k_warp_rows<MAX_HW><<<bgrid, WARP_THREADS, warp_smem_bytes(MAX_HW), st>>>(src, src_kp, plane_j, Minv, recs, warped, H, W, counters + 2, big_list, 1, B, 0);
+        k_warp_rows<MAX_HW><<<bgrid, WARP_THREADS, warp_smem_bytes(MAX_HW), st>>>(src, src_index, src_kp, plane_j, Minv, recs, warped, H, W, counters + 2, big_list, 1, B, 0);
         fusg_count_launch(2);
     } else {
         const int words = (W + 31) / 32;
@@ -1041,7 +1047,7 @@ static int warp_fused_impl(const uint8_t *src, const int32_t *src_kp, const int3
         if (frame_smem > 48 * 1024 &&
             fusg_once_per_device(2, frame_smem, [frame_smem] { return cudaFuncSetAttribute(k_warp_frame, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)frame_smem); }) != cudaSuccess)
             return fusg_check_launch();
-        k_warp_frame<<<dim3((H + WF_ROWS - 1) / WF_ROWS, N_TEX, B), 32 * WF_ROWS, frame_smem, st>>>(src, src_kp, plane_j, Minv, masks, warped, H, W, words, (int)row_smem);
+        k_warp_frame<<<dim3((H + WF_ROWS - 1) / WF_ROWS, N_TEX, B), 32 * WF_ROWS, frame_smem, st>>>(src, src_index, src_kp, plane_j, Minv, masks, warped, H, W, words, (int)row_smem);
         fusg_count_launch(4);
     }
     return fusg_check_launch();
@@ -1051,7 +1057,7 @@ extern "C" int fusg_warp_fused(const uint8_t *src, const int32_t *src_kp, const 
                                const double *E_src, const double *E_dst, const double *kp3d, uint8_t *warped, uint8_t *vis,
                                int8_t *plane_j, double *H12, void *workspace, size_t workspace_bytes, int B, int H, int W,
                                void *stream) {
-    return warp_fused_impl(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, nullptr, warped, vis, plane_j, H12, workspace, workspace_bytes, B, H, W, stream);
+    return warp_fused_impl(src, nullptr, 0, src_kp, dst_kp, K, E_src, E_dst, kp3d, nullptr, warped, vis, plane_j, H12, workspace, workspace_bytes, B, H, W, stream);
 }
 
 extern "C" int fusg_warp_fused_traj(const uint8_t *src, const int32_t *src_kp, const int32_t *dst_kp, const double *K,
@@ -1059,5 +1065,14 @@ extern "C" int fusg_warp_fused_traj(const uint8_t *src, const int32_t *src_kp, c
                                     uint8_t *warped, uint8_t *vis, int8_t *plane_j, double *H12, void *workspace, size_t workspace_bytes,
                                     int B, int H, int W, void *stream) {
     if (!kp3d_dst) return FUSG_ERR_ARG;
-    return warp_fused_impl(src, src_kp, dst_kp, K, E_src, E_dst, kp3d_src, kp3d_dst, warped, vis, plane_j, H12, workspace, workspace_bytes, B, H, W, stream);
+    return warp_fused_impl(src, nullptr, 0, src_kp, dst_kp, K, E_src, E_dst, kp3d_src, kp3d_dst, warped, vis, plane_j, H12, workspace, workspace_bytes, B, H, W, stream);
+}
+
+extern "C" int fusg_warp_fused_idx(const uint8_t *src, const int32_t *src_index, int n_src, const int32_t *src_kp, const int32_t *dst_kp,
+                                   const double *K, const double *E_src, const double *E_dst, const double *kp3d_src, const double *kp3d_dst,
+                                   uint8_t *warped, uint8_t *vis, int8_t *plane_j, double *H12, void *workspace, size_t workspace_bytes,
+                                   int B, int H, int W, void *stream) {
+    if (!src_index || n_src <= 0) return FUSG_ERR_ARG;
+    return warp_fused_impl(src, src_index, n_src, src_kp, dst_kp, K, E_src, E_dst, kp3d_src, kp3d_dst, warped, vis, plane_j, H12, workspace,
+                           workspace_bytes, B, H, W, stream);
 }

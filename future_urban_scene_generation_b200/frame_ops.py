@@ -272,6 +272,44 @@ def u8_to_vunet_inputs(mask_bbox_u8, normal_src_u8, normal_dst_u8):
     return x, y
 
 
+def u8_to_vunet_y(normal_dst_u8):
+    """y_tilde alone: (B,res,res,3) uint8 CUDA tensor -> (B,3,res,res) fp32, the y of u8_to_vunet_inputs.  For a trajectory
+    step, whose appearance input was encoded once per vehicle (trajectory_inference.py:413-426)."""
+    torch = _lib.require_cuda()
+    B, res = int(normal_dst_u8.shape[0]), int(normal_dst_u8.shape[1])
+    if tuple(normal_dst_u8.shape) != (B, res, res, 3) or normal_dst_u8.dtype != torch.uint8:
+        raise ValueError("u8_to_vunet_y: expected a (B, res, res, 3) uint8 tensor")
+    y = torch.empty((B, 3, res, res), dtype=torch.float32, device=normal_dst_u8.device)
+    _lib.check(_lib.lib().fusg_u8_to_vunet_y(_lib.ptr(normal_dst_u8), _lib.ptr(y), B, res, _lib.stream_ptr(torch)), "fusg_u8_to_vunet_y")
+    return y
+
+
+GATHER_MAX_SEGS = 8      # FUSG_GATHER_MAX_SEGS
+
+
+class GatherSeg(C.Structure):
+    """fusg_gather_seg (include/fusg.h)."""
+    _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("row_bytes", C.c_int64), ("n_src", C.c_int32), ("reserved", C.c_int32)]
+
+
+def gather_rows(pairs, index):
+    """pairs: up to 8 (src (n_src, ...), dst (B, ...)) contiguous CUDA tensors; index: (B,) int32 CUDA tensor.
+    dst[b] = src[index[b]] for every pair (zeros where index[b] is out of range), in ONE launch on the current stream."""
+    torch = _lib.require_cuda()
+    if not 0 < len(pairs) <= GATHER_MAX_SEGS:
+        raise ValueError(f"gather_rows: 1..{GATHER_MAX_SEGS} (src, dst) pairs")
+    if index.dtype != torch.int32 or index.dim() != 1 or not index.is_cuda:
+        raise ValueError("gather_rows: index must be a (B,) int32 CUDA tensor")
+    B = int(index.shape[0])
+    segs = (GatherSeg * len(pairs))()
+    for s, (src, dst) in zip(segs, pairs):
+        if dst.shape[0] != B or src.shape[1:] != dst.shape[1:] or src.dtype != dst.dtype:
+            raise ValueError("gather_rows: dst must be (B,) + src.shape[1:] of src's dtype")
+        s.src, s.dst = _lib.ptr(src).value, _lib.ptr(dst).value
+        s.row_bytes, s.n_src = dst[0].numel() * dst.element_size(), int(src.shape[0])
+    _lib.check(_lib.lib().fusg_gather_rows(segs, len(pairs), _lib.ptr(index), B, _lib.stream_ptr(torch)), "fusg_gather_rows")
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # ICN input packing (SURVEY.md 8f-1): warp_learn/models.py:323-366 get_icn_inputs on the device
 # ---------------------------------------------------------------------------------------------------------------------

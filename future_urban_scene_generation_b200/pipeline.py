@@ -4,8 +4,14 @@
     H2D of the pinned inputs (copy stream)  ->  fused planar warp + VUNet forward + to_image
     (compute stream)  ->  D2H of the completed uint8 crops and warped planes (output stream)
 and returns immediately; `result(ticket)` blocks until that batch's outputs are in host memory.
-With `depth` batches in flight the copies of batch n+1 overlap the kernels of batch n, which is how
-a caller that streams (vehicle, step) pairs -- trajectory_inference.py:55,267 -- would drive the path.
+With `depth` batches in flight the copies of batch n+1 overlap the kernels of batch n.  Each item is
+one full reference forward (`Vunet_fix_res.forward`: appearance encoded per item, decoded with the
+sampled z).
+
+`TrajectoryPipeline` is the form of the trajectory loop (traj_test, trajectory_inference.py:230-233,
+:413-426): the appearance of each vehicle is encoded once (`set_vehicles`) and each submitted
+(vehicle, step) item runs only the shape path, decoded with the vehicle's cached means -- the
+reference's results at a quarter of the convolution work.
 
 The ~125 kernel launches of one step are captured once per slot into a CUDA graph (static device
 buffers) and replayed, so the host issues one launch per step instead of ~125.  Sampler noise is
@@ -18,7 +24,7 @@ import threading
 import torch
 
 from . import _lib
-from .frame_ops import u8_to_vunet_inputs
+from .frame_ops import gather_rows, u8_to_vunet_inputs, u8_to_vunet_y
 from .warp_learn.batch import warp_batch
 from .warp_learn.planes_utils import to_image_batch
 
@@ -45,8 +51,10 @@ class _Slot:
         self.wkey = None         # the engine's folded-weight key the graph was captured against
 
 
-class NovelViewPipeline:
-    WARP_KEYS = ("src", "src_kp", "dst_kp", "K", "E_src", "E_dst", "kp3d")
+class _GraphPipeline:
+    """What NovelViewPipeline and TrajectoryPipeline share: slots of static buffers with one captured graph each, the copy /
+    compute / output streams, the background Sampler-noise draw, the side-stream warp branch and the multi-GPU exchange.
+    A subclass supplies `_compute_inner(inp)`: one step of device work on the slot's input buffers."""
 
     def __init__(self, model, depth: int = 2, gather_fn=None, use_graph: bool = True, shared_stream: bool = False,
                  prefetch_noise: bool = True, return_warped: bool = False, micro_batches_per_step: int = 1):
@@ -78,6 +86,7 @@ class NovelViewPipeline:
         for sl in self.slots:
             sl.stream = one if shared_stream else torch.cuda.Stream(self.dev)
         self.n = 0
+        self.captures = 0                 # graphs captured so far (one per slot; again after a weight reload or a shape change)
 
     # ------------------------------------------------------------------ one step of device work
     #: SMs the persistent conv grids leave to the warp stage's solver warps while both run in one step (a persistent CTA
@@ -92,23 +101,11 @@ class NovelViewPipeline:
             _lib.lib().fusg_conv2d_set_sm_reserve(prev)
 
     def _compute_inner(self, inp):
-        # the planar warp is a chain of small latency-bound kernels (visibility -> homographies -> gather) that does
-        # not feed the VUNet of the same batch: fork it onto a side stream so it fills the SMs the narrow VUNet
-        # layers leave idle, and join before the outputs are read (inside a graph this becomes a parallel branch)
-        cur = torch.cuda.current_stream(self.dev)
-        self.side_stream.wait_stream(cur)
-        with torch.cuda.stream(self.side_stream):
-            res = warp_batch(*(inp[k] for k in self.WARP_KEYS), device=self.dev)
-        if "x" in inp:
-            x, y = inp["x"], inp["y"]
-        else:                                   # uint8 form: to_tensor / flip / concat on the device (frame_ops.u8_to_vunet_inputs)
-            x, y = u8_to_vunet_inputs(inp["x_mask_u8"], inp["x_normal_u8"], inp["y_normal_u8"])
-        x_tilde, _, _ = self.model(y, x)
-        crops = to_image_batch(x_tilde)
-        cur.wait_stream(self.side_stream)
-        for t in (res.warped, res.plane_j, res.vis):
-            t.record_stream(cur)
-        return {"crops": crops, "warped": res.warped, "plane_j": res.plane_j, "vis": res.vis}
+        raise NotImplementedError
+
+    def _graph_key(self, eng):
+        """What a captured graph depends on besides its input shapes: the device pointers of the folded weights."""
+        return eng._wkey
 
     def _prepare_slot(self, slot: _Slot, batch: dict):
         """First use of a slot: allocate static buffers, run once eagerly (weight fold, function
@@ -139,8 +136,9 @@ class NovelViewPipeline:
             with torch.cuda.graph(slot.graph, stream=slot.stream):
                 self._relayout_noise(slot)
                 slot.dev_out = self._compute(slot.inp)
+            self.captures += 1
         slot.launches = _lib.kernel_launches() - n0
-        slot.wkey = eng._wkey
+        slot.wkey = self._graph_key(eng)
         eng.noise_provider = prev
 
     def _relayout_noise(self, slot: _Slot):
@@ -205,7 +203,7 @@ class NovelViewPipeline:
         eng.prepare_weights()                 # no-op unless the parameters changed (load_state_dict, .to, in-place update)
         # a captured graph bakes in the device pointers of the folded weights: re-capture after a reload instead of
         # replaying over freed memory
-        fresh = slot.inp is None or slot.wkey != eng._wkey or set(slot.inp) != set(batch) or \
+        fresh = slot.inp is None or slot.wkey != self._graph_key(eng) or set(slot.inp) != set(batch) or \
             any(tuple(slot.inp[k].shape) != tuple(v.shape) for k, v in batch.items())
         if not resident and not fresh:
             self._take_noise(slot)                                    # host RNG work overlaps the batches still in flight
@@ -332,3 +330,157 @@ class NovelViewPipeline:
 
     def d2h_bytes(self, ticket: int) -> int:
         return sum(v.numel() * v.element_size() for v in self.slots[ticket % self.depth].out.values())
+
+
+class NovelViewPipeline(_GraphPipeline):
+    """One complete reference forward per item: warp + `Vunet_fix_res.forward(y, x)` (appearance encoded for every item,
+    decoded with the sampled z) + to_image.  See submit() for the batch keys."""
+    WARP_KEYS = ("src", "src_kp", "dst_kp", "K", "E_src", "E_dst", "kp3d")
+
+    def _compute_inner(self, inp):
+        # the planar warp is a chain of small latency-bound kernels (visibility -> homographies -> gather) that does
+        # not feed the VUNet of the same batch: fork it onto a side stream so it fills the SMs the narrow VUNet
+        # layers leave idle, and join before the outputs are read (inside a graph this becomes a parallel branch)
+        cur = torch.cuda.current_stream(self.dev)
+        self.side_stream.wait_stream(cur)
+        with torch.cuda.stream(self.side_stream):
+            res = warp_batch(*(inp[k] for k in self.WARP_KEYS), device=self.dev)
+        if "x" in inp:
+            x, y = inp["x"], inp["y"]
+        else:                                   # uint8 form: to_tensor / flip / concat on the device (frame_ops.u8_to_vunet_inputs)
+            x, y = u8_to_vunet_inputs(inp["x_mask_u8"], inp["x_normal_u8"], inp["y_normal_u8"])
+        x_tilde, _, _ = self.model(y, x)
+        crops = to_image_batch(x_tilde)
+        cur.wait_stream(self.side_stream)
+        for t in (res.warped, res.plane_j, res.vis):
+            t.record_stream(cur)
+        return {"crops": crops, "warped": res.warped, "plane_j": res.plane_j, "vis": res.vis}
+
+
+class TrajectoryPipeline(_GraphPipeline):
+    """The trajectory loop (traj_test, trajectory_inference.py:230-233 and :413-426): each vehicle's appearance is encoded
+    ONCE (`set_vehicles`: enc_up -> enc_down -> the six nin_k convolutions on the means mu), and every submitted (vehicle,
+    future step) item runs only the shape path -- warp of the vehicle's source crop, dec_up(y), dec_down with that vehicle's
+    cached appearance -- which is what the reference computes per step (decoding with mu_app), at a quarter of the
+    convolution work of a full forward.  Source crops and cached appearance live in static buffers for `max_vehicles`
+    vehicles, so `set_vehicles` replaces them in place without recapturing the step graphs.
+
+        pipe = TrajectoryPipeline(model, max_vehicles=8)
+        pipe.set_vehicles({"src": src_u8, "x_mask_u8": m_u8, "x_normal_u8": n_u8})       # (V,256,256,3) each
+        t = pipe.submit({"vehicle": veh_i32, "src_kp": ..., "dst_kp": ..., "K": ..., "E_src": ..., "E_dst": ..., "kp3d": ...,
+                         "kp3d_dst": ..., "y_normal_u8": y_u8})
+        crops = pipe.result(t)["crops"]
+    """
+    WARP_KEYS = ("src_kp", "dst_kp", "K", "E_src", "E_dst", "kp3d")
+    AR_BLOCKS = ("shape_decoder_1", "shape_decoder_2")
+
+    def __init__(self, model, max_vehicles: int, depth: int = 2, **kw):
+        super().__init__(model, depth=depth, **kw)
+        if int(max_vehicles) <= 0:
+            raise ValueError("max_vehicles must be positive")
+        self.max_vehicles = int(max_vehicles)
+        self.n_vehicles = 0
+        self.veh_src = None      # (max_vehicles,H,W,3) u8 source crops
+        self.veh_gk = None       # six (max_vehicles,h,w,512) ELU(nin_k(mu)) tensors, engine dtype: n = 0 (h = 2) k = 0..2, then n = 1 (h = 4)
+        self.veh_wkey = None     # the folded weights the cache was encoded with
+
+    def _graph_key(self, eng):
+        # the graphs read the per-vehicle buffers by address: a reallocation (other crop size / engine dtype) recaptures
+        return eng._wkey, None if self.veh_src is None else tuple(t.data_ptr() for t in [self.veh_src] + self.veh_gk)
+
+    # ------------------------------------------------------------------ per-vehicle state
+    def set_vehicles(self, batch: dict):
+        """batch: `src` (V,H,W,3) u8 source crops and the appearance input of each vehicle -- `x` (V,6,256,256) f32, or the two
+        uint8 images it is made of, `x_mask_u8` and `x_normal_u8` (V,256,256,3); host or device tensors.  Waits for every
+        batch in flight, encodes the appearance (draws enc_down's two Sampler tensors from the CPU generator, as the
+        reference does at step 0) and copies it and the source crops into the static per-vehicle buffers."""
+        src = batch.get("src")
+        if src is None or ("x" not in batch and not ("x_mask_u8" in batch and "x_normal_u8" in batch)):
+            raise ValueError("set_vehicles: needs `src` and either `x` or `x_mask_u8` + `x_normal_u8`")
+        V = int(src.shape[0])
+        if not 0 < V <= self.max_vehicles:
+            raise ValueError(f"set_vehicles: {V} vehicles, this pipeline holds 1..{self.max_vehicles}")
+        if src.dim() != 4 or src.shape[-1] != 3 or src.dtype != torch.uint8:
+            raise ValueError("set_vehicles: src must be (V,H,W,3) uint8")
+        xs = [batch[k] for k in (("x",) if "x" in batch else ("x_mask_u8", "x_normal_u8"))]
+        if any(int(t.shape[0]) != V for t in xs):
+            raise ValueError("set_vehicles: appearance inputs and src disagree on V")
+        for sl in self.slots:                                         # nothing in flight reads the buffers any more
+            if sl.done is not None:
+                sl.done.synchronize()
+        dev = self.dev
+        with torch.no_grad(), torch.cuda.device(dev):
+            eng = self.model.engine()
+            xs = [t.to(dev, non_blocking=True) for t in xs]
+            if len(xs) == 1:
+                x = xs[0].float().contiguous()
+            else:                                                     # the y it writes as well is not needed
+                x, _ = u8_to_vunet_inputs(xs[0].contiguous(), xs[1].contiguous(), xs[1].contiguous())
+            gk = eng.encode_vehicles(x)
+            shapes = [tuple(src.shape[1:])] + [tuple(t.shape[1:]) for t in gk]
+            if self.veh_src is None or [tuple(t.shape[1:]) for t in [self.veh_src] + self.veh_gk] != shapes or \
+                    self.veh_gk[0].dtype != gk[0].dtype:
+                self.veh_src = torch.zeros((self.max_vehicles,) + shapes[0], dtype=torch.uint8, device=dev)
+                self.veh_gk = [torch.zeros((self.max_vehicles,) + tuple(t.shape[1:]), dtype=t.dtype, device=dev) for t in gk]
+            self.veh_src[:V].copy_(src, non_blocking=True)
+            for buf, t in zip(self.veh_gk, gk):
+                buf[:V].copy_(t)
+            ready = torch.cuda.Event()
+            ready.record(torch.cuda.current_stream(dev))
+        for sl in self.slots:                                         # the next steps start after the new appearance is in place
+            sl.stream.wait_event(ready)
+        self.n_vehicles = V
+        self.veh_wkey = eng._wkey
+
+    # ------------------------------------------------------------------ one step of device work
+    def _compute_inner(self, inp):
+        cur = torch.cuda.current_stream(self.dev)
+        self.side_stream.wait_stream(cur)
+        with torch.cuda.stream(self.side_stream):                     # the warp branch, as in NovelViewPipeline
+            res = warp_batch(self.veh_src, *(inp[k] for k in self.WARP_KEYS), device=self.dev, kp3d_dst=inp.get("kp3d_dst"),
+                             src_index=inp["vehicle"])
+        y = inp["y"] if "y" in inp else u8_to_vunet_y(inp["y_normal_u8"])
+        B = y.shape[0]
+        with torch.no_grad(), torch.cuda.device(self.dev):
+            eng = self.model.engine()
+            keep = eng.raw_skips
+            eng.raw_skips = False                                     # skips are consumed pre-activated only
+            try:
+                out_d, skips_d = eng.dec_up(y)
+                gk = [torch.empty((B,) + tuple(t.shape[1:]), dtype=t.dtype, device=self.dev) for t in self.veh_gk]
+                gather_rows(list(zip(self.veh_gk, gk)), inp["vehicle"])    # one launch: every item's cached appearance
+                x_tilde, _, _ = eng.dec_down(out_d, skips_d, enc_gk=[gk[:3], gk[3:]])
+            finally:
+                eng.raw_skips = keep
+        crops = to_image_batch(x_tilde)
+        cur.wait_stream(self.side_stream)
+        for t in (res.warped, res.plane_j, res.vis):
+            t.record_stream(cur)
+        return {"crops": crops, "warped": res.warped, "plane_j": res.plane_j, "vis": res.vis}
+
+    # ------------------------------------------------------------------ public API
+    def submit(self, batch: dict, resident: bool = False) -> int:
+        """batch, per item: `vehicle` (B,) int32 index into the vehicles of the last set_vehicles; the warp inputs `src_kp` /
+        `dst_kp` (B,12,2) i32, `K` (B,3,3), `E_src` / `E_dst` (B,3,4), `kp3d` (B,12,3) f64 and optionally `kp3d_dst` (B,12,3)
+        (the moved keypoints, kinematics.step_keypoints_batch); `y` (B,3,256,256) f32 or `y_normal_u8` (B,256,256,3) u8.
+        The source crop is the vehicle's (set_vehicles).  Outputs as NovelViewPipeline: crops, plane_j, vis (+ warped)."""
+        if self.veh_src is None:
+            raise ValueError("TrajectoryPipeline.submit: call set_vehicles first")
+        if "src" in batch:
+            raise ValueError("TrajectoryPipeline.submit: the source crops are per vehicle (set_vehicles), not per item")
+        missing = [k for k in ("vehicle",) + self.WARP_KEYS if k not in batch]
+        if missing or ("y" in batch) == ("y_normal_u8" in batch):
+            raise ValueError(f"TrajectoryPipeline.submit: needs {missing or ''} and exactly one of `y` / `y_normal_u8`")
+        veh = batch["vehicle"]
+        veh = veh if isinstance(veh, torch.Tensor) else torch.as_tensor(veh)
+        if veh.dim() != 1 or veh.dtype.is_floating_point or veh.numel() == 0:
+            raise ValueError("TrajectoryPipeline.submit: vehicle must be a non-empty (B,) integer array")
+        lo, hi = int(veh.min()), int(veh.max())
+        if lo < 0 or hi >= self.n_vehicles:
+            raise ValueError(f"TrajectoryPipeline.submit: vehicle index {lo if lo < 0 else hi} outside [0, {self.n_vehicles})")
+        eng = self.model.engine()
+        if eng._wkey != self.veh_wkey:
+            raise ValueError("TrajectoryPipeline.submit: the weights changed since set_vehicles; call it again to re-encode")
+        if veh.dtype != torch.int32:
+            batch = dict(batch, vehicle=veh.to(torch.int32))
+        return super().submit(batch, resident)

@@ -402,15 +402,18 @@ class VunetEngine:
         z.aux["eps"] = eps
         return mu, z
 
-    def ar_block(self, path, x, skip_a, B, g_s2d_elu=None):
+    def ar_block(self, path, x, skip_a, B, g_s2d_elu=None, gk=None):
         """AutoRegressiveBlock (models.py:17-89).  g_s2d_elu: (B,h/2,w/2,512) ELU(SpaceToDepth(enc_down_mu))
-        or None.  Returns (x, mu Act with .f32, z Act with .f32 and .elu)."""
+        or None.  gk: three (B,h,w,512) tensors ELU(nin_k(g)), k = 0..2, computed beforehand (encode_vehicles): the
+        block then skips its three nin_k launches.  Returns (x, mu Act with .f32, z Act with .f32 and .elu)."""
         torch = self.torch
         x = self.residual(path + ".residual_init", x, skip_a, B=B)
         x_ = self.residual(path + ".residual_s2d", x, B=B, out_mode=S2D)
         h, w = x_.H, x_.W
-        gk = None
-        if g_s2d_elu is not None:
+        if gk is not None:
+            assert len(gk) == 3 and all(tuple(t.shape) == (B, h, w, 512) for t in gk), f"{path}: gk must be three (B,{h},{w},512) tensors"
+            gk = [Act(512, h, w, elu=t) for t in gk]
+        elif g_s2d_elu is not None:
             g = Act(512, h, w, elu=g_s2d_elu)
             gk = [self.nin(f"{path}.nin_{k}", [g.slice(128 * k, 128)], B, raw=False) for k in range(3)]
         mu = Act(128, 2 * h, 2 * w, f32=self._empty(B, 128, 2 * h, 2 * w, dtype=torch.float32))
@@ -469,6 +472,22 @@ class VunetEngine:
         mu1, z1 = self.sampler_plain("app_decoder_2_b", xf, B)
         return [mu0, mu1], [z0, z1]
 
+    def encode_vehicles(self, x_nchw):
+        """The appearance side of the trajectory loop, once per vehicle (trajectory_inference.py:230-233): enc_up, enc_down,
+        then the six nin_k convolutions of the two auto-regressive blocks on the MEANS mu (traj_test decodes with mu_app,
+        :413-426).  enc_down still draws its two Sampler tensors, (V,128,4,4) and (V,128,8,8), like the reference, although
+        z is not used.  Returns [ELU(nin_k(ELU(S2D(mu_n))))] for n = 0, 1 and k = 0..2: six (V,h,w,512) tensors, h = 2 then 4,
+        whose rows dec_down(..., enc_gk=...) takes per item."""
+        V = x_nchw.shape[0]
+        out_e, skips_e = self.enc_up(x_nchw)
+        mu, _ = self.enc_down(out_e, skips_e)
+        gk = []
+        for n, blk in enumerate(("shape_decoder_1", "shape_decoder_2")):
+            g = mu[n].aux["s2d_elu"]
+            ga = Act(512, g.shape[1], g.shape[2], elu=g)
+            gk += [self.nin(f"{blk}.nin_{k}", [ga.slice(128 * k, 128)], V, raw=False).elu for k in range(3)]
+        return gk
+
     def dec_up(self, y_nchw):
         """models.py:355-388 -> (outputs [Act], skips [14 Acts])."""
         B = y_nchw.shape[0]
@@ -484,10 +503,11 @@ class VunetEngine:
             skips += [self.nin(sk + "_b", [sl[-2]], B, raw=rs), self.nin(sk + "_c", [sl[-1]], B, raw=rs)]
         return [x], skips
 
-    def dec_down(self, outputs, skips, enc_g=()):
+    def dec_down(self, outputs, skips, enc_g=(), enc_gk=None):
         """models.py:410-459.  skips: list of 14 Acts (consumed from the end, like the reference's pop()).
         enc_g: () or two (B,h/2,w/2,512) ELU(SpaceToDepth(enc_down_mu)) tensors.
-        Returns (x_tilde fp32 NCHW tensor, [mu Acts], [z Acts])."""
+        enc_gk: None or, per auto-regressive block, the three ELU(nin_k(g)) tensors encode_vehicles returns (gathered to the
+        items); replaces enc_g.  Returns (x_tilde fp32 NCHW tensor, [mu Acts], [z Acts])."""
         torch = self.torch
         skips = list(skips)
         x0 = outputs[-1]
@@ -497,7 +517,10 @@ class VunetEngine:
         mus, zs = [], []
         for n, blk in enumerate(("shape_decoder_1", "shape_decoder_2")):
             skip_a, skip_b = skips.pop(), skips.pop()
-            x, mu_n, z_n = self.ar_block(blk, x, skip_a, B, None if len(enc_g) == 0 else enc_g[n])
+            if enc_gk is not None:
+                x, mu_n, z_n = self.ar_block(blk, x, skip_a, B, gk=enc_gk[n])
+            else:
+                x, mu_n, z_n = self.ar_block(blk, x, skip_a, B, None if len(enc_g) == 0 else enc_g[n])
             mus.append(mu_n)
             zs.append(z_n)
             x = self.nin(blk + "_n", [x, z_n], B)

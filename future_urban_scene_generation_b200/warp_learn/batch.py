@@ -47,7 +47,8 @@ def check_refused(result: "WarpResult"):
     return result
 
 
-def warp_batch(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, device=None, out=None, kp3d_dst=None, check=False) -> WarpResult:
+def warp_batch(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, device=None, out=None, kp3d_dst=None, check=False,
+               src_index=None) -> WarpResult:
     """src (B,H,W,3) u8; src_kp/dst_kp (B,12,2) i32 plane vertices (_KP_NAMES order, already
     truncated as in planes_utils.py:22-27); K (B,3,3) or (3,3); E_* (B,3,4) or (B,4,4); kp3d (B,12,3).
     numpy arrays or torch tensors on host or device.  Asynchronous on the current CUDA stream.
@@ -55,13 +56,28 @@ def warp_batch(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, device=None, out=None
     trajectory_inference.py:359-379 -- see kinematics.step_keypoints_batch); default: kp3d for both poses.
     Keypoints outside the frame are handled like cv2 does (clipped polygons).  check=True synchronises and raises
     RefusedCrops when a crop came back refused (plane_j == -2); asynchronous callers use check_refused(result)
-    once the stream is done (NovelViewPipeline.result does)."""
+    once the stream is done (NovelViewPipeline.result does).
+    src_index (B,) int32, optional: crop b warps source image src_index[b] of src (n_src,H,W,3) -- one source crop per vehicle
+    shared by all its steps (TrajectoryPipeline).  A host-side index is range-checked (ValueError); on the device an index
+    outside [0, n_src) refuses that crop (plane_j == -2, zero planes)."""
     torch = _lib.require_cuda()
     device = torch.device(device if device is not None else "cuda")
     src = _dev(torch, src, torch.uint8, src.shape, device)
-    B, H, W, ch = src.shape
+    n_src, H, W, ch = src.shape
     if ch != 3:
         raise ValueError("src must be (B,H,W,3) uint8")
+    B = n_src
+    idx = None
+    if src_index is not None:
+        it = torch.as_tensor(src_index) if not isinstance(src_index, torch.Tensor) else src_index
+        if it.dim() != 1:
+            raise ValueError("src_index must be a (B,) integer array")
+        if not it.is_cuda and it.numel() and (int(it.min()) < 0 or int(it.max()) >= n_src):
+            raise ValueError(f"src_index out of range [0, {n_src})")
+        B = int(it.shape[0])
+        if B <= 0:
+            raise ValueError("src_index is empty")
+        idx = _dev(torch, it, torch.int32, (B,), device)
 
     def _E(E):
         E = torch.as_tensor(E) if not isinstance(E, torch.Tensor) else E
@@ -88,7 +104,11 @@ def warp_batch(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, device=None, out=None
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=device)
     Xd = _dev(torch, kp3d_dst, torch.float64, (B, 12, 3), device) if kp3d_dst is not None else None
     with torch.cuda.device(device):
-        if Xd is None:
+        if idx is not None:
+            rc = L.fusg_warp_fused_idx(_lib.ptr(src), _lib.ptr(idx), n_src, _lib.ptr(skp), _lib.ptr(dkp), _lib.ptr(Kt), _lib.ptr(Es),
+                                       _lib.ptr(Ed), _lib.ptr(X), _lib.ptr(Xd), _lib.ptr(out.warped), _lib.ptr(out.vis),
+                                       _lib.ptr(out.plane_j), _lib.ptr(out.H12), _lib.ptr(ws), ws_bytes, B, H, W, _lib.stream_ptr(torch))
+        elif Xd is None:
             rc = L.fusg_warp_fused(_lib.ptr(src), _lib.ptr(skp), _lib.ptr(dkp), _lib.ptr(Kt), _lib.ptr(Es), _lib.ptr(Ed),
                                    _lib.ptr(X), _lib.ptr(out.warped), _lib.ptr(out.vis), _lib.ptr(out.plane_j),
                                    _lib.ptr(out.H12), _lib.ptr(ws), ws_bytes, B, H, W, _lib.stream_ptr(torch))
@@ -98,5 +118,5 @@ def warp_batch(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, device=None, out=None
                                         _lib.ptr(out.H12), _lib.ptr(ws), ws_bytes, B, H, W, _lib.stream_ptr(torch))
     _lib.check(rc, "fusg_warp_fused")
     # keep inputs/workspace alive until the stream has consumed them
-    out._keep = (src, skp, dkp, Kt, Es, Ed, X, Xd, ws)
+    out._keep = (src, skp, dkp, Kt, Es, Ed, X, Xd, ws, idx)
     return check_refused(out) if check else out

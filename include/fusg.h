@@ -94,6 +94,18 @@ int fusg_warp_fused_traj(const uint8_t *src, const int32_t *src_kp, const int32_
                          void *workspace, size_t workspace_bytes, int B, int H, int W, void *stream);
 
 /*
+ * The same call with source images shared between crops (the trajectory loop warps one source crop of a vehicle for every
+ * future step, trajectory_inference.py:165-174,413): src [n_src,H,W,3] u8 holds n_src images and crop b reads image
+ * src_index[b] (src_index [B] i32, device).  Every other array is per crop as above.  kp3d_dst == NULL means fusg_warp_fused,
+ * otherwise fusg_warp_fused_traj.  A crop whose index lies outside [0, n_src) is refused like a vertex beyond 2^20 px: outputs
+ * zero, plane_j = -2; no source byte is read for it.  A NULL src_index or n_src <= 0 is FUSG_ERR_ARG.  Same workspace.
+ */
+int fusg_warp_fused_idx(const uint8_t *src, const int32_t *src_index, int n_src, const int32_t *src_kp, const int32_t *dst_kp,
+                        const double *K, const double *E_src, const double *E_dst, const double *kp3d_src, const double *kp3d_dst,
+                        uint8_t *warped, uint8_t *vis, int8_t *plane_j, double *H12,
+                        void *workspace, size_t workspace_bytes, int B, int H, int W, void *stream);
+
+/*
  * Per-step keypoint kinematics of the trajectory loop (SURVEY.md section 8f-4) for N (vehicle, future step) items:
  *   moved = v @ z_rot(theta) + tr                         trajectory_inference.py:359-361, utils/geometry.py:80-113
  *   kp2d  = cv2.projectPoints(moved, rvec, tvec, K, 0)    trajectory_inference.py:363-367
@@ -303,6 +315,25 @@ int fusg_pack_icn_inputs(const uint8_t *planes, const uint8_t *normals, const ui
  * inputs [B,res,res,3] u8 -> x [B,6,res,res] f32, y [B,3,res,res] f32.  Lets a host ship 9 bytes per pixel instead of 36. */
 int fusg_u8_to_vunet_inputs(const uint8_t *mask_bbox, const uint8_t *normal_src, const uint8_t *normal_dst, float *x, float *y, int B,
                             int res, void *stream);
+/* y alone, for a step whose appearance input was encoded beforehand (the trajectory loop, trajectory_inference.py:413-426):
+ *   normal_dst [B,res,res,3] u8 -> y [B,3,res,res] f32, the same values fusg_u8_to_vunet_inputs writes to y. */
+int fusg_u8_to_vunet_y(const uint8_t *normal_dst, float *y, int B, int res, void *stream);
+/* ---- per-item gather of per-vehicle rows --------------------------------------------------------------------
+ * For every segment: dst [B,row_bytes] row b = src [n_src,row_bytes] row index[b], or zeros where index[b] is outside
+ * [0, n_src).  index [B] i32 (device).  `segs` is a HOST array of nseg <= FUSG_GATHER_MAX_SEGS entries, passed to the kernel
+ * by value (one launch, capturable in a graph).  row_bytes must be a non-zero multiple of 16 and src / dst 16-byte aligned
+ * (copies are 16-byte vectors); anything else is FUSG_ERR_ARG.  Brings a vehicle's cached appearance tensors to its items. */
+#define FUSG_GATHER_MAX_SEGS 8
+typedef struct fusg_gather_seg {
+    const void *src;
+    void *dst;
+    int64_t row_bytes;
+    int32_t n_src;
+    int32_t reserved;
+} fusg_gather_seg;
+int fusg_gather_rows(const fusg_gather_seg *segs, int nseg, const int32_t *index, int B, void *stream);
+/* sizeof(fusg_gather_seg) as this library was compiled (binding self-check). */
+size_t fusg_sizeof_gather_seg(void);
 /* ====================================================================================== */
 /* ICN generator G_Resnet (SURVEY.md section 8f-1; warp_learn/models.py:15-208): the pieces   */
 /* between its convolutions.  The convolutions themselves run on fusg_conv2d (pad_mode 1).    */
