@@ -54,9 +54,10 @@ class _Slot:
 class _GraphPipeline:
     """What NovelViewPipeline and TrajectoryPipeline share: slots of static buffers with one captured graph each, the copy /
     compute / output streams, the background Sampler-noise draw, the side-stream warp branch and the multi-GPU exchange.
-    A subclass supplies `_compute_inner(inp)`: one step of device work on the slot's input buffers."""
+    A subclass supplies the two branches of one step on the slot's input buffers: `_warp(inp)` returns the WarpResult,
+    `_decode(inp)` the VUNet output x_tilde."""
 
-    def __init__(self, model, depth: int = 2, gather_fn=None, use_graph: bool = True, shared_stream: bool = False,
+    def __init__(self, model, depth: int = 2, gather_fn=None, shared_stream: bool = False,
                  prefetch_noise: bool = True, return_warped: bool = False, micro_batches_per_step: int = 1):
         """return_warped: also copy the (B,5,256,256,3) warped planes back to the host (63 of 75 MB per 64 crops).  The
         reference never reads the planes on the host for their own sake -- they feed get_icn_inputs
@@ -70,7 +71,6 @@ class _GraphPipeline:
         self.dev = next(model.parameters()).device
         self.depth = depth
         self.gather_fn = gather_fn        # optional device-side collective on the completed crops (parallel.gather_crops)
-        self.use_graph = use_graph        # the collective (if any) is issued eagerly after the graph replay
         self.prefetch_noise = prefetch_noise
         self.return_warped = return_warped
         self.mps = max(1, int(micro_batches_per_step))
@@ -96,12 +96,22 @@ class _GraphPipeline:
     def _compute(self, inp):
         prev = _lib.lib().fusg_conv2d_set_sm_reserve(self.SM_RESERVE)      # baked into the captured launches' grids
         try:
-            return self._compute_inner(inp)
+            # the planar warp is a chain of small latency-bound kernels (visibility -> homographies -> gather) that does
+            # not feed the VUNet of the same batch: fork it onto a side stream so it fills the SMs the narrow VUNet
+            # layers leave idle, and join before the outputs are read (inside a graph this becomes a parallel branch)
+            cur = torch.cuda.current_stream(self.dev)
+            self.side_stream.wait_stream(cur)
+            with torch.cuda.stream(self.side_stream):
+                res = self._warp(inp)
+            with torch.no_grad(), torch.cuda.device(self.dev):
+                x_tilde = self._decode(inp)
+            crops = to_image_batch(x_tilde)
+            cur.wait_stream(self.side_stream)
+            for t in (res.warped, res.plane_j, res.vis):
+                t.record_stream(cur)
+            return {"crops": crops, "warped": res.warped, "plane_j": res.plane_j, "vis": res.vis}
         finally:
             _lib.lib().fusg_conv2d_set_sm_reserve(prev)
-
-    def _compute_inner(self, inp):
-        raise NotImplementedError
 
     def _graph_key(self, eng):
         """What a captured graph depends on besides its input shapes: the device pointers of the folded weights."""
@@ -111,6 +121,7 @@ class _GraphPipeline:
         """First use of a slot: allocate static buffers, run once eagerly (weight fold, function
         attributes, allocator warm-up), then capture the step into a graph."""
         eng = self.model.engine()
+        slot.wkey = None                      # until the capture below succeeds: a failed preparation is redone next time
         slot.inp = {k: torch.empty(tuple(v.shape), dtype=v.dtype, device=self.dev) for k, v in batch.items()}
         for k, v in batch.items():
             slot.inp[k].copy_(v)
@@ -119,9 +130,7 @@ class _GraphPipeline:
         def recording_provider(b, c, h, w):
             shapes.append((b, c, h, w))
             return torch.zeros((b, h, w, c), dtype=torch.float32, device=self.dev)
-        prev = eng.noise_provider
-        eng.noise_provider = recording_provider
-        with torch.cuda.stream(slot.stream):
+        with eng.noise_from(recording_provider), torch.cuda.stream(slot.stream):
             self._compute(slot.inp)                                   # eager warm-up
         slot.stream.synchronize()
         slot.noise_shapes = list(shapes)
@@ -129,17 +138,14 @@ class _GraphPipeline:
         slot.noise_nchw = [torch.zeros((b, c, h, w), dtype=torch.float32, device=self.dev) for b, c, h, w in shapes]
         slot.noise_stage = [torch.empty((b, c, h, w), dtype=torch.float32).pin_memory() for b, c, h, w in shapes]
         it = iter(slot.noise)
-        eng.noise_provider = lambda b, c, h, w: next(it)
         n0 = _lib.kernel_launches()
-        if self.use_graph:
-            slot.graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(slot.graph, stream=slot.stream):
-                self._relayout_noise(slot)
-                slot.dev_out = self._compute(slot.inp)
-            self.captures += 1
+        slot.graph = torch.cuda.CUDAGraph()
+        with eng.noise_from(lambda b, c, h, w: next(it)), torch.cuda.graph(slot.graph, stream=slot.stream):
+            self._relayout_noise(slot)
+            slot.dev_out = self._compute(slot.inp)
+        self.captures += 1
         slot.launches = _lib.kernel_launches() - n0
         slot.wkey = self._graph_key(eng)
-        eng.noise_provider = prev
 
     def _relayout_noise(self, slot: _Slot):
         """NCHW (as the reference draws it) -> NHWC (as the Sampler epilogues read it), on the device, on the current
@@ -199,8 +205,7 @@ class _GraphPipeline:
         resident=True skips the host copies (inputs / noise already in the slot; outputs stay on the device)."""
         ticket = self.n
         slot = self.slots[ticket % self.depth]
-        eng = self.model.engine()
-        eng.prepare_weights()                 # no-op unless the parameters changed (load_state_dict, .to, in-place update)
+        eng = self.model.engine()             # folds the weights again if the parameters changed (load_state_dict, .to, ...)
         # a captured graph bakes in the device pointers of the folded weights: re-capture after a reload instead of
         # replaying over freed memory
         fresh = slot.inp is None or slot.wkey != self._graph_key(eng) or set(slot.inp) != set(batch) or \
@@ -226,15 +231,7 @@ class _GraphPipeline:
             slot.copied = copied
             slot.stream.wait_event(copied)
         with torch.cuda.stream(slot.stream):
-            if slot.graph is not None:
-                slot.graph.replay()
-            else:
-                self._relayout_noise(slot)
-                it = iter(slot.noise)
-                prev = eng.noise_provider
-                eng.noise_provider = lambda b, c, h, w: next(it)
-                slot.dev_out = self._compute(slot.inp)
-                eng.noise_provider = prev
+            slot.graph.replay()
             dev_out = dict(slot.dev_out)
             if self.gather_fn is not None:
                 # the exchange step: every rank gets all completed crops ON THE DEVICE (for a device-side paste-back,
@@ -337,24 +334,15 @@ class NovelViewPipeline(_GraphPipeline):
     decoded with the sampled z) + to_image.  See submit() for the batch keys."""
     WARP_KEYS = ("src", "src_kp", "dst_kp", "K", "E_src", "E_dst", "kp3d")
 
-    def _compute_inner(self, inp):
-        # the planar warp is a chain of small latency-bound kernels (visibility -> homographies -> gather) that does
-        # not feed the VUNet of the same batch: fork it onto a side stream so it fills the SMs the narrow VUNet
-        # layers leave idle, and join before the outputs are read (inside a graph this becomes a parallel branch)
-        cur = torch.cuda.current_stream(self.dev)
-        self.side_stream.wait_stream(cur)
-        with torch.cuda.stream(self.side_stream):
-            res = warp_batch(*(inp[k] for k in self.WARP_KEYS), device=self.dev)
+    def _warp(self, inp):
+        return warp_batch(*(inp[k] for k in self.WARP_KEYS), device=self.dev)
+
+    def _decode(self, inp):
         if "x" in inp:
             x, y = inp["x"], inp["y"]
         else:                                   # uint8 form: to_tensor / flip / concat on the device (frame_ops.u8_to_vunet_inputs)
             x, y = u8_to_vunet_inputs(inp["x_mask_u8"], inp["x_normal_u8"], inp["y_normal_u8"])
-        x_tilde, _, _ = self.model(y, x)
-        crops = to_image_batch(x_tilde)
-        cur.wait_stream(self.side_stream)
-        for t in (res.warped, res.plane_j, res.vis):
-            t.record_stream(cur)
-        return {"crops": crops, "warped": res.warped, "plane_j": res.plane_j, "vis": res.vis}
+        return self.model(y, x)[0]
 
 
 class TrajectoryPipeline(_GraphPipeline):
@@ -433,30 +421,17 @@ class TrajectoryPipeline(_GraphPipeline):
         self.veh_wkey = eng._wkey
 
     # ------------------------------------------------------------------ one step of device work
-    def _compute_inner(self, inp):
-        cur = torch.cuda.current_stream(self.dev)
-        self.side_stream.wait_stream(cur)
-        with torch.cuda.stream(self.side_stream):                     # the warp branch, as in NovelViewPipeline
-            res = warp_batch(self.veh_src, *(inp[k] for k in self.WARP_KEYS), device=self.dev, kp3d_dst=inp.get("kp3d_dst"),
-                             src_index=inp["vehicle"])
+    def _warp(self, inp):
+        return warp_batch(self.veh_src, *(inp[k] for k in self.WARP_KEYS), device=self.dev, kp3d_dst=inp.get("kp3d_dst"),
+                          src_index=inp["vehicle"])
+
+    def _decode(self, inp):
         y = inp["y"] if "y" in inp else u8_to_vunet_y(inp["y_normal_u8"])
-        B = y.shape[0]
-        with torch.no_grad(), torch.cuda.device(self.dev):
-            eng = self.model.engine()
-            keep = eng.raw_skips
-            eng.raw_skips = False                                     # skips are consumed pre-activated only
-            try:
-                out_d, skips_d = eng.dec_up(y)
-                gk = [torch.empty((B,) + tuple(t.shape[1:]), dtype=t.dtype, device=self.dev) for t in self.veh_gk]
-                gather_rows(list(zip(self.veh_gk, gk)), inp["vehicle"])    # one launch: every item's cached appearance
-                x_tilde, _, _ = eng.dec_down(out_d, skips_d, enc_gk=[gk[:3], gk[3:]])
-            finally:
-                eng.raw_skips = keep
-        crops = to_image_batch(x_tilde)
-        cur.wait_stream(self.side_stream)
-        for t in (res.warped, res.plane_j, res.vis):
-            t.record_stream(cur)
-        return {"crops": crops, "warped": res.warped, "plane_j": res.plane_j, "vis": res.vis}
+        eng = self.model.engine()
+        out_d, skips_d = eng.dec_up(y, raw_skips=False)                  # skips are consumed pre-activated only
+        gk = [torch.empty((y.shape[0],) + tuple(t.shape[1:]), dtype=t.dtype, device=self.dev) for t in self.veh_gk]
+        gather_rows(list(zip(self.veh_gk, gk)), inp["vehicle"])        # one launch: every item's cached appearance
+        return eng.dec_down(out_d, skips_d, enc_gk=[gk[:3], gk[3:]])[0]
 
     # ------------------------------------------------------------------ public API
     def submit(self, batch: dict, resident: bool = False) -> int:

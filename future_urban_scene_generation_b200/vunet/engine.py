@@ -9,6 +9,7 @@ kernel's epilogue writes the activated copy once instead.
 dtype 'bf16' is the product path (tcgen05 kernels); dtype 'fp32' is the verification build
 (north_star: <=1e-4), which runs the same program on the CUDA-core direct kernel.
 """
+import contextlib
 import ctypes as C
 
 from .. import _lib
@@ -79,7 +80,6 @@ class VunetEngine:
         self.launches = 0
         self.profile = None            # list -> per-launch (path, impl, flops, start, end) CUDA-event records
         self.noise_provider = None     # callable(B,C,H,W) -> NHWC fp32 device tensor; None = CPU torch.randn (reference semantics)
-        self.raw_skips = True          # also keep raw copies of NiN skips (needed by the sub-forward API)
 
     # ------------------------------------------------------------------ plumbing
     @property
@@ -326,6 +326,16 @@ class VunetEngine:
         stage.copy_(eps.permute(0, 2, 3, 1))
         return stage.to(self.device(), non_blocking=True)
 
+    @contextlib.contextmanager
+    def noise_from(self, provider):
+        """Draws the Sampler noise from `provider` inside the block.  The engine is shared by every user of its model, so
+        the previous provider is put back however the block ends."""
+        prev, self.noise_provider = self.noise_provider, provider
+        try:
+            yield
+        finally:
+            self.noise_provider = prev
+
     # ------------------------------------------------------------------ blocks
     def residual(self, path, x, skip=None, B=None, raw=True, elu=True, out_mode=PLAIN):
         """Residual (layers.py:83-105): x + conv3x3(elu(cat[x, skip])), optionally written SpaceToDepth'ed."""
@@ -488,19 +498,19 @@ class VunetEngine:
             gk += [self.nin(f"{blk}.nin_{k}", [ga.slice(128 * k, 128)], V, raw=False).elu for k in range(3)]
         return gk
 
-    def dec_up(self, y_nchw):
-        """models.py:355-388 -> (outputs [Act], skips [14 Acts])."""
+    def dec_up(self, y_nchw, raw_skips=True):
+        """models.py:355-388 -> (outputs [Act], skips [14 Acts]).  raw_skips=False writes only the ELU copies of the NiN
+        skips, which is all dec_down reads; the sub-forward API (forward_dec_up) also returns the raw values."""
         B = y_nchw.shape[0]
         yin = self.from_nchw(y_nchw, elu_only=True, cpad=32, cphys=16)
-        rs = self.raw_skips
         skips = []
         x, sl = self.init_block("shape_encoder_1", yin, B, last_elu=True)
-        skips += [self.nin("shape_skip_1_b", [sl[-2]], B, raw=rs), self.nin("shape_skip_1_c", [sl[-1]], B, raw=rs)]
+        skips += [self.nin("shape_skip_1_b", [sl[-2]], B, raw=raw_skips), self.nin("shape_skip_1_c", [sl[-1]], B, raw=raw_skips)]
         for enc, sk in (("shape_encoder_1_a", "shape_skip_1_a"), ("shape_encoder_2", "shape_skip_2"),
                         ("shape_encoder_3", "shape_skip_3"), ("shape_encoder_4", "shape_skip_4"),
                         ("shape_encoder_5", "shape_skip_5"), ("shape_encoder_6", "shape_skip_6")):
             x, sl = self.down_block(enc, x, B, last_elu=True)
-            skips += [self.nin(sk + "_b", [sl[-2]], B, raw=rs), self.nin(sk + "_c", [sl[-1]], B, raw=rs)]
+            skips += [self.nin(sk + "_b", [sl[-2]], B, raw=raw_skips), self.nin(sk + "_c", [sl[-1]], B, raw=raw_skips)]
         return [x], skips
 
     def dec_down(self, outputs, skips, enc_g=(), enc_gk=None):

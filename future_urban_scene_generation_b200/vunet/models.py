@@ -217,37 +217,33 @@ class Vunet_fix_res(nn.Module):
         assert mean_mode in ['mean_appearance', 'mean_shape']
         with torch.no_grad(), self._dev_ctx():
             e = self.engine()
-            keep = e.raw_skips
-            e.raw_skips = False                # fused path: skips are consumed pre-activated only
-            try:
-                if mean_mode == 'mean_appearance':
-                    # the shape encoder (dec_up) does not depend on the appearance branch (enc_up -> enc_down):
-                    # run it on a forked stream so its layers fill the SMs the narrow appearance layers leave idle
-                    # (fork_branches = False keeps everything on the current stream, e.g. for per-launch timing)
-                    if getattr(self, "fork_branches", True):
-                        cur = torch.cuda.current_stream()
-                        side = self._side_stream()
-                        side.wait_stream(cur)
-                        with torch.cuda.stream(side):
-                            out_d, skips_d = e.dec_up(y_tilde)
-                        out_e, skips_e = e.enc_up(x)
-                        mu_app, z_app = e.enc_down(out_e, skips_e)
-                        cur.wait_stream(side)
-                        # the shape-encoder activations were allocated on the side stream and are consumed on `cur`:
-                        # tell the caching allocator, or another caller stream could be handed their blocks too early
-                        for a in list(out_d) + list(skips_d):
-                            e.record_stream(a, cur)
-                    else:
-                        out_e, skips_e = e.enc_up(x)
-                        mu_app, z_app = e.enc_down(out_e, skips_e)
-                        out_d, skips_d = e.dec_up(y_tilde)
-                    x_tilde, mu_shape, _ = e.dec_down(out_d, skips_d, [z.aux["s2d_elu"] for z in z_app])
-                    return x_tilde, [e.to_nchw(a) for a in mu_app], [e.to_nchw(a) for a in mu_shape]
-                out_d, skips_d = e.dec_up(y_tilde)
-                x_tilde, _, _ = e.dec_down(out_d, skips_d)
-                return x_tilde
-            finally:
-                e.raw_skips = keep
+            # raw_skips=False: the fused path consumes the skips pre-activated only
+            if mean_mode == 'mean_appearance':
+                # the shape encoder (dec_up) does not depend on the appearance branch (enc_up -> enc_down):
+                # run it on a forked stream so its layers fill the SMs the narrow appearance layers leave idle
+                # (fork_branches = False keeps everything on the current stream, e.g. for per-launch timing)
+                if getattr(self, "fork_branches", True):
+                    cur = torch.cuda.current_stream()
+                    side = self._side_stream()
+                    side.wait_stream(cur)
+                    with torch.cuda.stream(side):
+                        out_d, skips_d = e.dec_up(y_tilde, raw_skips=False)
+                    out_e, skips_e = e.enc_up(x)
+                    mu_app, z_app = e.enc_down(out_e, skips_e)
+                    cur.wait_stream(side)
+                    # the shape-encoder activations were allocated on the side stream and are consumed on `cur`:
+                    # tell the caching allocator, or another caller stream could be handed their blocks too early
+                    for a in list(out_d) + list(skips_d):
+                        e.record_stream(a, cur)
+                else:
+                    out_e, skips_e = e.enc_up(x)
+                    mu_app, z_app = e.enc_down(out_e, skips_e)
+                    out_d, skips_d = e.dec_up(y_tilde, raw_skips=False)
+                x_tilde, mu_shape, _ = e.dec_down(out_d, skips_d, [z.aux["s2d_elu"] for z in z_app])
+                return x_tilde, [e.to_nchw(a) for a in mu_app], [e.to_nchw(a) for a in mu_shape]
+            out_d, skips_d = e.dec_up(y_tilde, raw_skips=False)
+            x_tilde, _, _ = e.dec_down(out_d, skips_d)
+            return x_tilde
 
     def __call__(self, *args, **kwargs):
         return super().__call__(*args, **kwargs)

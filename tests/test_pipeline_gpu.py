@@ -115,6 +115,72 @@ def test_reloading_weights_after_capture_recaptures_the_graph(cuda):
         assert not torch.equal(a, b)
 
 
+@pytest.mark.parametrize("kind", ["novel_view", "trajectory"])
+def test_a_failed_first_submit_leaves_the_engine_as_it_found_it(cuda, monkeypatch, kind):
+    """The model's engine is shared with every eager caller: a step that raises during its first submit (here in
+    to_image_batch, after the VUNet forward drew its noise from the warm-up's zero provider) must not leave that provider
+    or the SM reserve installed, and the pipeline must prepare the slot again on the next submit."""
+    torch = cuda
+    from future_urban_scene_generation_b200 import _lib, pipeline, synth
+    from future_urban_scene_generation_b200.vunet.models import Vunet_fix_res
+    from future_urban_scene_generation_b200.warp_learn.planes_utils import to_image_batch
+    from oracle import vunet_oracle as VO
+    B = 2
+    m = Vunet_fix_res(Namespace(up_mode='subpixel', w_norm=True, drop_prob=0.2, vunet_256=True))
+    m.load_state_dict(VO.make_state_dict(0), strict=True)
+    m = m.cuda().eval()
+    wb = synth.make_warp_batch(5, B)
+    xs, ys = synth.make_vunet_inputs(5, B)
+    host = {k: torch.from_numpy(np.ascontiguousarray(v)).pin_memory() for k, v in wb.items()}
+    x, y = torch.from_numpy(xs).pin_memory(), torch.from_numpy(ys).pin_memory()
+    host["y"] = y
+    if kind == "novel_view":
+        host["x"] = x
+        pipe = pipeline.NovelViewPipeline(m, depth=1)
+        vehicles = None
+    else:
+        vehicles = {"src": host.pop("src"), "x": x}                       # vehicle b is item b
+        host["vehicle"] = torch.arange(B, dtype=torch.int32)
+        pipe = pipeline.TrajectoryPipeline(m, max_vehicles=B, depth=1)
+
+    def eager_x_tilde():
+        with torch.no_grad():
+            return m(y.cuda(), x.cuda())[0]
+
+    def eager_crops():
+        if vehicles is None:
+            return to_image_batch(eager_x_tilde()).cpu()
+        with torch.no_grad():                                            # set_vehicles, then one step, on the engine
+            e = m.engine()
+            mu, _ = e.enc_down(*e.enc_up(x.cuda()))
+            od, sd = e.dec_up(y.cuda())
+            return to_image_batch(e.dec_down(od, sd, [g.aux["s2d_elu"] for g in mu])[0]).cpu()
+
+    torch.manual_seed(4)
+    before = eager_x_tilde()
+
+    def fail(*a, **k):
+        raise RuntimeError("injected failure")
+    with monkeypatch.context() as mp:
+        mp.setattr(pipeline, "to_image_batch", fail)
+        if vehicles is not None:
+            pipe.set_vehicles(vehicles)
+        with pytest.raises(RuntimeError, match="injected failure"):
+            pipe.submit(host)
+    torch.cuda.synchronize()
+    assert m.engine().noise_provider is None
+    assert _lib.lib().fusg_conv2d_set_sm_reserve(-1) == 0
+    torch.manual_seed(4)
+    assert torch.equal(eager_x_tilde(), before)
+    torch.manual_seed(6)
+    if vehicles is not None:
+        pipe.set_vehicles(vehicles)
+    crops = pipe.result(pipe.submit(host))["crops"].clone()
+    assert pipe.captures == 1
+    torch.manual_seed(6)
+    assert torch.equal(crops, eager_crops())
+
+
 def test_noise_prefetch_keeps_generator_semantics(cuda):
     """The background noise draw is adopted only when it is bit-identical to drawing inside submit(): same outputs as
     prefetch_noise=False for one seed, also when the caller reseeds or draws from the global generator between steps."""
