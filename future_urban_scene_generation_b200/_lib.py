@@ -33,6 +33,8 @@ def _load():
         "fusg_warp_fused": ([vp] * 11 + [vp, sz, i, i, i, vp], i),
         "fusg_warp_fused_traj": ([vp] * 12 + [vp, sz, i, i, i, vp], i),
         "fusg_warp_fused_idx": ([vp, vp, i] + [vp] * 11 + [vp, sz, i, i, i, vp], i),
+        "fusg_warp_window_workspace_bytes": ([i, i, i], sz),
+        "fusg_warp_fused_window": ([vp, vp, i] + [vp] * 9 + [i] + [vp] * 4 + [vp, sz, i, i, i, vp], i),
         "fusg_step_keypoints": ([vp] * 10 + [i, i, i, vp], i),
         "fusg_visibility": ([vp] * 6 + [i, i, i, vp], i),
         "fusg_get_planes": ([vp] * 3 + [i, i, i, vp], i),
@@ -63,6 +65,7 @@ def _load():
         "fusg_sizeof_gather_seg": ([], sz),
         "fusg_mask_bbox": ([vp] * 4 + [i, i, vp], i),
         "fusg_pack_icn_inputs": ([vp] * 8 + [i, vp, vp, i, i, i, i, vp], i),
+        "fusg_pack_icn_inputs_window": ([vp] * 10 + [i, vp, vp, i, i, i, i, vp], i),
         "fusg_pack_vunet_inputs": ([vp] * 10 + [i, i, i, i, vp], i),
         "fusg_render_workspace_bytes": ([i, i, i, i], sz),
         "fusg_render_normals": ([vp] * 4 + [i, i] + [vp] * 6 + [vp, sz, i, i, i, vp], i),

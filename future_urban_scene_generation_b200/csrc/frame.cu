@@ -332,17 +332,23 @@ __device__ __forceinline__ void rgb2lab_u8(const LabTables &T, int r, int g, int
     }
 }
 
-// pixel (cy, cx) of the square crop of a full-frame image (zero in the padding)
-__device__ __forceinline__ void crop_fetch3(const uint8_t *__restrict__ img, const CropGeom &g, int Hf, int Wf, int cy, int cx, int *v) {
-    const int fy = g.ny0 + cy - g.pyb, fx = g.nx0 + cx - g.pxb;
-    if (fy < 0 || fy >= Hf || fx < 0 || fx >= Wf) { v[0] = v[1] = v[2] = 0; return; }
-    const uint8_t *p = img + ((size_t)fy * Wf + fx) * 3;
+// pixel (cy, cx) of the square crop of an image that holds the frame rectangle (rx0, ry0, rw, rh) -- the whole frame, or a
+// window of it -- zero outside it (the crop's padding, and for a window that covers the crop square clipped to the frame, only that)
+__device__ __forceinline__ void crop_fetch3(const uint8_t *__restrict__ img, const CropGeom &g, int rx0, int ry0, int rw, int rh, int cy, int cx,
+                                            int *v) {
+    const int fy = g.ny0 + cy - g.pyb - ry0, fx = g.nx0 + cx - g.pxb - rx0;
+    if (fy < 0 || fy >= rh || fx < 0 || fx >= rw) { v[0] = v[1] = v[2] = 0; return; }
+    const uint8_t *p = img + ((size_t)fy * rw + fx) * 3;
     v[0] = p[0]; v[1] = p[1]; v[2] = p[2];
 }
 
+// WINDOW: the warped planes of item b are the window win[b] = (x0, y0, w, h) of the frame, five [h,w,3] planes at planes + win_off[b]
+// (fusg_warp_fused_window's layout); otherwise planes is [B,5,Hf,Wf,3].
+template <bool WINDOW>
 __global__ void __launch_bounds__(256) k_pack_icn(const uint8_t *__restrict__ planes, const uint8_t *__restrict__ normals,
                                                   const uint8_t *__restrict__ central, const int *__restrict__ bbox, LabTables T,
-                                                  float *__restrict__ out, int Hf, int Wf, int res) {
+                                                  float *__restrict__ out, int Hf, int Wf, int res, const int32_t *__restrict__ win,
+                                                  const long long *__restrict__ win_off) {
     const int b = blockIdx.z, q = blockIdx.y;            // q: 0 normal sketch, 1 central crop, 2..6 warped plane q-2
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= res * res) return;
@@ -352,19 +358,26 @@ __global__ void __launch_bounds__(256) k_pack_icn(const uint8_t *__restrict__ pl
         const uint8_t *c = central + ((size_t)b * res * res + p) * 3;
         v[0] = c[0]; v[1] = c[1]; v[2] = c[2];
     } else {
-        const uint8_t *img = q == 0 ? normals + (size_t)b * Hf * Wf * 3 : planes + ((size_t)b * 5 + (q - 2)) * Hf * Wf * 3;
+        const uint8_t *img;
+        int rx0 = 0, ry0 = 0, rw = Wf, rh = Hf;
+        if (q == 0) img = normals + (size_t)b * Hf * Wf * 3;
+        else if (!WINDOW) img = planes + ((size_t)b * 5 + (q - 2)) * Hf * Wf * 3;
+        else {
+            rx0 = win[4 * b]; ry0 = win[4 * b + 1]; rw = win[4 * b + 2]; rh = win[4 * b + 3];
+            img = planes + win_off[b] + (size_t)(q - 2) * rh * rw * 3;
+        }
         const CropGeom g = crop_geometry(bbox + 4 * b, Hf, Wf);
         if (g.cw == 2 * res && g.ch == 2 * res) {                              // exact halving -> 2x2 box average
             int a[3], bq[3], c[3], d[3];
-            crop_fetch3(img, g, Hf, Wf, 2 * oy, 2 * ox, a); crop_fetch3(img, g, Hf, Wf, 2 * oy, 2 * ox + 1, bq);
-            crop_fetch3(img, g, Hf, Wf, 2 * oy + 1, 2 * ox, c); crop_fetch3(img, g, Hf, Wf, 2 * oy + 1, 2 * ox + 1, d);
+            crop_fetch3(img, g, rx0, ry0, rw, rh, 2 * oy, 2 * ox, a); crop_fetch3(img, g, rx0, ry0, rw, rh, 2 * oy, 2 * ox + 1, bq);
+            crop_fetch3(img, g, rx0, ry0, rw, rh, 2 * oy + 1, 2 * ox, c); crop_fetch3(img, g, rx0, ry0, rw, rh, 2 * oy + 1, 2 * ox + 1, d);
 #pragma unroll
             for (int ch = 0; ch < 3; ++ch) v[ch] = (a[ch] + bq[ch] + c[ch] + d[ch] + 2) >> 2;
         } else {
             const Tap tx = resize_tap(res, g.cw, ox, true), ty = resize_tap(res, g.ch, oy, false);
             int p00[3], p01[3], p10[3], p11[3];
-            crop_fetch3(img, g, Hf, Wf, ty.i0, tx.i0, p00); crop_fetch3(img, g, Hf, Wf, ty.i0, tx.i1, p01);
-            crop_fetch3(img, g, Hf, Wf, ty.i1, tx.i0, p10); crop_fetch3(img, g, Hf, Wf, ty.i1, tx.i1, p11);
+            crop_fetch3(img, g, rx0, ry0, rw, rh, ty.i0, tx.i0, p00); crop_fetch3(img, g, rx0, ry0, rw, rh, ty.i0, tx.i1, p01);
+            crop_fetch3(img, g, rx0, ry0, rw, rh, ty.i1, tx.i0, p10); crop_fetch3(img, g, rx0, ry0, rw, rh, ty.i1, tx.i1, p11);
 #pragma unroll
             for (int ch = 0; ch < 3; ++ch) {
                 const int s0 = p00[ch] * tx.a0 + p01[ch] * tx.a1, s1 = p10[ch] * tx.a0 + p11[ch] * tx.a1;
@@ -577,7 +590,22 @@ extern "C" int fusg_pack_icn_inputs(const uint8_t *planes, const uint8_t *normal
     if (B > 65535) return FUSG_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     LabTables T{gamma_tab, cbrt_tab, exc_keys, exc_vals, n_exc, exc_bitmap};
-    k_pack_icn<<<dim3((res * res + 255) / 256, 7, B), 256, 0, st>>>(planes, normals, central, bbox, T, out, Hf, Wf, res);
+    k_pack_icn<false><<<dim3((res * res + 255) / 256, 7, B), 256, 0, st>>>(planes, normals, central, bbox, T, out, Hf, Wf, res, nullptr, nullptr);
+    fusg_count_launch(1);
+    return fusg_check_launch();
+}
+
+extern "C" int fusg_pack_icn_inputs_window(const uint8_t *planes, const int32_t *win, const long long *win_off, const uint8_t *normals,
+                                           const uint8_t *central, const int32_t *bbox, const uint16_t *gamma_tab, const uint16_t *cbrt_tab,
+                                           const uint32_t *exc_keys, const uint16_t *exc_vals, int n_exc, const uint32_t *exc_bitmap, float *out,
+                                           int B, int Hf, int Wf, int res, void *stream) {
+    if (!planes || !win || !win_off || !normals || !central || !bbox || !gamma_tab || !cbrt_tab || !out) return FUSG_ERR_ARG;
+    if (B <= 0 || Hf <= 0 || Wf <= 0 || res <= 0 || n_exc < 0) return FUSG_ERR_ARG;
+    if (n_exc > 0 && (!exc_keys || !exc_vals)) return FUSG_ERR_ARG;
+    if (B > 65535) return FUSG_ERR_UNSUPPORTED;
+    cudaStream_t st = (cudaStream_t)stream;
+    LabTables T{gamma_tab, cbrt_tab, exc_keys, exc_vals, n_exc, exc_bitmap};
+    k_pack_icn<true><<<dim3((res * res + 255) / 256, 7, B), 256, 0, st>>>(planes, normals, central, bbox, T, out, Hf, Wf, res, win, win_off);
     fusg_count_launch(1);
     return fusg_check_launch();
 }

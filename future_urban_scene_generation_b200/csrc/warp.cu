@@ -168,17 +168,26 @@ struct PlaneRec {
     int ok;                       // 0: horizon through the polygon / absurd magnification -> bbox spans only
 };
 
+// Output window (x0, y0, w, h) of an item of fusg_warp_fused_window: non-empty, inside the H x W frame, at most max_h rows.
+__device__ __forceinline__ bool window_ok(const int32_t *win, int max_h, int H, int W) {
+    const int x0 = win[0], y0 = win[1], w = win[2], h = win[3];
+    return x0 >= 0 && y0 >= 0 && w >= 1 && h >= 1 && h <= max_h && x0 <= W - w && y0 <= H - h;
+}
+
+// WINDOW: the items also carry an output window (win [B,4]); an item whose window is not window_ok is refused.
+template <bool WINDOW>
 __global__ void __launch_bounds__(256) k_plane_gate(const int32_t *__restrict__ src_kp, const int32_t *__restrict__ dst_kp,
                                                     const uint8_t *__restrict__ vis, int8_t *__restrict__ plane_j, double *__restrict__ H12,
                                                     double *__restrict__ Minv, int *__restrict__ counters, int *__restrict__ list6,
                                                     int *__restrict__ list4, const int32_t *__restrict__ src_index, int n_src,
-                                                    int B, int H, int W) {
+                                                    const int32_t *__restrict__ win, int max_win_h, int B, int H, int W) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= B * N_TEX) return;
     const int b = t / N_TEX, i = t % N_TEX;
     const uint8_t *sv = vis + 2 * N_VIS * b, *dv = sv + N_VIS;
     bool bad = sv[0] == 0xff || dv[0] == 0xff;
     if (src_index && (src_index[b] < 0 || src_index[b] >= n_src)) bad = true;     // no source image: refused like an absurd vertex
+    if (WINDOW && !window_ok(win + 4 * b, max_win_h, H, W)) bad = true;
     const int32_t *sk = src_kp + 2 * N_KP * b, *dk = dst_kp + 2 * N_KP * b;
     for (int k = 0; k < 2 * N_KP && !bad; ++k)
         if (abs(sk[k]) > POLY_COORD_MAX || abs(dk[k]) > POLY_COORD_MAX) bad = true;
@@ -832,16 +841,27 @@ __global__ void __launch_bounds__(32 * PM_ROWS) k_plane_masks(const int32_t *__r
 
 constexpr int WF_ROWS = 8;        // output rows per CTA of k_warp_frame: one per warp
 
+// WINDOW: only the window win[b] = (x0, y0, w, h) of every output plane is produced, written window-relative at warped + win_off[b]
+// (plane j = [h, w, 3] at byte j*h*w*3): output row r is frame row y0 + r, pixel (r, c) equals frame pixel (y0 + r, x0 + c) of the
+// whole-frame output bit for bit.  The grid then covers max_win_h rows; an item whose window is not window_ok (k_plane_gate has
+// refused it) is not written at all.
+template <bool WINDOW>
 __global__ void __launch_bounds__(32 * WF_ROWS) k_warp_frame(const uint8_t *__restrict__ src, const int32_t *__restrict__ src_index,
                                                             const int32_t *__restrict__ src_kp,
                                                             const int8_t *__restrict__ plane_j, const double *__restrict__ Minv,
                                                             const uint32_t *__restrict__ masks, uint8_t *__restrict__ warped, int H, int W, int words,
-                                                            int row_smem) {
+                                                            int row_smem, const int32_t *__restrict__ win, const long long *__restrict__ win_off,
+                                                            int max_win_h) {
     // grid (ceil(H / WF_ROWS), 5, B): WF_ROWS output rows of output plane j, one warp per row (a CTA per row meant 3.2 million CTAs
     // for the 600-item 1080p clip).  Rows are assembled in shared memory and leave with 16-byte stores.
     extern __shared__ __align__(16) uint8_t s_rows[];
     const int j = blockIdx.y, b = blockIdx.z;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    int x0 = 0, y0 = 0, ww = W, wh = H;                  // the output rectangle in frame coordinates
+    if (WINDOW) {
+        if (!window_ok(win + 4 * b, max_win_h, H, W)) return;
+        x0 = win[4 * b]; y0 = win[4 * b + 1]; ww = win[4 * b + 2]; wh = win[4 * b + 3];
+    }
     __shared__ double M[9];
     __shared__ int s_i, s_bbox[4];
     if (threadIdx.x == 0) {
@@ -859,16 +879,21 @@ __global__ void __launch_bounds__(32 * WF_ROWS) k_warp_frame(const uint8_t *__re
         }
     }
     __syncthreads();
-    const int y = blockIdx.x * WF_ROWS + warp;
-    if (y >= H) return;
-    uint8_t *orow = warped + ((((size_t)b * N_TEX + j) * H + y) * W) * 3;
+    const int r = blockIdx.x * WF_ROWS + warp;
+    if (r >= wh) return;
+    const int y = y0 + r;
+    uint8_t *orow = WINDOW ? warped + win_off[b] + ((size_t)j * wh + r) * ww * 3 : warped + ((((size_t)b * N_TEX + j) * H + y) * W) * 3;
     const int i = s_i;
-    const int row_bytes = W * 3;
+    const int row_bytes = ww * 3;
     const bool vec = (row_bytes % 16 == 0) && ((reinterpret_cast<uintptr_t>(orow) & 15) == 0);   // rows of 16-byte-multiple frames stay aligned
     const int4 z4 = make_int4(0, 0, 0, 0);
     int xlo = 1, xhi = 0;
     if (i >= 0) {
-        if (lane == 0) { int bb[4] = {s_bbox[0], s_bbox[1], s_bbox[2], s_bbox[3]}; row_active_span(M, y, W, bb, xlo, xhi); }
+        if (lane == 0) {
+            int bb[4] = {s_bbox[0], s_bbox[1], s_bbox[2], s_bbox[3]};
+            row_active_span(M, y, W, bb, xlo, xhi);
+            if (WINDOW) { xlo = max(xlo, x0); xhi = min(xhi, x0 + ww - 1); }
+        }
         xlo = __shfl_sync(0xffffffffu, xlo, 0);
         xhi = __shfl_sync(0xffffffffu, xhi, 0);
     }
@@ -881,7 +906,8 @@ __global__ void __launch_bounds__(32 * WF_ROWS) k_warp_frame(const uint8_t *__re
     const uint8_t *simg = src + (size_t)(src_index ? src_index[b] : b) * H * W * 3;     // a refused index selects no plane (i < 0 above)
     const uint32_t *mk = masks + ((size_t)b * N_TEX + i) * H * words;
     const int bw = warp_block_w(H, W);
-    for (int x = lane; x < W; x += 32) {
+    for (int c = lane; c < ww; c += 32) {
+        const int x = x0 + c;
         uchar3 v = make_uchar3(0, 0, 0);
         if (x >= xlo && x <= xhi) {
             const int bx = (x / bw) * bw;
@@ -890,7 +916,7 @@ __global__ void __launch_bounds__(32 * WF_ROWS) k_warp_frame(const uint8_t *__re
             src_coord(M, rb, x - bx, X, Y);
             v = bilinear_tap4<true>(simg, mk, words, 0, H - 1, W, X, Y);
         }
-        s_row[3 * x] = v.x; s_row[3 * x + 1] = v.y; s_row[3 * x + 2] = v.z;
+        s_row[3 * c] = v.x; s_row[3 * c + 1] = v.y; s_row[3 * c + 2] = v.z;
     }
     __syncwarp();
     if (vec) {
@@ -981,6 +1007,74 @@ extern "C" int fusg_warp_perspective(const uint8_t *img, const double *Hm, uint8
     return fusg_check_launch();
 }
 
+// Workspace carve-up shared by the fused entry points (layout at warp_ws_base).
+struct WarpWs {
+    double *Minv;
+    int *counters, *list6, *list4, *big_list;
+    PlaneRec *recs;
+    uint32_t *masks;              // plane bit masks of the global-memory gather
+};
+static WarpWs warp_ws(void *workspace, int B) {
+    WarpWs w;
+    w.Minv = reinterpret_cast<double *>(workspace);
+    w.counters = reinterpret_cast<int *>(w.Minv + (size_t)B * N_TEX * 9);
+    w.list6 = w.counters + 4; w.list4 = w.list6 + 2 * (size_t)B; w.big_list = w.list4 + 3 * (size_t)B;
+    w.recs = reinterpret_cast<PlaneRec *>(w.big_list + (size_t)B);
+    w.masks = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(workspace) + ((warp_ws_base(B) + 15) & ~(size_t)15));
+    return w;
+}
+
+// The front half of every fused entry point: visibility of both poses, plane gating (win != nullptr: the window check of
+// fusg_warp_fused_window), homographies.  recs (may be NULL) receives the destination bounds k_warp_rows uses.
+static int warp_front(const int32_t *src_index, int n_src, const int32_t *src_kp, const int32_t *dst_kp, const double *K, const double *E_src,
+                      const double *E_dst, const double *kp3d, const double *kp3d_dst, const int32_t *win, int max_win_h, uint8_t *vis,
+                      int8_t *plane_j, double *H12, const WarpWs &ws, PlaneRec *recs, int B, int H, int W, cudaStream_t st) {
+    k_visibility<<<(2 * B + VIS_WARPS - 1) / VIS_WARPS, VIS_WARPS * 32, 0, st>>>(K, E_src, E_dst, kp3d, kp3d_dst, vis, nullptr, nullptr, 2 * B, H, W);
+    if (fusg_record_cuda(cudaMemsetAsync(ws.counters, 0, 4 * sizeof(int), st)) != FUSG_OK) return FUSG_ERR_CUDA;
+    if (win)
+        k_plane_gate<true><<<(B * N_TEX + 255) / 256, 256, 0, st>>>(src_kp, dst_kp, vis, plane_j, H12, ws.Minv, ws.counters, ws.list6, ws.list4,
+                                                                     src_index, n_src, win, max_win_h, B, H, W);
+    else
+        k_plane_gate<false><<<(B * N_TEX + 255) / 256, 256, 0, st>>>(src_kp, dst_kp, vis, plane_j, H12, ws.Minv, ws.counters, ws.list6, ws.list4,
+                                                                      src_index, n_src, nullptr, 0, B, H, W);
+    fusg_count_launch(2);
+    if (solver_prepare() != FUSG_OK) return FUSG_ERR_CUDA;
+    // 32 point sets per warp whatever the batch: the lanes of a warp run in lock step, so a fuller warp costs no
+    // latency, and the fewest possible SMs lose 52 KB of shared memory to a solver warp (the VUNet convolutions of the
+    // same step want all of it); the grid covers the worst case, warps beyond the task count exit at once
+    const int lanes = 32;
+    const int blocks6 = (2 * B + lanes - 1) / lanes, blocks4 = (3 * B + lanes - 1) / lanes;
+    k_solve<<<blocks6 + blocks4, 32, SOLVER_SMEM_BYTES, st>>>(src_kp, dst_kp, plane_j, H12, ws.Minv, ws.counters, ws.list6, ws.list4, recs, blocks6, lanes);
+    fusg_count_launch(1);
+    return FUSG_OK;
+}
+
+// Polygon bit masks of every warped source plane, then the global-memory gather (whole frame, or the windows when win != nullptr).
+static int warp_gather_global(const uint8_t *src, const int32_t *src_index, const int32_t *src_kp, const int8_t *plane_j, const WarpWs &ws,
+                              uint8_t *warped, const int32_t *win, const long long *win_off, int max_win_h, int B, int H, int W, cudaStream_t st) {
+    const int words = (W + 31) / 32;
+    k_plane_masks<<<dim3((H + PM_ROWS - 1) / PM_ROWS, N_TEX, B), 32 * PM_ROWS, 0, st>>>(src_kp, plane_j, ws.masks, H, W, words);
+    const size_t row_smem = ((size_t)W * 3 + 15) & ~(size_t)15;
+    const size_t frame_smem = row_smem * WF_ROWS;
+    if (frame_smem > 200 * 1024) return FUSG_ERR_UNSUPPORTED;
+    if (win) {
+        if (frame_smem > 48 * 1024 &&
+            fusg_once_per_device(4, frame_smem, [frame_smem] { return cudaFuncSetAttribute(k_warp_frame<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)frame_smem); }) != cudaSuccess)
+            return fusg_check_launch();
+        const int rows = max_win_h < H ? max_win_h : H;          // a window that passes window_ok has at most H rows
+        k_warp_frame<true><<<dim3((rows + WF_ROWS - 1) / WF_ROWS, N_TEX, B), 32 * WF_ROWS, frame_smem, st>>>(src, src_index, src_kp, plane_j, ws.Minv, ws.masks,
+                                                                                                             warped, H, W, words, (int)row_smem, win, win_off, max_win_h);
+    } else {
+        if (frame_smem > 48 * 1024 &&
+            fusg_once_per_device(2, frame_smem, [frame_smem] { return cudaFuncSetAttribute(k_warp_frame<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)frame_smem); }) != cudaSuccess)
+            return fusg_check_launch();
+        k_warp_frame<false><<<dim3((H + WF_ROWS - 1) / WF_ROWS, N_TEX, B), 32 * WF_ROWS, frame_smem, st>>>(src, src_index, src_kp, plane_j, ws.Minv, ws.masks,
+                                                                                                           warped, H, W, words, (int)row_smem, nullptr, nullptr, 0);
+    }
+    fusg_count_launch(4);
+    return FUSG_OK;
+}
+
 // src_index == nullptr: crop b reads src[b].  Otherwise src holds n_src images and crop b reads src[src_index[b]].
 static int warp_fused_impl(const uint8_t *src, const int32_t *src_index, int n_src, const int32_t *src_kp, const int32_t *dst_kp, const double *K,
                            const double *E_src, const double *E_dst, const double *kp3d, const double *kp3d_dst, uint8_t *warped, uint8_t *vis,
@@ -993,10 +1087,7 @@ static int warp_fused_impl(const uint8_t *src, const int32_t *src_index, int n_s
     const bool frame_path = H > MAX_HW || W > MAX_HW;
     if (workspace_bytes < fusg_warp_workspace_bytes_hw(B, H, W)) return FUSG_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
-    double *Minv = reinterpret_cast<double *>(workspace);
-    int *counters = reinterpret_cast<int *>(Minv + (size_t)B * N_TEX * 9);
-    int *list6 = counters + 4, *list4 = list6 + 2 * (size_t)B, *big_list = list4 + 3 * (size_t)B;
-    PlaneRec *recs = reinterpret_cast<PlaneRec *>(big_list + (size_t)B);
+    const WarpWs ws = warp_ws(workspace, B);
     if (!frame_path) {
         if (fusg_once_per_device(1, 0, [] {
                 cudaError_t e = cudaFuncSetAttribute(k_warp_rows<WIN_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)warp_smem_bytes(WIN_SMALL));
@@ -1004,10 +1095,6 @@ static int warp_fused_impl(const uint8_t *src, const int32_t *src_index, int n_s
             }) != cudaSuccess)
             return fusg_check_launch();
     }
-    k_visibility<<<(2 * B + VIS_WARPS - 1) / VIS_WARPS, VIS_WARPS * 32, 0, st>>>(K, E_src, E_dst, kp3d, kp3d_dst, vis, nullptr, nullptr, 2 * B, H, W);
-    if (fusg_record_cuda(cudaMemsetAsync(counters, 0, 4 * sizeof(int), st)) != FUSG_OK) return FUSG_ERR_CUDA;
-    k_plane_gate<<<(B * N_TEX + 255) / 256, 256, 0, st>>>(src_kp, dst_kp, vis, plane_j, H12, Minv, counters, list6, list4, src_index, n_src, B, H, W);
-    fusg_count_launch(2);
     // The zero fill of the five planes (97 % of the output bytes stay zero) rides inside k_warp_rows as TMA bulk stores issued
     // two crops ahead of the gather (see the kernel); only outputs that are not 16-byte granular are cleared by a memset.
     // (Measured alternatives, 16k crops: a fill kernel of its own costs 2.6 ms when serial; on a helper stream underneath
@@ -1019,37 +1106,48 @@ static int warp_fused_impl(const uint8_t *src, const int32_t *src_index, int n_s
         if (fusg_record_cuda(cudaMemsetAsync(warped, 0, (size_t)B * N_TEX * H * W * 3, st)) != FUSG_OK) return FUSG_ERR_CUDA;
         fusg_count_launch(1);
     }
-    {
-        if (solver_prepare() != FUSG_OK) return FUSG_ERR_CUDA;
-        // 32 point sets per warp whatever the batch: the lanes of a warp run in lock step, so a fuller warp costs no
-        // latency, and the fewest possible SMs lose 52 KB of shared memory to a solver warp (the VUNet convolutions of the
-        // same step want all of it); the grid covers the worst case, warps beyond the task count exit at once
-        const int lanes = 32;
-        const int blocks6 = (2 * B + lanes - 1) / lanes, blocks4 = (3 * B + lanes - 1) / lanes;
-        k_solve<<<blocks6 + blocks4, 32, SOLVER_SMEM_BYTES, st>>>(src_kp, dst_kp, plane_j, H12, Minv, counters, list6, list4, frame_path ? nullptr : recs, blocks6, lanes);
-        fusg_count_launch(1);
-    }
+    const int rc = warp_front(src_index, n_src, src_kp, dst_kp, K, E_src, E_dst, kp3d, kp3d_dst, nullptr, 0, vis, plane_j, H12, ws,
+                              frame_path ? nullptr : ws.recs, B, H, W, st);
+    if (rc != FUSG_OK) return rc;
     if (!frame_path) {
         // persistent: two CTAs per SM stride over the crops
         const int grid = B < 2 * fusg_num_sms() ? B : 2 * fusg_num_sms();
-        k_warp_rows<WIN_SMALL><<<grid, WARP_THREADS, warp_smem_bytes(WIN_SMALL), st>>>(src, src_index, src_kp, plane_j, Minv, recs, warped, H, W, counters + 2, big_list, 0, B, bulk_zero ? ZERO_AHEAD : 0);
+        k_warp_rows<WIN_SMALL><<<grid, WARP_THREADS, warp_smem_bytes(WIN_SMALL), st>>>(src, src_index, src_kp, plane_j, ws.Minv, ws.recs, warped, H, W, ws.counters + 2,
+                                                                                       ws.big_list, 0, B, bulk_zero ? ZERO_AHEAD : 0);
         // crops whose polygons span more than WIN_SMALL source rows (a vehicle filling the crop): full-height window
         const int bgrid = B < fusg_num_sms() ? B : fusg_num_sms();
-        k_warp_rows<MAX_HW><<<bgrid, WARP_THREADS, warp_smem_bytes(MAX_HW), st>>>(src, src_index, src_kp, plane_j, Minv, recs, warped, H, W, counters + 2, big_list, 1, B, 0);
+        k_warp_rows<MAX_HW><<<bgrid, WARP_THREADS, warp_smem_bytes(MAX_HW), st>>>(src, src_index, src_kp, plane_j, ws.Minv, ws.recs, warped, H, W, ws.counters + 2,
+                                                                                  ws.big_list, 1, B, 0);
         fusg_count_launch(2);
     } else {
-        const int words = (W + 31) / 32;
-        uint32_t *masks = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(workspace) + ((warp_ws_base(B) + 15) & ~(size_t)15));
-        k_plane_masks<<<dim3((H + PM_ROWS - 1) / PM_ROWS, N_TEX, B), 32 * PM_ROWS, 0, st>>>(src_kp, plane_j, masks, H, W, words);
-        const size_t row_smem = ((size_t)W * 3 + 15) & ~(size_t)15;
-        const size_t frame_smem = row_smem * WF_ROWS;
-        if (frame_smem > 200 * 1024) return FUSG_ERR_UNSUPPORTED;
-        if (frame_smem > 48 * 1024 &&
-            fusg_once_per_device(2, frame_smem, [frame_smem] { return cudaFuncSetAttribute(k_warp_frame, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)frame_smem); }) != cudaSuccess)
-            return fusg_check_launch();
-        k_warp_frame<<<dim3((H + WF_ROWS - 1) / WF_ROWS, N_TEX, B), 32 * WF_ROWS, frame_smem, st>>>(src, src_index, src_kp, plane_j, Minv, masks, warped, H, W, words, (int)row_smem);
-        fusg_count_launch(4);
+        const int grc = warp_gather_global(src, src_index, src_kp, plane_j, ws, warped, nullptr, nullptr, 0, B, H, W, st);
+        if (grc != FUSG_OK) return grc;
     }
+    return fusg_check_launch();
+}
+
+extern "C" size_t fusg_warp_window_workspace_bytes(int B, int H, int W) {
+    if (B <= 0 || H <= 0 || W <= 0) return 0;
+    return ((warp_ws_base(B) + 15) & ~(size_t)15) + (size_t)B * N_TEX * H * ((W + 31) / 32) * sizeof(uint32_t);
+}
+
+extern "C" int fusg_warp_fused_window(const uint8_t *src, const int32_t *src_index, int n_src, const int32_t *src_kp, const int32_t *dst_kp,
+                                      const double *K, const double *E_src, const double *E_dst, const double *kp3d_src, const double *kp3d_dst,
+                                      const int32_t *win, const long long *win_off, int max_win_h, uint8_t *warped, uint8_t *vis, int8_t *plane_j,
+                                      double *H12, void *workspace, size_t workspace_bytes, int B, int H, int W, void *stream) {
+    if (!src || !src_kp || !dst_kp || !K || !E_src || !E_dst || !kp3d_src || !win || !win_off || !warped || !vis || !plane_j || !workspace)
+        return FUSG_ERR_ARG;
+    if (B <= 0 || max_win_h <= 0) return FUSG_ERR_ARG;
+    if (src_index && n_src <= 0) return FUSG_ERR_ARG;
+    if (H < 8 || W < 8 || H > 65535 || B > 65535) return FUSG_ERR_UNSUPPORTED;
+    if (workspace_bytes < fusg_warp_window_workspace_bytes(B, H, W)) return FUSG_ERR_WORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    const WarpWs ws = warp_ws(workspace, B);
+    const int rc = warp_front(src_index, n_src, src_kp, dst_kp, K, E_src, E_dst, kp3d_src, kp3d_dst, win, max_win_h, vis, plane_j, H12, ws, nullptr,
+                              B, H, W, st);
+    if (rc != FUSG_OK) return rc;
+    const int grc = warp_gather_global(src, src_index, src_kp, plane_j, ws, warped, win, win_off, max_win_h, B, H, W, st);
+    if (grc != FUSG_OK) return grc;
     return fusg_check_launch();
 }
 

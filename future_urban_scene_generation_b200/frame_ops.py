@@ -359,38 +359,159 @@ def square_crop_info(image_hw, bbox):
             "crop_size_orig": (min(ny1, image_h + pyb + pya) - ny0, min(nx1, image_w + pxb + pxa) - nx0)}
 
 
-def get_icn_inputs_batch(planes, sketch_normals, sketch_masks, central_crops, icn_w=256, icn_h=256):
-    """`get_icn_inputs` for B vehicles at once.  planes (B,5,Hf,Wf,3) uint8 BGR (e.g. `warp_batch(...).warped` for whole
-    frames, still on the device), sketch_normals (B,Hf,Wf,3) uint8 RGB, sketch_masks (B,Hf,Wf) bool / uint8 (non-zero =
-    vehicle), central_crops (B,icn_h,icn_w,3) uint8 RGB; numpy or torch, host or device.
-    Returns (gen_in (B,21,icn_h,icn_w) float32 CUDA tensor == the reference's tensors stacked, list of B crop_info dicts)."""
-    if icn_w != icn_h:
-        raise NotImplementedError("get_icn_inputs_batch: square ICN inputs only (the reference uses 256 x 256)")
-    torch = _lib.require_cuda()
-    pl = _dev(torch, planes, torch.uint8)
-    if pl.dim() != 5 or pl.shape[1] != 5 or pl.shape[4] != 3:
-        raise ValueError("get_icn_inputs_batch: planes must be (B, 5, Hf, Wf, 3) uint8")
-    B, Hf, Wf = int(pl.shape[0]), int(pl.shape[2]), int(pl.shape[3])
-    dev = pl.device
-    nm = _dev(torch, sketch_normals, torch.uint8).to(dev)
-    ct = _dev(torch, central_crops, torch.uint8).to(dev)
+def _sketch_mask_bbox(torch, sketch_masks, B, Hf, Wf, dev, what):
+    """sketch_masks (B,Hf,Wf) -> (uint8 masks on dev, bbox (B,4) int32 on dev, the same bbox on the host) via fusg_mask_bbox.
+    Synchronises (crop_info is host data in the reference too: a few ints per vehicle)."""
     mk = sketch_masks if isinstance(sketch_masks, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(sketch_masks))
     mk = (mk != 0).to(torch.uint8).to(dev).contiguous()
-    if tuple(nm.shape) != (B, Hf, Wf, 3) or tuple(mk.shape) != (B, Hf, Wf) or tuple(ct.shape) != (B, icn_h, icn_w, 3):
-        raise ValueError("get_icn_inputs_batch: sketch_normals (B,Hf,Wf,3), sketch_masks (B,Hf,Wf), central_crops (B,res,res,3) expected")
-    L = _lib.lib()
+    if tuple(mk.shape) != (B, Hf, Wf):
+        raise ValueError(f"{what}: sketch_masks must be {(B, Hf, Wf)}, got {tuple(mk.shape)}")
     off = torch.arange(B, dtype=torch.int64, device=dev) * (Hf * Wf)
     rect = torch.tensor([[0, 0, Wf, Hf]] * B, dtype=torch.int32, device=dev)
     bbox = torch.empty((B, 4), dtype=torch.int32, device=dev)
-    _lib.check(L.fusg_mask_bbox(_lib.ptr(mk), _lib.ptr(off), _lib.ptr(rect), _lib.ptr(bbox), B, Hf * Wf, _lib.stream_ptr(torch)), "fusg_mask_bbox")
-    bb = bbox.cpu().numpy()                              # crop_info is host data in the reference too (a few ints per vehicle)
+    _lib.check(_lib.lib().fusg_mask_bbox(_lib.ptr(mk), _lib.ptr(off), _lib.ptr(rect), _lib.ptr(bbox), B, Hf * Wf, _lib.stream_ptr(torch)),
+               "fusg_mask_bbox")
+    bb = bbox.cpu().numpy()
     if (bb[:, 2] < 0).any():
-        raise ValueError("get_icn_inputs_batch: empty sketch mask (np.min of an empty array in the reference)")
+        raise ValueError(f"{what}: empty sketch mask (np.min of an empty array in the reference)")
+    return mk, bbox, bb
+
+
+def icn_window_rect(frame_hw, crop_info):
+    """(x0, y0, w, h): the frame pixels `get_icn_inputs` reads for this crop_info -- its square crop clipped to the frame (crop
+    pixel (cy, cx) is frame pixel (y_min - pad_y_before + cy, x_min - pad_x_before + cx)).  A mask one pixel thin can give a crop
+    side of 0, whose resize taps clamp to index -1, the pixel before the crop; where that pixel lies outside the frame nothing is
+    read along that axis and the window keeps one (unread) pixel at the border, so that every window is non-empty."""
+    Hf, Wf = frame_hw
+    (nx0, ny0), (pxb, pyb) = crop_info["crop_xy_min"], crop_info["pad_xy_before"]
+    ch, cw = crop_info["crop_size_orig"]
+
+    def span(n0, pad, size, limit):
+        lo = n0 - pad if size > 0 else n0 - pad - 1
+        a, b = max(lo, 0), min(lo + max(size, 1), limit)
+        if b <= a:
+            a = min(max(lo, 0), limit - 1)
+            b = a + 1
+        return a, b
+
+    x0, x1 = span(int(nx0), int(pxb), int(cw), Wf)
+    y0, y1 = span(int(ny0), int(pyb), int(ch), Hf)
+    return x0, y0, x1 - x0, y1 - y0
+
+
+class IcnWindows:
+    """Per-item frame windows of the ICN branch (`icn_windows`): what `warp_batch(..., window=)` writes and
+    `get_icn_inputs_batch` reads.
+      bbox (B,4) int32 device / bbox_host numpy: (x_min, y_min, x_max, y_max) of each sketch mask (fusg_mask_bbox)
+      crop_infos: square_crop_info of each bbox, as get_icn_inputs_batch returns them
+      rect (B,4) int32 numpy / rect_dev: (x0, y0, w, h) = icn_window_rect
+      off (B,) int64 numpy / off_dev: byte offset of item b's block, 16-byte aligned; the block holds 5 planes of h*w*3 bytes
+      nbytes: total bytes of the blocks; max_h: the tallest window; frame_hw: (Hf, Wf)."""
+
+    def __init__(self, bbox, bbox_host, crop_infos, rect, off, nbytes, frame_hw):
+        torch = _lib.require_cuda()
+        self.bbox, self.bbox_host, self.crop_infos = bbox, bbox_host, crop_infos
+        self.rect, self.off, self.nbytes, self.frame_hw = rect, off, int(nbytes), tuple(frame_hw)
+        self.max_h = int(rect[:, 3].max())
+        self.rect_dev = torch.from_numpy(rect).to(bbox.device)
+        self.off_dev = torch.from_numpy(off).to(bbox.device)
+
+    def __len__(self):
+        return int(self.rect.shape[0])
+
+
+def window_layout(rects):
+    """(B,4) (x0, y0, w, h) -> (off (B,) int64, nbytes): item b's five [h,w,3] planes at off[b], blocks 16-byte aligned."""
+    sizes = 5 * rects[:, 2].astype(np.int64) * rects[:, 3] * 3
+    off = np.zeros(len(rects), np.int64)
+    o = 0
+    for b, s in enumerate(sizes):
+        off[b] = o
+        o += (int(s) + 15) & ~15
+    return off, o
+
+
+def icn_windows(sketch_masks, frame_hw):
+    """sketch_masks (B,Hf,Wf) bool / uint8 (non-zero = vehicle, the masks get_icn_inputs_batch will be given), numpy or torch ->
+    IcnWindows: for each item, the frame window whose pixels get_icn_inputs reads.  One fusg_mask_bbox pass, synchronised to
+    the host.  An empty mask raises ValueError, as get_icn_inputs_batch does."""
+    torch = _lib.require_cuda()
+    Hf, Wf = (int(v) for v in frame_hw)
+    B = int(sketch_masks.shape[0])
+    if B == 0:
+        raise ValueError("icn_windows: no items")
+    dev = sketch_masks.device if isinstance(sketch_masks, torch.Tensor) and sketch_masks.is_cuda else torch.device("cuda")
+    _, bbox, bb = _sketch_mask_bbox(torch, sketch_masks, B, Hf, Wf, dev, "icn_windows")
+    infos = [square_crop_info((Hf, Wf), bb[b]) for b in range(B)]
+    rect = np.array([icn_window_rect((Hf, Wf), ci) for ci in infos], np.int32).reshape(B, 4)
+    off, nbytes = window_layout(rect)
+    return IcnWindows(bbox, bb, infos, rect, off, nbytes, (Hf, Wf))
+
+
+class WindowedPlanes:
+    """The five warped planes of each item, only inside its window: `warp_batch(..., window=)`'s `warped`.
+    data: flat uint8 CUDA tensor of windows.nbytes bytes; item(b) -> (5, h, w, 3) view of item b's planes (BGR)."""
+
+    def __init__(self, data, windows: IcnWindows):
+        self.data, self.windows = data, windows
+
+    @property
+    def rect(self):
+        return self.windows.rect
+
+    @property
+    def off(self):
+        return self.windows.off
+
+    def item(self, b):
+        x0, y0, w, h = (int(v) for v in self.windows.rect[b])
+        o = int(self.windows.off[b])
+        return self.data[o:o + 5 * h * w * 3].view(5, h, w, 3)
+
+
+def get_icn_inputs_batch(planes, sketch_normals, sketch_masks, central_crops, icn_w=256, icn_h=256):
+    """`get_icn_inputs` for B vehicles at once.  planes (B,5,Hf,Wf,3) uint8 BGR (e.g. `warp_batch(...).warped` for whole
+    frames, still on the device) -- or a WindowedPlanes (`warp_batch(..., window=icn_windows(sketch_masks, (Hf, Wf)))`), which
+    holds only the pixels read here and gives the same result bit for bit --, sketch_normals (B,Hf,Wf,3) uint8 RGB, sketch_masks
+    (B,Hf,Wf) bool / uint8 (non-zero = vehicle), central_crops (B,icn_h,icn_w,3) uint8 RGB; numpy or torch, host or device.
+    Returns (gen_in (B,21,icn_h,icn_w) float32 CUDA tensor == the reference's tensors stacked, list of B crop_info dicts).
+    With WindowedPlanes, masks whose bounding boxes differ from those the windows were cut for raise ValueError."""
+    if icn_w != icn_h:
+        raise NotImplementedError("get_icn_inputs_batch: square ICN inputs only (the reference uses 256 x 256)")
+    torch = _lib.require_cuda()
+    windowed = isinstance(planes, WindowedPlanes)
+    if windowed:
+        pl = planes.data
+        if pl.dtype != torch.uint8 or pl.dim() != 1 or not pl.is_cuda or pl.numel() < planes.windows.nbytes:
+            raise ValueError("get_icn_inputs_batch: WindowedPlanes.data must be a flat uint8 CUDA tensor of windows.nbytes bytes")
+        B, (Hf, Wf) = len(planes.windows), planes.windows.frame_hw
+    else:
+        pl = _dev(torch, planes, torch.uint8)
+        if pl.dim() != 5 or pl.shape[1] != 5 or pl.shape[4] != 3:
+            raise ValueError("get_icn_inputs_batch: planes must be (B, 5, Hf, Wf, 3) uint8")
+        B, Hf, Wf = int(pl.shape[0]), int(pl.shape[2]), int(pl.shape[3])
+    dev = pl.device
+    nm = _dev(torch, sketch_normals, torch.uint8).to(dev)
+    ct = _dev(torch, central_crops, torch.uint8).to(dev)
+    if tuple(nm.shape) != (B, Hf, Wf, 3) or tuple(ct.shape) != (B, icn_h, icn_w, 3):
+        raise ValueError("get_icn_inputs_batch: sketch_normals (B,Hf,Wf,3), sketch_masks (B,Hf,Wf), central_crops (B,res,res,3) expected")
+    _, bbox, bb = _sketch_mask_bbox(torch, sketch_masks, B, Hf, Wf, dev, "get_icn_inputs_batch")
+    L = _lib.lib()
     g, c, ek, ev, bm = _lab_tables(torch, dev)
     out = torch.empty((B, 21, icn_h, icn_w), dtype=torch.float32, device=dev)
-    _lib.check(L.fusg_pack_icn_inputs(_lib.ptr(pl), _lib.ptr(nm), _lib.ptr(ct), _lib.ptr(bbox), _lib.ptr(g), _lib.ptr(c), _lib.ptr(ek), _lib.ptr(ev),
-                                      int(ek.numel()), _lib.ptr(bm), _lib.ptr(out), B, Hf, Wf, icn_h, _lib.stream_ptr(torch)), "fusg_pack_icn_inputs")
-    out._keep = (pl, nm, ct, bbox)
+    if windowed:
+        w = planes.windows
+        if not np.array_equal(bb, w.bbox_host):
+            bad = np.nonzero((bb != w.bbox_host).any(1))[0]
+            raise ValueError(f"get_icn_inputs_batch: the sketch masks of items {bad[:8].tolist()} are not those the planes' windows were cut for")
+        _lib.check(L.fusg_pack_icn_inputs_window(_lib.ptr(pl), _lib.ptr(w.rect_dev), _lib.ptr(w.off_dev), _lib.ptr(nm), _lib.ptr(ct), _lib.ptr(bbox),
+                                                 _lib.ptr(g), _lib.ptr(c), _lib.ptr(ek), _lib.ptr(ev), int(ek.numel()), _lib.ptr(bm), _lib.ptr(out),
+                                                 B, Hf, Wf, icn_h, _lib.stream_ptr(torch)), "fusg_pack_icn_inputs_window")
+        out._keep = (pl, nm, ct, bbox, w.rect_dev, w.off_dev)
+    else:
+        _lib.check(L.fusg_pack_icn_inputs(_lib.ptr(pl), _lib.ptr(nm), _lib.ptr(ct), _lib.ptr(bbox), _lib.ptr(g), _lib.ptr(c), _lib.ptr(ek), _lib.ptr(ev),
+                                          int(ek.numel()), _lib.ptr(bm), _lib.ptr(out), B, Hf, Wf, icn_h, _lib.stream_ptr(torch)), "fusg_pack_icn_inputs")
+        out._keep = (pl, nm, ct, bbox)
     return out, [square_crop_info((Hf, Wf), bb[b]) for b in range(B)]
 
 

@@ -106,6 +106,25 @@ int fusg_warp_fused_idx(const uint8_t *src, const int32_t *src_index, int n_src,
                         void *workspace, size_t workspace_bytes, int B, int H, int W, void *stream);
 
 /*
+ * The same call writing only a window of each item's five planes: the pixels get_icn_inputs reads (the square crop of
+ * warp_learn/models.py:334-342 around the destination sketch mask, clipped to the frame -- trajectory_inference.py:374-391 warps the
+ * whole frame and reads only that square).  win [B,4] i32 = (x0, y0, w, h) in frame pixels, win_off [B] i64 = byte offset of item b's
+ * block in `warped`; the block holds planes j = 0..4, each [h,w,3] u8 row major, plane j at win_off[b] + j*h*w*3.  Pixel (r, c) of
+ * plane j equals warped[b, j, y0 + r, x0 + c] of fusg_warp_fused_idx (src_index != NULL) / fusg_warp_fused(_traj) bit for bit, for any
+ * frame size; every byte of every window is written (zeros where no plane writes) and nothing outside the windows.  vis, plane_j and
+ * H12 are those of the whole-frame call.  src_index may be NULL (crop b reads src[b], src [B,H,W,3]), otherwise as fusg_warp_fused_idx;
+ * kp3d_dst may be NULL (kp3d_src for both poses).  An item is refused (plane_j = -2) like there, and also when its window is empty,
+ * not inside the H x W frame or has more than max_win_h rows -- such a window is not written at all; a refused item with a valid
+ * window gets an all-zero window.  Workspace >= fusg_warp_window_workspace_bytes(B, H, W).  max_win_h <= 0 is FUSG_ERR_ARG.
+ */
+size_t fusg_warp_window_workspace_bytes(int B, int H, int W);
+int fusg_warp_fused_window(const uint8_t *src, const int32_t *src_index, int n_src, const int32_t *src_kp, const int32_t *dst_kp,
+                           const double *K, const double *E_src, const double *E_dst, const double *kp3d_src, const double *kp3d_dst,
+                           const int32_t *win, const long long *win_off, int max_win_h,
+                           uint8_t *warped, uint8_t *vis, int8_t *plane_j, double *H12,
+                           void *workspace, size_t workspace_bytes, int B, int H, int W, void *stream);
+
+/*
  * Per-step keypoint kinematics of the trajectory loop (SURVEY.md section 8f-4) for N (vehicle, future step) items:
  *   moved = v @ z_rot(theta) + tr                         trajectory_inference.py:359-361, utils/geometry.py:80-113
  *   kp2d  = cv2.projectPoints(moved, rvec, tvec, K, 0)    trajectory_inference.py:363-367
@@ -310,6 +329,14 @@ int fusg_pack_vunet_inputs(const uint8_t *frames, const int32_t *frame_idx, cons
 int fusg_pack_icn_inputs(const uint8_t *planes, const uint8_t *normals, const uint8_t *central, const int32_t *bbox,
                          const uint16_t *gamma_tab, const uint16_t *cbrt_tab, const uint32_t *exc_keys, const uint16_t *exc_vals, int n_exc,
                          const uint32_t *exc_bitmap, float *out, int B, int Hf, int Wf, int res, void *stream);
+/* The same packing with the warped planes as fusg_warp_fused_window writes them: item b's five planes are the frame window
+ * win[b] = (x0, y0, w, h) at planes + win_off[b] (plane k = [h,w,3] u8 at byte k*h*w*3).  The window must hold the square crop of
+ * bbox[b] clipped to the Hf x Wf frame (every pixel the crop reads); then out equals fusg_pack_icn_inputs on the whole-frame planes
+ * bit for bit.  Every other argument as there. */
+int fusg_pack_icn_inputs_window(const uint8_t *planes, const int32_t *win, const long long *win_off, const uint8_t *normals,
+                                const uint8_t *central, const int32_t *bbox, const uint16_t *gamma_tab, const uint16_t *cbrt_tab,
+                                const uint32_t *exc_keys, const uint16_t *exc_vals, int n_exc, const uint32_t *exc_bitmap, float *out,
+                                int B, int Hf, int Wf, int res, void *stream);
 /* The tail of the same assembly when the three 256x256 uint8 images already exist (trajectory_inference.py:221-225):
  *   x = cat(to_tensor(mask_bbox), to_tensor(normal_src[..., ::-1])), y = to_tensor(normal_dst[..., ::-1]);
  * inputs [B,res,res,3] u8 -> x [B,6,res,res] f32, y [B,3,res,res] f32.  Lets a host ship 9 bytes per pixel instead of 36. */
