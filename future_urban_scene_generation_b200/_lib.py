@@ -63,6 +63,9 @@ def _load():
         "fusg_u8_to_vunet_y": ([vp, vp, i, i, vp], i),
         "fusg_gather_rows": ([vp, i, vp, i, vp], i),
         "fusg_sizeof_gather_seg": ([], sz),
+        "fusg_randn_mt19937": ([vp, vp, i, vp], i),
+        "fusg_sizeof_randn_draw": ([], sz),
+        "fusg_mt19937_advance": ([vp, i, C.c_longlong, C.c_longlong, vp, C.POINTER(i), C.POINTER(C.c_longlong)], i),
         "fusg_mask_bbox": ([vp] * 4 + [i, i, vp], i),
         "fusg_pack_icn_inputs": ([vp] * 8 + [i, vp, vp, i, i, i, i, vp], i),
         "fusg_pack_icn_inputs_window": ([vp] * 10 + [i, vp, vp, i, i, i, i, vp], i),

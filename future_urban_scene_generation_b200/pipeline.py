@@ -15,15 +15,18 @@ reference's results at a quarter of the convolution work.
 
 The ~125 kernel launches of one step are captured once per slot into a CUDA graph (static device
 buffers) and replayed, so the host issues one launch per step instead of ~125.  Sampler noise is
-still drawn on the CPU default generator in the reference's order and shapes (vunet/layers.py:166)
--- `torch.manual_seed` reproduces the reference's outputs -- and copied into the graph's static
-noise buffers before each replay.
+drawn from the CPU default generator in the reference's order and shapes (vunet/layers.py:166) --
+`torch.manual_seed` reproduces the reference's outputs.  With noise="host" (the default) torch.randn draws it on
+the host and it is copied into the graph's static noise buffers before each replay; with noise="device" the graph
+itself generates the same numbers from the generator's 2.5 KB start state (noise.py, csrc/noise.cu).
 """
+import contextlib
 import threading
 
 import torch
 
 from . import _lib
+from . import noise as device_noise
 from .frame_ops import gather_rows, u8_to_vunet_inputs, u8_to_vunet_y
 from .warp_learn.batch import warp_batch
 from .warp_learn.planes_utils import to_image_batch
@@ -39,6 +42,7 @@ class _Slot:
         self.noise_nchw = []     # device copies of the staging buffers, NCHW as drawn; re-laid out to `noise` inside the graph
         self.noise_shapes = []   # (B,C,H,W) per draw
         self.noise_stage = []    # pinned NCHW staging buffers (one per draw): torch.randn writes straight into them
+        self.draws = None        # noise="device": the DrawPlan that generates `noise` inside the graph (no staging, no relayout)
         self.dev_out = None      # device outputs (static)
         self.out = None          # pinned host outputs
         self.done = None
@@ -58,8 +62,13 @@ class _GraphPipeline:
     `_decode(inp)` the VUNet output x_tilde."""
 
     def __init__(self, model, depth: int = 2, gather_fn=None, shared_stream: bool = False,
-                 prefetch_noise: bool = True, return_warped: bool = False, micro_batches_per_step: int = 1):
-        """return_warped: also copy the (B,5,256,256,3) warped planes back to the host (63 of 75 MB per 64 crops).  The
+                 prefetch_noise: bool = True, return_warped: bool = False, micro_batches_per_step: int = 1,
+                 noise: str = "host"):
+        """noise: where the Sampler noise is made.  "host": torch.randn on the CPU generator, drawn ahead on a worker
+        thread, uploaded and re-laid out to NHWC in the graph.  "device": the same numbers, bit for bit, generated inside
+        the captured graph (noise.py); a submit only reads the CPU generator's state and advances it past the step's draws.
+        Both leave the CPU generator in the same state and give the same outputs.
+        return_warped: also copy the (B,5,256,256,3) warped planes back to the host (63 of 75 MB per 64 crops).  The
         reference never reads the planes on the host for their own sake -- they feed get_icn_inputs
         (trajectory_inference.py:175-182), which runs on the device here -- so the default keeps them in HBM
         (`device_outputs(ticket)["warped"]`).
@@ -67,6 +76,8 @@ class _GraphPipeline:
         rank = 8 micro-batches of 64); the completed crops of a step are collected in one device buffer and `gather_fn`
         runs ONCE per step on it, on its own stream, overlapping the next step's kernels."""
         _lib.require_cuda()
+        if noise not in ("host", "device"):
+            raise ValueError(f"noise must be 'host' or 'device', got {noise!r}")
         self.model = model
         self.dev = next(model.parameters()).device
         self.depth = depth
@@ -81,6 +92,10 @@ class _GraphPipeline:
         self.copy_stream = torch.cuda.Stream(self.dev)
         self.out_stream = torch.cuda.Stream(self.dev)
         self.side_stream = torch.cuda.Stream(self.dev)
+        self.noise = noise
+        if noise == "device":
+            device_noise.ensure_checked(self.dev)      # raises rather than give other numbers than torch.randn
+            self.noise_stream = torch.cuda.Stream(self.dev)
         self.slots = [_Slot() for _ in range(depth)]
         one = torch.cuda.Stream(self.dev)
         for sl in self.slots:
@@ -135,13 +150,28 @@ class _GraphPipeline:
         slot.stream.synchronize()
         slot.noise_shapes = list(shapes)
         slot.noise = [torch.zeros((b, h, w, c), dtype=torch.float32, device=self.dev) for b, c, h, w in shapes]
-        slot.noise_nchw = [torch.zeros((b, c, h, w), dtype=torch.float32, device=self.dev) for b, c, h, w in shapes]
-        slot.noise_stage = [torch.empty((b, c, h, w), dtype=torch.float32).pin_memory() for b, c, h, w in shapes]
+        if self.noise == "device":
+            slot.draws = device_noise.DrawPlan(slot.noise, shapes, True, self.dev)
+            slot.noise_nchw, slot.noise_stage = [], []
+        else:
+            slot.draws = None
+            slot.noise_nchw = [torch.zeros((b, c, h, w), dtype=torch.float32, device=self.dev) for b, c, h, w in shapes]
+            slot.noise_stage = [torch.empty((b, c, h, w), dtype=torch.float32).pin_memory() for b, c, h, w in shapes]
         it = iter(slot.noise)
+        joined = []
+
+        def static_provider(b, c, h, w):
+            if slot.draws is not None and not joined:                 # the generation branch joins before the first Sampler
+                torch.cuda.current_stream(self.dev).wait_stream(self.noise_stream)
+                joined.append(True)
+            return next(it)
         n0 = _lib.kernel_launches()
         slot.graph = torch.cuda.CUDAGraph()
-        with eng.noise_from(lambda b, c, h, w: next(it)), torch.cuda.graph(slot.graph, stream=slot.stream):
-            self._relayout_noise(slot)
+        with eng.noise_from(static_provider), torch.cuda.graph(slot.graph, stream=slot.stream):
+            if slot.draws is not None:
+                self._fork_noise(slot)
+            else:
+                self._relayout_noise(slot)
             slot.dev_out = self._compute(slot.inp)
         self.captures += 1
         slot.launches = _lib.kernel_launches() - n0
@@ -153,6 +183,13 @@ class _GraphPipeline:
         L = _lib.lib()
         for src, dst, (b, c, h, w) in zip(slot.noise_nchw, slot.noise, slot.noise_shapes):
             _lib.check(L.fusg_nchw_to_nhwc(_lib.ptr(src), _lib.ptr(dst), b, c, h, w, c, 0, 1, _lib.stream_ptr(torch)), "fusg_nchw_to_nhwc(noise)")      # elu 0, dtype 1 = fp32
+
+    def _fork_noise(self, slot: _Slot):
+        """noise="device": the step's generation on its own branch, forked from the head of the captured step.  It needs
+        nothing but the start state, so it runs beside enc_up / dec_up and the warp until the first Sampler joins it."""
+        self.noise_stream.wait_stream(torch.cuda.current_stream(self.dev))
+        with torch.cuda.stream(self.noise_stream):
+            slot.draws.launch()
 
     def _draw_noise(self, slot: _Slot, generator=None):
         """CPU generator (default: the global one), reference order and shapes (NCHW, vunet/layers.py:166), drawn straight
@@ -183,7 +220,13 @@ class _GraphPipeline:
         slot.prefetch = (th, state0, holder)
 
     def _take_noise(self, slot: _Slot):
-        """Fill the slot's staging buffers with this step's noise (adopt the prefetched draw when it is valid)."""
+        """Fill the slot's staging buffers with this step's noise (adopt the prefetched draw when it is valid) -- or, with
+        noise="device", take the generator's start state for the graph and advance the generator past the step."""
+        if slot.draws is not None:
+            if slot.copied is not None:
+                slot.copied.synchronize()      # the previous H2D out of the pinned start state has completed
+            slot.draws.take()
+            return
         pf, slot.prefetch = slot.prefetch, None
         if pf is not None:
             th, state0, holder = pf
@@ -194,6 +237,9 @@ class _GraphPipeline:
         self._draw_noise(slot)
 
     def _upload_noise(self, slot: _Slot):
+        if slot.draws is not None:
+            slot.draws.upload()
+            return
         for buf, stage in zip(slot.noise_nchw, slot.noise_stage):
             buf.copy_(stage, non_blocking=True)
 
@@ -404,7 +450,9 @@ class TrajectoryPipeline(_GraphPipeline):
                 x = xs[0].float().contiguous()
             else:                                                     # the y it writes as well is not needed
                 x, _ = u8_to_vunet_inputs(xs[0].contiguous(), xs[1].contiguous(), xs[1].contiguous())
-            gk = eng.encode_vehicles(x)
+            # noise="device": enc_down's two Sampler tensors are made on the device too
+            with eng.noise_from(device_noise.device_provider(device=dev)) if self.noise == "device" else contextlib.nullcontext():
+                gk = eng.encode_vehicles(x)
             shapes = [tuple(src.shape[1:])] + [tuple(t.shape[1:]) for t in gk]
             if self.veh_src is None or [tuple(t.shape[1:]) for t in [self.veh_src] + self.veh_gk] != shapes or \
                     self.veh_gk[0].dtype != gk[0].dtype:

@@ -361,6 +361,28 @@ typedef struct fusg_gather_seg {
 int fusg_gather_rows(const fusg_gather_seg *segs, int nseg, const int32_t *index, int B, void *stream);
 /* sizeof(fusg_gather_seg) as this library was compiled (binding self-check). */
 size_t fusg_sizeof_gather_seg(void);
+/* ---- VUNet Sampler noise on the device (vunet/layers.py:166) --------------------------------------------------
+ * torch.randn(b, c, h, w) on torch's CPU generator, bit for bit, for each draw of `draws` in turn (DESIGN.md §4.8).
+ *   state [626] u32 (device): the generator's 624 MT19937 words, then `left` and `next` (torch's position in them);
+ *   draws: a HOST array of ndraw <= FUSG_RANDN_MAX_DRAWS entries, passed to the kernels by value (capturable in a graph);
+ *   each writes b*c*h*w fp32 normals to `out` in NCHW (nhwc = 0, as torch.randn lays them out) or NHWC (nhwc = 1, what the
+ *   Sampler epilogues read).  numel must be a multiple of 16 and >= 16 (FUSG_ERR_UNSUPPORTED otherwise: torch draws such a
+ *   tensor another way).  A position torch's generator never reaches (left outside [1, 624], next + left - 1 > 624)
+ *   fills every output with NaN.  Two launches: one CTA expands the word stream, a grid-wide pass makes the normals. */
+#define FUSG_RANDN_MAX_DRAWS 16
+typedef struct fusg_randn_draw {
+    void *out;
+    int32_t b, c, h, w;
+    int32_t nhwc;
+    int32_t reserved;
+} fusg_randn_draw;
+int fusg_randn_mt19937(const uint32_t *state, const fusg_randn_draw *draws, int ndraw, void *stream);
+/* sizeof(fusg_randn_draw) as this library was compiled (binding self-check). */
+size_t fusg_sizeof_randn_draw(void);
+/* Host only, synchronous: the generator position n words after (state_host, left, next) -- twists, no tempering, no
+ * transforms.  Sets the CPU generator to where torch.randn would leave it without waiting for the device draw. */
+int fusg_mt19937_advance(const uint32_t *state_host, int left, long long next, long long n, uint32_t *state_out_host,
+                         int *left_out_host, long long *next_out_host);
 /* ====================================================================================== */
 /* ICN generator G_Resnet (SURVEY.md section 8f-1; warp_learn/models.py:15-208): the pieces   */
 /* between its convolutions.  The convolutions themselves run on fusg_conv2d (pad_mode 1).    */
