@@ -1253,8 +1253,13 @@ __global__ void k_nchw_to_nhwc(const float *__restrict__ in, T *__restrict__ out
             if (c0 + k < C) { a = __ldg(src + (size_t)(c0 + k) * HW); if (elu) a = elu1(a); }
             v[k] = a;
         }
-        if constexpr (sizeof(T) == 2) {
+        if constexpr (std::is_same_v<T, __nv_bfloat16>) {
             *reinterpret_cast<uint4 *>(dst + c0) = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+        } else if constexpr (std::is_same_v<T, __half>) {
+            __half2 h[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) h[k] = __floats2half2_rn(v[2 * k], v[2 * k + 1]);
+            *reinterpret_cast<uint4 *>(dst + c0) = *reinterpret_cast<const uint4 *>(h);
         } else {
             *reinterpret_cast<float4 *>(dst + c0) = make_float4(v[0], v[1], v[2], v[3]);
             *reinterpret_cast<float4 *>(dst + c0 + 4) = make_float4(v[4], v[5], v[6], v[7]);
@@ -1321,9 +1326,19 @@ static bool tc_supported(const fusg_conv_desc &d, int Ho, int Wo) {
     if (d.dtype != FUSG_DTYPE_BF16 && d.dtype != FUSG_DTYPE_F16) return false;
     if (d.dtype == FUSG_DTYPE_F16) {
         // fp16 activations (the ICN row): raw NHWC outputs or NCHW fp32 slots only -- no residual, noise or ELU copy
+        // A raw NHWC fp16 slot is written by the lean epilogue only, so it must be the launch's one output: the general
+        // epilogue (epilogue16<__nv_bfloat16>) would store it as bf16.
         if (d.residual || d.noise) return false;
-        for (int s = 0; s < FUSG_CONV_MAX_OUTS; ++s)
-            if (d.outs[s].ptr && d.outs[s].layout == 0 && (d.outs[s].elu || d.outs[s].mode != FUSG_OUT_PLAIN || d.cout % 16)) return false;
+        int nouts = 0, nhwc = 0;
+        for (int s = 0; s < FUSG_CONV_MAX_OUTS; ++s) {
+            if (!d.outs[s].ptr) continue;
+            ++nouts;
+            if (d.outs[s].layout == 0) {
+                ++nhwc;
+                if (d.outs[s].elu || d.outs[s].mode != FUSG_OUT_PLAIN || d.outs[s].source || d.cout % 16) return false;
+            }
+        }
+        if (nhwc && nouts > 1) return false;
     }
     if (d.c0 % 32 != 0 || (d.in1 && d.c1 % 32 != 0)) return false;
     if (d.cout_pad % 16 != 0) return false;
@@ -1715,7 +1730,9 @@ extern "C" int fusg_fold_weightnorm(const float *v, const float *g, void *w_out,
     if (!v || !g || !w_out || cout <= 0 || cin <= 0 || cout_pad < cout || cin_pad < cin) return FUSG_ERR_ARG;
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == FUSG_DTYPE_BF16) k_fold_weightnorm<__nv_bfloat16><<<cout_pad, 256, 0, st>>>(v, g, (__nv_bfloat16 *)w_out, cout, cin, ksize, cout_pad, cin_pad);
-    else k_fold_weightnorm<float><<<cout_pad, 256, 0, st>>>(v, g, (float *)w_out, cout, cin, ksize, cout_pad, cin_pad);
+    else if (dtype == FUSG_DTYPE_F16) k_fold_weightnorm<__half><<<cout_pad, 256, 0, st>>>(v, g, (__half *)w_out, cout, cin, ksize, cout_pad, cin_pad);
+    else if (dtype == FUSG_DTYPE_F32) k_fold_weightnorm<float><<<cout_pad, 256, 0, st>>>(v, g, (float *)w_out, cout, cin, ksize, cout_pad, cin_pad);
+    else return FUSG_ERR_ARG;
     fusg_count_launch(1);
     return fusg_check_launch();
 }
@@ -1726,7 +1743,9 @@ extern "C" int fusg_fold_weightnorm_paired(const float *v, const float *g, const
     if (ksize != 1 && ksize != 3) return FUSG_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == FUSG_DTYPE_BF16) k_fold_weightnorm_paired<__nv_bfloat16><<<cout_pad, 256, 0, st>>>(v, g, bias, (__nv_bfloat16 *)w_out, bias_out, cout, cin0, cin1, ksize, cout_pad);
-    else k_fold_weightnorm_paired<float><<<cout_pad, 256, 0, st>>>(v, g, bias, (float *)w_out, bias_out, cout, cin0, cin1, ksize, cout_pad);
+    else if (dtype == FUSG_DTYPE_F16) k_fold_weightnorm_paired<__half><<<cout_pad, 256, 0, st>>>(v, g, bias, (__half *)w_out, bias_out, cout, cin0, cin1, ksize, cout_pad);
+    else if (dtype == FUSG_DTYPE_F32) k_fold_weightnorm_paired<float><<<cout_pad, 256, 0, st>>>(v, g, bias, (float *)w_out, bias_out, cout, cin0, cin1, ksize, cout_pad);
+    else return FUSG_ERR_ARG;
     fusg_count_launch(1);
     return fusg_check_launch();
 }
@@ -1741,7 +1760,9 @@ extern "C" int fusg_nchw_to_nhwc(const float *in, void *out, int B, int C, int H
     const dim3 grid((unsigned)((npix + (split ? 63 : 255)) / (split ? 64 : 256)), split ? (unsigned)(cpad / 8) : 1u);
     const unsigned threads = split ? 64 : 256;
     if (dtype == FUSG_DTYPE_BF16) k_nchw_to_nhwc<__nv_bfloat16><<<grid, threads, 0, st>>>(in, (__nv_bfloat16 *)out, C, H * W, cpad, elu, npix);
-    else k_nchw_to_nhwc<float><<<grid, threads, 0, st>>>(in, (float *)out, C, H * W, cpad, elu, npix);
+    else if (dtype == FUSG_DTYPE_F16) k_nchw_to_nhwc<__half><<<grid, threads, 0, st>>>(in, (__half *)out, C, H * W, cpad, elu, npix);
+    else if (dtype == FUSG_DTYPE_F32) k_nchw_to_nhwc<float><<<grid, threads, 0, st>>>(in, (float *)out, C, H * W, cpad, elu, npix);
+    else return FUSG_ERR_ARG;
     fusg_count_launch(1);
     return fusg_check_launch();
 }
@@ -1752,7 +1773,9 @@ extern "C" int fusg_nhwc_to_nchw(const void *in, float *out, int B, int C, int H
     const size_t total = (size_t)B * C * H * W;
     const unsigned grid = (unsigned)((total + 255) / 256);
     if (dtype == FUSG_DTYPE_BF16) k_nhwc_to_nchw<__nv_bfloat16><<<grid, 256, 0, st>>>((const __nv_bfloat16 *)in, out, C, H * W, pitch, total);
-    else k_nhwc_to_nchw<float><<<grid, 256, 0, st>>>((const float *)in, out, C, H * W, pitch, total);
+    else if (dtype == FUSG_DTYPE_F16) k_nhwc_to_nchw<__half><<<grid, 256, 0, st>>>((const __half *)in, out, C, H * W, pitch, total);
+    else if (dtype == FUSG_DTYPE_F32) k_nhwc_to_nchw<float><<<grid, 256, 0, st>>>((const float *)in, out, C, H * W, pitch, total);
+    else return FUSG_ERR_ARG;
     fusg_count_launch(1);
     return fusg_check_launch();
 }
@@ -1771,7 +1794,9 @@ extern "C" int fusg_elu(const void *in, void *out, size_t n, int dtype, void *st
     cudaStream_t st = (cudaStream_t)stream;
     const unsigned grid = (unsigned)((n + 255) / 256);
     if (dtype == FUSG_DTYPE_BF16) k_elu<__nv_bfloat16><<<grid, 256, 0, st>>>((const __nv_bfloat16 *)in, (__nv_bfloat16 *)out, n);
-    else k_elu<float><<<grid, 256, 0, st>>>((const float *)in, (float *)out, n);
+    else if (dtype == FUSG_DTYPE_F16) k_elu<__half><<<grid, 256, 0, st>>>((const __half *)in, (__half *)out, n);
+    else if (dtype == FUSG_DTYPE_F32) k_elu<float><<<grid, 256, 0, st>>>((const float *)in, (float *)out, n);
+    else return FUSG_ERR_ARG;
     fusg_count_launch(1);
     return fusg_check_launch();
 }
