@@ -67,6 +67,7 @@ def _load():
         "fusg_sizeof_randn_draw": ([], sz),
         "fusg_mt19937_advance": ([vp, i, C.c_longlong, C.c_longlong, vp, C.POINTER(i), C.POINTER(C.c_longlong)], i),
         "fusg_mask_bbox": ([vp] * 4 + [i, i, vp], i),
+        "fusg_crop_geometry": ([vp, vp, i, i, i, C.c_longlong, i, vp, vp, vp, vp, vp], i),
         "fusg_pack_icn_inputs": ([vp] * 8 + [i, vp, vp, i, i, i, i, vp], i),
         "fusg_pack_icn_inputs_window": ([vp] * 10 + [i, vp, vp, i, i, i, i, vp], i),
         "fusg_pack_vunet_inputs": ([vp] * 10 + [i, i, i, i, vp], i),

@@ -80,13 +80,15 @@ __global__ void __launch_bounds__(256) k_resize_u8(const uint8_t *__restrict__ s
 
 constexpr int PASTE_INFO = 9;   // frame, h_orig, w_orig, pad_x0, pad_y0, pad_x1, pad_y1, x_min, y_min
 
-// owner[frame][y][x] = highest item index whose mask covers the pixel (-1: nobody)
+// owner[frame][y][x] = highest item index whose mask covers the pixel (-1: nobody).  An item whose frame index is outside [0, F) --
+// possible when the info comes from device data (fusg_crop_geometry's frame_index) that the host never range-checked -- pastes nothing.
 __global__ void __launch_bounds__(256) k_paste_owner(const uint8_t *__restrict__ masks, const long long *__restrict__ mask_off,
                                                      const int *__restrict__ mask_rect, const int *__restrict__ info,
-                                                     int *__restrict__ owner, int Hf, int Wf) {
+                                                     int *__restrict__ owner, int F, int Hf, int Wf) {
     const int b = blockIdx.y;
     const int x0 = mask_rect[4 * b], y0 = mask_rect[4 * b + 1], w = mask_rect[4 * b + 2], h = mask_rect[4 * b + 3];
     const int frame = info[PASTE_INFO * b];
+    if (frame < 0 || frame >= F) return;
     const uint8_t *m = masks + mask_off[b];
     int *own = owner + (size_t)frame * Hf * Wf;
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < (long long)w * h; p += (long long)gridDim.x * blockDim.x) {
@@ -149,28 +151,106 @@ __global__ void k_bbox_init(int *__restrict__ bbox, int B) {
     if (b < B) { bbox[4 * b] = 0x7fffffff; bbox[4 * b + 1] = 0x7fffffff; bbox[4 * b + 2] = -1; bbox[4 * b + 3] = -1; }
 }
 
-struct CropGeom { int nx0, ny0, pxb, pyb, cw, ch; };
+struct CropGeom { int nx0, ny0, pxb, pyb, pxa, pya, cw, ch; };
 
-// utils/crop_utils.py:14-50 for dataset='pascal' (Python float = double, int() truncates toward zero)
+// utils/crop_utils.py:14-50 for dataset='pascal' (Python float = double, int() truncates toward zero -- also for the values in
+// (-1, 0), which give 0).  Each fp64 operation rounds on its own, as in the interpreter.
 __device__ __forceinline__ CropGeom crop_geometry(const int *bb, int image_h, int image_w) {
     const int x_min = bb[0], y_min = bb[1], side_x = bb[2] - bb[0], side_y = bb[3] - bb[1];
-    const double major = (double)max(side_x, side_y) * 1.1;
-    const double cx = (double)x_min + (double)side_x / 2.0, cy = (double)y_min + (double)side_y / 2.0;
+    const double major = __dmul_rn((double)max(side_x, side_y), 1.1), half = __ddiv_rn(major, 2.0);
+    const double cx = __dadd_rn((double)x_min, __ddiv_rn((double)side_x, 2.0)), cy = __dadd_rn((double)y_min, __ddiv_rn((double)side_y, 2.0));
     CropGeom g;
-    g.pxb = g.pyb = 0;
-    g.nx0 = (int)(cx - major / 2.0);
+    g.pxb = g.pyb = g.pxa = g.pya = 0;
+    g.nx0 = (int)__dsub_rn(cx, half);
     if (g.nx0 < 0) { g.pxb = -g.nx0; g.nx0 = 0; }
-    int nx1 = (int)(cx + major / 2.0) + g.pxb;
-    int pxa = 0;
-    if (nx1 > image_w) { pxa = nx1 - image_w; nx1 = image_w + pxa; }
-    g.ny0 = (int)(cy - major / 2.0);
+    int nx1 = (int)__dadd_rn(cx, half) + g.pxb;
+    if (nx1 > image_w) { g.pxa = nx1 - image_w; nx1 = image_w + g.pxa; }
+    g.ny0 = (int)__dsub_rn(cy, half);
     if (g.ny0 < 0) { g.pyb = -g.ny0; g.ny0 = 0; }
-    int ny1 = (int)(cy + major / 2.0) + g.pyb;
-    int pya = 0;
-    if (ny1 > image_h) { pya = ny1 - image_h; ny1 = image_h + pya; }
-    g.cw = min(nx1, image_w + g.pxb + pxa) - g.nx0;
-    g.ch = min(ny1, image_h + g.pyb + pya) - g.ny0;
+    int ny1 = (int)__dadd_rn(cy, half) + g.pyb;
+    if (ny1 > image_h) { g.pya = ny1 - image_h; ny1 = image_h + g.pya; }
+    g.cw = min(nx1, image_w + g.pxb + g.pxa) - g.nx0;
+    g.ch = min(ny1, image_h + g.pyb + g.pya) - g.ny0;
     return g;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Crop geometry of a batch of sketch masks on the device (fusg_crop_geometry): from fusg_mask_bbox's output, what the kernels
+// downstream read -- paste info (frame_ops.pack_crop_info of square_crop_info), the ICN window (icn_window_rect) and its byte
+// offset (window_layout: exclusive scan of 16-byte-aligned five-plane blocks, in item order) -- plus a status per item.
+// B is a few thousand at most, so one CTA walks the items in chunks with a block-wide scan and a running carry.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int GEOM_THREADS = 1024;
+
+// icn_window_rect along one axis: the frame span [a, a+n) the resize taps of a crop side of `size` read (size 0 reads index -1)
+__device__ __forceinline__ void window_span(int n0, int pad, int size, int limit, int &a, int &n) {
+    const int lo = size > 0 ? n0 - pad : n0 - pad - 1;
+    a = max(lo, 0);
+    int e = min(lo + max(size, 1), limit);
+    if (e <= a) { a = min(max(lo, 0), limit - 1); e = a + 1; }
+    n = e - a;
+}
+
+__global__ void __launch_bounds__(GEOM_THREADS) k_crop_geometry(const int32_t *__restrict__ bbox, const int32_t *__restrict__ frame_index, int B,
+                                                                int Hf, int Wf, long long capacity, int max_win_h, int32_t *__restrict__ info,
+                                                                int32_t *__restrict__ win, long long *__restrict__ win_off,
+                                                                int8_t *__restrict__ status) {
+    __shared__ long long s_warp[GEOM_THREADS / 32];
+    __shared__ long long s_carry;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    if (threadIdx.x == 0) s_carry = 0;
+    for (int base = 0; base < B; base += GEOM_THREADS) {
+        const int b = base + threadIdx.x;
+        int st = 0, in[PASTE_INFO] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, wx = 0, wy = 0, ww = 0, wh = 0;
+        long long bytes = 0;
+        if (b < B) {
+            in[0] = frame_index ? frame_index[b] : 0;
+            if (bbox[4 * b + 2] < 0) {
+                st = 1;                                                      // empty mask: fusg_mask_bbox's (INT_MAX, INT_MAX, -1, -1)
+            } else {
+                const CropGeom g = crop_geometry(bbox + 4 * b, Hf, Wf);
+                in[1] = g.ch; in[2] = g.cw; in[3] = g.pxb; in[4] = g.pyb; in[5] = g.pxa; in[6] = g.pya; in[7] = g.nx0; in[8] = g.ny0;
+                window_span(g.nx0, g.pxb, g.cw, Wf, wx, ww);
+                window_span(g.ny0, g.pyb, g.ch, Hf, wy, wh);
+                bytes = ((5LL * ww * wh * 3) + 15) & ~15LL;
+            }
+        }
+        long long v = bytes;                                                 // inclusive scan of the block sizes
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const long long n = __shfl_up_sync(0xffffffffu, v, o);
+            if (lane >= o) v += n;
+        }
+        __syncthreads();                                                     // s_warp / s_carry of the previous chunk consumed
+        if (lane == 31) s_warp[wid] = v;
+        __syncthreads();
+        if (wid == 0) {
+            long long w = s_warp[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const long long n = __shfl_up_sync(0xffffffffu, w, o);
+                if (lane >= o) w += n;
+            }
+            s_warp[lane] = w;
+        }
+        __syncthreads();
+        const long long end = s_carry + (wid ? s_warp[wid - 1] : 0) + v, off = end - bytes;
+        if (b < B) {
+            // the offsets only grow: the first block that ends past the capacity refuses itself and every later item
+            if (st == 0 && capacity > 0 && (end > capacity || wh > max_win_h)) st = 2;
+            int32_t *io = info + (size_t)PASTE_INFO * b;
+#pragma unroll
+            for (int k = 0; k < PASTE_INFO; ++k) io[k] = in[k];
+            if (win) {
+                const bool ok = st == 0;
+                win[4 * b] = ok ? wx : 0; win[4 * b + 1] = ok ? wy : 0; win[4 * b + 2] = ok ? ww : 0; win[4 * b + 3] = ok ? wh : 0;
+            }
+            if (win_off) win_off[b] = off;
+            status[b] = (int8_t)st;
+        }
+        __syncthreads();
+        if (threadIdx.x == GEOM_THREADS - 1) s_carry = end;
+    }
 }
 
 struct Px9 { uint8_t m[3], ns[3], nd[3]; };
@@ -204,6 +284,15 @@ __global__ void __launch_bounds__(256) k_pack_inputs(const uint8_t *__restrict__
     const int b = blockIdx.y;
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= res * res) return;
+    const size_t plane = (size_t)res * res;
+    float *xb = x + (size_t)b * 6 * plane + p, *yb = y + (size_t)b * 3 * plane + p;
+    if (frame_idx[b] < 0) {                                                     // a refused item: zero rows
+#pragma unroll
+        for (int ch = 0; ch < 6; ++ch) xb[ch * plane] = 0.f;
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) yb[ch * plane] = 0.f;
+        return;
+    }
     const int oy = p / res, ox = p - oy * res;
     const CropGeom g = crop_geometry(bbox + 4 * b, Hf, Wf);
     const uint8_t *frame = frames + (size_t)frame_idx[b] * Hf * Wf * 3;
@@ -238,8 +327,6 @@ __global__ void __launch_bounds__(256) k_pack_inputs(const uint8_t *__restrict__
         }
     }
     if (vs[0] == 0 && vs[1] == 0 && vs[2] == 0) vm[0] = vm[1] = vm[2] = 255;      // trajectory_inference.py:219-220
-    const size_t plane = (size_t)res * res;
-    float *xb = x + (size_t)b * 6 * plane + p, *yb = y + (size_t)b * 3 * plane + p;
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) {
         xb[ch * plane] = to_tensor1(vm[ch]);                  // x_1: masked frame crop, channel order kept
@@ -352,6 +439,13 @@ __global__ void __launch_bounds__(256) k_pack_icn(const uint8_t *__restrict__ pl
     const int b = blockIdx.z, q = blockIdx.y;            // q: 0 normal sketch, 1 central crop, 2..6 warped plane q-2
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= res * res) return;
+    const size_t plane = (size_t)res * res;
+    float *o = out + ((size_t)b * 21 + q * 3) * plane + p;
+    if (WINDOW && (win[4 * b + 2] < 1 || win[4 * b + 3] < 1)) {     // no window (an item fusg_crop_geometry refused): a zero row
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) o[ch * plane] = 0.f;
+        return;
+    }
     const int oy = p / res, ox = p - oy * res;
     int v[3];
     if (q == 1) {
@@ -388,8 +482,6 @@ __global__ void __launch_bounds__(256) k_pack_icn(const uint8_t *__restrict__ pl
     int lab[3];
     if (q >= 2) rgb2lab_u8(T, v[2], v[1], v[0], lab);    // planes are BGR (COLOR_BGR2LAB, planes_utils.py:88)
     else rgb2lab_u8(T, v[0], v[1], v[2], lab);           // sketches are RGB (COLOR_RGB2LAB, models.py:355,358)
-    const size_t plane = (size_t)res * res;
-    float *o = out + ((size_t)b * 21 + q * 3) * plane + p;
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) o[ch * plane] = ((float)lab[ch] / 255.f - 0.5f) / 0.5f;
 }
@@ -485,6 +577,16 @@ extern "C" int fusg_mask_bbox(const uint8_t *masks, const long long *mask_off, c
     return fusg_check_launch();
 }
 
+extern "C" int fusg_crop_geometry(const int32_t *bbox, const int32_t *frame_index, int B, int Hf, int Wf, long long window_capacity_bytes,
+                                  int max_win_h, int32_t *info, int32_t *win, long long *win_off, int8_t *status, void *stream) {
+    if (!bbox || !info || !status || B <= 0 || Hf <= 0 || Wf <= 0 || window_capacity_bytes < 0) return FUSG_ERR_ARG;
+    if (window_capacity_bytes > 0 && (!win || !win_off || max_win_h <= 0)) return FUSG_ERR_ARG;
+    k_crop_geometry<<<1, GEOM_THREADS, 0, (cudaStream_t)stream>>>(bbox, frame_index, B, Hf, Wf, window_capacity_bytes, max_win_h, info, win,
+                                                                win_off, status);
+    fusg_count_launch(1);
+    return fusg_check_launch();
+}
+
 extern "C" int fusg_pack_vunet_inputs(const uint8_t *frames, const int32_t *frame_idx, const uint8_t *masks, const uint8_t *normal_src,
                                       const uint8_t *normal_dst, const long long *off, const int32_t *rect, const int32_t *bbox, float *x,
                                       float *y, int B, int Hf, int Wf, int res, void *stream) {
@@ -524,7 +626,7 @@ extern "C" int fusg_paste_back(uint8_t *frames, const uint8_t *crops, const uint
     if (fusg_record_cuda(cudaMemsetAsync(owner, 0xFF, (size_t)F * Hf * Wf * sizeof(int), st)) != FUSG_OK) return FUSG_ERR_CUDA;
     int gx = (max_mask_pixels + 255) / 256;
     if (gx > 8192) gx = 8192;
-    k_paste_owner<<<dim3(gx, B), 256, 0, st>>>(masks, mask_off, mask_rect, info, owner, Hf, Wf);
+    k_paste_owner<<<dim3(gx, B), 256, 0, st>>>(masks, mask_off, mask_rect, info, owner, F, Hf, Wf);
     int gf = (int)(((long long)Hf * Wf + 255) / 256);
     if (gf > 16384) gf = 16384;
     k_paste_apply<<<dim3(gf, F), 256, 0, st>>>(frames, crops, info, owner, Hf, Wf, S);

@@ -92,6 +92,22 @@ class PastePlan:
         self.masks, self.off, self.rect, self.info = masks, off, rect, info
         self.max_mask_pixels, self.B, self.frame_hw = max_mask_pixels, B, frame_hw
 
+    @classmethod
+    def from_geometry(cls, geometry, vehicle_masks):
+        """The plan of `geometry`'s items (crop_geometry): item b pastes into frame geometry.frame_index[b] inside
+        vehicle_masks[b] ((B, Hf, Wf) bool / uint8, non-zero = vehicle).  Built with device ops only (capturable); an item with a
+        non-zero status pastes nothing, so its frame pixels stay as they were.  Frame indices are not range-checked here."""
+        torch = _lib.require_cuda()
+        B, (Hf, Wf) = len(geometry), geometry.frame_hw
+        if tuple(vehicle_masks.shape) != (B, Hf, Wf):
+            raise ValueError(f"paste_back: vehicle_masks are {tuple(vehicle_masks.shape)}, expected {(B, Hf, Wf)}")
+        dev = geometry.info.device
+        mk = vehicle_masks if isinstance(vehicle_masks, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(vehicle_masks))
+        mk = (mk.view(torch.uint8) if mk.dtype == torch.bool else (mk != 0).to(torch.uint8)).to(dev).contiguous().reshape(-1)
+        off, rect = _full_frame_rects(torch, B, Hf, Wf, dev)
+        rect = rect * (geometry.status == 0).to(torch.int32).view(B, 1)      # a refused item covers no pixel
+        return cls(mk, off, rect, geometry.info, Hf * Wf, B, (Hf, Wf))
+
 
 def prepare_paste(masks, crop_infos, frame_index, frame_hw, n_frames, mask_rects=None):
     torch = _lib.require_cuda()
@@ -178,21 +194,37 @@ def paste_back(img_output, net_image, crop_info, dst_sketch_mask):
 # ---------------------------------------------------------------------------------------------------------------
 # VUNet input packing (SURVEY.md 8f-3): trajectory_inference.py:205-227 / :414-421 on the device
 # ---------------------------------------------------------------------------------------------------------------
-def pack_vunet_inputs_batch(frames, frame_index, src_sketch_masks, src_sketch_normals, dst_sketch_normals, rects=None, res=256):
+def pack_vunet_inputs_batch(frames, frame_index, src_sketch_masks, src_sketch_normals, dst_sketch_normals, rects=None, res=256,
+                            geometry=None):
     """frames: (F, Hf, Wf, 3) uint8; per item b: `src_sketch_masks[b]` bool (True = background, as the reference holds it
     at that point), `src_sketch_normals[b]` / `dst_sketch_normals[b]` uint8 (h, w, 3) -- full-frame arrays, or sub-rectangles
     `rects[b] = (x, y, w, h)` outside of which the item is background.  Returns CUDA tensors
-    (x (B,6,res,res) f32, y_tilde (B,3,res,res) f32, bbox (B,4) int32) == the reference's `x`, `y_tilde` stacked."""
+    (x (B,6,res,res) f32, y_tilde (B,3,res,res) f32, bbox (B,4) int32) == the reference's `x`, `y_tilde` stacked.
+    geometry (crop_geometry of the same vehicle masks, optional): the bboxes come from it -- no bbox pass, no synchronisation; the
+    inputs must then be stacked full-frame tensors and frame_index a (B,) int32 CUDA tensor: the frame of `frames` each item is cut
+    from (not the geometry's frame_index, which says where the item is pasted).  An item with a non-zero status, or whose frame
+    index is outside [0, F), gets zero x and y rows -- the range is checked on the device, so the call stays capturable."""
     torch = _lib.require_cuda()
     fr = _dev(torch, frames, torch.uint8)
     if fr.dim() != 4 or fr.shape[3] != 3:
         raise ValueError("pack_vunet_inputs_batch: frames must be (F, Hf, Wf, 3) uint8")
     F, Hf, Wf = int(fr.shape[0]), int(fr.shape[1]), int(fr.shape[2])
-    B = len(frame_index)
+    if geometry is not None:
+        B = len(geometry)
+        if geometry.frame_hw != (Hf, Wf) or rects is not None:
+            raise ValueError(f"pack_vunet_inputs_batch: the geometry is for full {geometry.frame_hw} frames, the frames are {(Hf, Wf)}")
+        if not (isinstance(frame_index, torch.Tensor) and frame_index.is_cuda and frame_index.dtype == torch.int32
+                and tuple(frame_index.shape) == (B,)):
+            raise ValueError("pack_vunet_inputs_batch: with a geometry, frame_index is a (B,) int32 CUDA tensor of source frames")
+    else:
+        B = len(frame_index)
     if B == 0 or not (len(src_sketch_masks) == len(src_sketch_normals) == len(dst_sketch_normals) == B):
         raise ValueError("pack_vunet_inputs_batch: one mask and two normal sketches per item")
-    if any(f < 0 or f >= F for f in frame_index):
+    if geometry is None and any(f < 0 or f >= F for f in frame_index):
         raise ValueError("pack_vunet_inputs_batch: frame index out of range")
+    if geometry is not None and not all(isinstance(a, torch.Tensor) and a.dim() == d
+                                        for a, d in ((src_sketch_masks, 3), (src_sketch_normals, 4), (dst_sketch_normals, 4))):
+        raise ValueError("pack_vunet_inputs_batch: with a geometry, the masks and normal sketches are stacked (B,Hf,Wf[,3]) tensors")
     if rects is None and all(isinstance(a, torch.Tensor) and a.dim() == d for a, d in ((src_sketch_masks, 3), (src_sketch_normals, 4), (dst_sketch_normals, 4))):
         # stacked full-frame tensors (B, Hf, Wf[, 3]), e.g. already on the device: no per-item work on the host
         if tuple(src_sketch_masks.shape) != (B, Hf, Wf) or tuple(src_sketch_normals.shape) != (B, Hf, Wf, 3) or tuple(dst_sketch_normals.shape) != (B, Hf, Wf, 3):
@@ -201,6 +233,9 @@ def pack_vunet_inputs_batch(frames, frame_index, src_sketch_masks, src_sketch_no
         masks = (src_sketch_masks == 0).to(torch.uint8).to(dev).contiguous().reshape(-1)
         nsrc = _dev(torch, src_sketch_normals, torch.uint8).to(dev).reshape(-1)
         ndst = _dev(torch, dst_sketch_normals, torch.uint8).to(dev).reshape(-1)
+        if geometry is not None:
+            t_off, t_rect = _full_frame_rects(torch, B, Hf, Wf, dev)
+            return _pack_vunet_launch(torch, fr, frame_index, masks, nsrc, ndst, t_off, t_rect, Hf * Wf, B, Hf, Wf, res, geometry)
         t_off = torch.arange(B, dtype=torch.int64, device=dev) * (Hf * Wf)
         t_rect = torch.tensor([0, 0, Wf, Hf], dtype=torch.int32, device=dev).repeat(B, 1)
         return _pack_vunet_launch(torch, fr, frame_index, masks, nsrc, ndst, t_off, t_rect, Hf * Wf, B, Hf, Wf, res)
@@ -234,14 +269,19 @@ def pack_vunet_inputs_batch(frames, frame_index, src_sketch_masks, src_sketch_no
     return _pack_vunet_launch(torch, fr, frame_index, masks, nsrc, ndst, t_off, t_rect, int((rect[:, 2].astype(np.int64) * rect[:, 3]).max()), B, Hf, Wf, res)
 
 
-def _pack_vunet_launch(torch, fr, frame_index, masks, nsrc, ndst, t_off, t_rect, mx, B, Hf, Wf, res):
+def _pack_vunet_launch(torch, fr, frame_index, masks, nsrc, ndst, t_off, t_rect, mx, B, Hf, Wf, res, geometry=None):
     dev = fr.device
-    t_fidx = torch.tensor(list(frame_index), dtype=torch.int32, device=dev)
-    bbox = torch.empty((B, 4), dtype=torch.int32, device=dev)
     L = _lib.lib()
-    _lib.check(L.fusg_mask_bbox(_lib.ptr(masks), _lib.ptr(t_off), _lib.ptr(t_rect), _lib.ptr(bbox), B, mx, _lib.stream_ptr(torch)), "fusg_mask_bbox")
-    if bool((bbox[:, 2] < 0).any()):
-        raise ValueError("pack_vunet_inputs_batch: empty vehicle mask (np.min of an empty array in the reference)")
+    if geometry is not None:
+        ok = (geometry.status == 0) & (frame_index >= 0) & (frame_index < int(fr.shape[0]))
+        t_fidx = torch.where(ok, frame_index, -1).to(torch.int32)           # a negative frame index: the kernel writes zero rows
+        bbox = geometry.bbox
+    else:
+        t_fidx = torch.tensor(list(frame_index), dtype=torch.int32, device=dev)
+        bbox = torch.empty((B, 4), dtype=torch.int32, device=dev)
+        _lib.check(L.fusg_mask_bbox(_lib.ptr(masks), _lib.ptr(t_off), _lib.ptr(t_rect), _lib.ptr(bbox), B, mx, _lib.stream_ptr(torch)), "fusg_mask_bbox")
+        if bool((bbox[:, 2] < 0).any()):
+            raise ValueError("pack_vunet_inputs_batch: empty vehicle mask (np.min of an empty array in the reference)")
     x = torch.empty((B, 6, res, res), dtype=torch.float32, device=dev)
     y = torch.empty((B, 3, res, res), dtype=torch.float32, device=dev)
     _lib.check(L.fusg_pack_vunet_inputs(_lib.ptr(fr), _lib.ptr(t_fidx), _lib.ptr(masks), _lib.ptr(nsrc), _lib.ptr(ndst), _lib.ptr(t_off),
@@ -359,18 +399,29 @@ def square_crop_info(image_hw, bbox):
             "crop_size_orig": (min(ny1, image_h + pyb + pya) - ny0, min(nx1, image_w + pxb + pxa) - nx0)}
 
 
-def _sketch_mask_bbox(torch, sketch_masks, B, Hf, Wf, dev, what):
-    """sketch_masks (B,Hf,Wf) -> (uint8 masks on dev, bbox (B,4) int32 on dev, the same bbox on the host) via fusg_mask_bbox.
-    Synchronises (crop_info is host data in the reference too: a few ints per vehicle)."""
+def _full_frame_rects(torch, B, Hf, Wf, dev):
+    """(off (B,) int64 = b * Hf * Wf, rect (B,4) int32 = (0, 0, Wf, Hf)): B stacked full-frame masks, made by device fills (no copy)."""
+    rect = torch.zeros((B, 4), dtype=torch.int32, device=dev)
+    rect[:, 2], rect[:, 3] = Wf, Hf
+    return torch.arange(B, dtype=torch.int64, device=dev) * (Hf * Wf), rect
+
+
+def _mask_bbox(torch, sketch_masks, B, Hf, Wf, dev, what):
+    """sketch_masks (B,Hf,Wf) -> (uint8 masks on dev, bbox (B,4) int32 on dev) via fusg_mask_bbox, without synchronising."""
     mk = sketch_masks if isinstance(sketch_masks, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(sketch_masks))
-    mk = (mk != 0).to(torch.uint8).to(dev).contiguous()
+    mk = (mk.view(torch.uint8) if mk.dtype == torch.bool else (mk != 0).to(torch.uint8)).to(dev).contiguous()   # k_mask_bbox tests != 0
     if tuple(mk.shape) != (B, Hf, Wf):
         raise ValueError(f"{what}: sketch_masks must be {(B, Hf, Wf)}, got {tuple(mk.shape)}")
-    off = torch.arange(B, dtype=torch.int64, device=dev) * (Hf * Wf)
-    rect = torch.tensor([[0, 0, Wf, Hf]] * B, dtype=torch.int32, device=dev)
+    off, rect = _full_frame_rects(torch, B, Hf, Wf, dev)
     bbox = torch.empty((B, 4), dtype=torch.int32, device=dev)
     _lib.check(_lib.lib().fusg_mask_bbox(_lib.ptr(mk), _lib.ptr(off), _lib.ptr(rect), _lib.ptr(bbox), B, Hf * Wf, _lib.stream_ptr(torch)),
                "fusg_mask_bbox")
+    return mk, bbox
+
+
+def _sketch_mask_bbox(torch, sketch_masks, B, Hf, Wf, dev, what):
+    """_mask_bbox plus the bbox on the host.  Synchronises (crop_info is host data in the reference too: a few ints per vehicle)."""
+    mk, bbox = _mask_bbox(torch, sketch_masks, B, Hf, Wf, dev, what)
     bb = bbox.cpu().numpy()
     if (bb[:, 2] < 0).any():
         raise ValueError(f"{what}: empty sketch mask (np.min of an empty array in the reference)")
@@ -419,6 +470,10 @@ class IcnWindows:
     def __len__(self):
         return int(self.rect.shape[0])
 
+    def window(self, b):
+        """(x0, y0, w, h, off) of item b."""
+        return tuple(int(v) for v in self.rect[b]) + (int(self.off[b]),)
+
 
 def window_layout(rects):
     """(B,4) (x0, y0, w, h) -> (off (B,) int64, nbytes): item b's five [h,w,3] planes at off[b], blocks 16-byte aligned."""
@@ -448,9 +503,87 @@ def icn_windows(sketch_masks, frame_hw):
     return IcnWindows(bbox, bb, infos, rect, off, nbytes, (Hf, Wf))
 
 
+class CropGeometry:
+    """The crop geometry of a batch of sketch masks, computed on the device by `crop_geometry` (fusg_mask_bbox + fusg_crop_geometry):
+      bbox (B,4) int32: (x_min, y_min, x_max, y_max) of each mask, (INT_MAX, INT_MAX, -1, -1) when it is empty
+      info (B,9) int32: fusg_paste_back's info == pack_crop_info(square_crop_info(bbox), frame_index)
+      win (B,4) int32 / win_off (B,) int64: icn_window_rect / window_layout (None without a window capacity)
+      status (B,) int8: 0 ok, 1 empty mask, 2 the window does not fit the capacity (see fusg.h); refused items get win (0, 0, 0, 0)
+      frame_index (B,) int32 or None (frame 0), all on the device; capacity_bytes, max_win_h, frame_hw: the host ints chosen by the caller.
+    It also offers IcnWindows' interface (rect_dev, off_dev, nbytes, max_h, rect, off), so that warp_batch(..., window=) and
+    WindowedPlanes take it in place of icn_windows; rect / off copy the device arrays to the host (they synchronise)."""
+
+    def __init__(self, bbox, info, win, win_off, status, frame_index, capacity_bytes, max_win_h, frame_hw):
+        self.bbox, self.info, self.win, self.win_off, self.status, self.frame_index = bbox, info, win, win_off, status, frame_index
+        self.capacity_bytes, self.max_win_h, self.frame_hw = int(capacity_bytes), int(max_win_h), tuple(frame_hw)
+
+    def __len__(self):
+        return int(self.status.shape[0])
+
+    rect_dev = property(lambda self: self.win)
+    off_dev = property(lambda self: self.win_off)
+    nbytes = property(lambda self: self.capacity_bytes)
+    max_h = property(lambda self: self.max_win_h)
+    rect = property(lambda self: self.win.cpu().numpy())
+    off = property(lambda self: self.win_off.cpu().numpy())
+
+    def window(self, b):
+        """(x0, y0, w, h, off) of item b: one small device-to-host copy (not cached: a graph replay rewrites the device arrays)."""
+        torch = _lib.require_cuda()
+        return tuple(int(v) for v in torch.cat([self.win[b].to(torch.int64), self.win_off[b:b + 1]]).tolist())
+
+    def crop_infos(self):
+        """Synchronises; the crop_info dicts get_icn_inputs_batch returns for the same masks (None for an empty mask)."""
+        info, st = self.info.cpu().numpy(), self.status.cpu().numpy()
+        return [None if st[b] == 1 else {"crop_xy_min": (int(i[7]), int(i[8])), "pad_xy_before": (int(i[3]), int(i[4])),
+                                          "pad_xy_after": (int(i[5]), int(i[6])), "crop_size_orig": (int(i[1]), int(i[2]))}
+                for b, i in enumerate(info)]
+
+    def check(self):
+        """Synchronises; raises ValueError for empty masks and warp_learn.RefusedCrops for windows that do not fit the capacity."""
+        from .warp_learn.batch import RefusedCrops
+        st = self.status.cpu().numpy()
+        empty = np.nonzero(st == 1)[0].tolist()
+        if empty:
+            raise ValueError(f"crop_geometry: empty sketch mask (np.min of an empty array in the reference): items {empty[:8]}")
+        refused = np.nonzero(st == 2)[0].tolist()
+        if refused:
+            raise RefusedCrops(refused, reason="crop geometry refused {n} window(s) (past the capacity or taller than max_win_h)")
+        return self
+
+
+def crop_geometry(vehicle_masks, frame_hw, frame_index=None, window_capacity=None):
+    """vehicle_masks (B,Hf,Wf) bool / uint8 (non-zero = vehicle), numpy or torch -> CropGeometry, with one fusg_mask_bbox pass and one
+    fusg_crop_geometry launch: no synchronisation and, for device masks, no host-to-device copy -- capturable in a CUDA graph.
+    frame_index: (B,) int32 CUDA tensor (the frame each item is pasted into) or None (frame 0).  window_capacity (bytes, rows):
+    the window buffer warp_batch(..., window=) writes -- its size and the tallest window it serves; needed for windowed warping.
+    Fixed per graph, sized by the caller; items past it get status 2.  Nothing is checked on the host: see CropGeometry.check."""
+    torch = _lib.require_cuda()
+    Hf, Wf = (int(v) for v in frame_hw)
+    B = int(vehicle_masks.shape[0])
+    if B == 0:
+        raise ValueError("crop_geometry: no items")
+    dev = vehicle_masks.device if isinstance(vehicle_masks, torch.Tensor) and vehicle_masks.is_cuda else torch.device("cuda")
+    if frame_index is not None and not (isinstance(frame_index, torch.Tensor) and frame_index.is_cuda and frame_index.dtype == torch.int32
+                                        and tuple(frame_index.shape) == (B,) and frame_index.is_contiguous()):
+        raise ValueError("crop_geometry: frame_index must be a contiguous (B,) int32 CUDA tensor")
+    cap, rows = (0, 0) if window_capacity is None else (int(v) for v in window_capacity)
+    if window_capacity is not None and (cap <= 0 or rows <= 0):
+        raise ValueError("crop_geometry: window_capacity is (bytes, rows), both positive")
+    _, bbox = _mask_bbox(torch, vehicle_masks, B, Hf, Wf, dev, "crop_geometry")
+    info = torch.empty((B, INFO_FIELDS), dtype=torch.int32, device=dev)
+    status = torch.empty((B,), dtype=torch.int8, device=dev)
+    win = torch.empty((B, 4), dtype=torch.int32, device=dev) if cap else None
+    win_off = torch.empty((B,), dtype=torch.int64, device=dev) if cap else None
+    _lib.check(_lib.lib().fusg_crop_geometry(_lib.ptr(bbox), _lib.ptr(frame_index), B, Hf, Wf, cap, rows, _lib.ptr(info), _lib.ptr(win),
+                                             _lib.ptr(win_off), _lib.ptr(status), _lib.stream_ptr(torch)), "fusg_crop_geometry")
+    return CropGeometry(bbox, info, win, win_off, status, frame_index, cap, rows, (Hf, Wf))
+
+
 class WindowedPlanes:
     """The five warped planes of each item, only inside its window: `warp_batch(..., window=)`'s `warped`.
-    data: flat uint8 CUDA tensor of windows.nbytes bytes; item(b) -> (5, h, w, 3) view of item b's planes (BGR)."""
+    data: flat uint8 CUDA tensor of windows.nbytes bytes; item(b) -> (5, h, w, 3) view of item b's planes (BGR).
+    windows: the IcnWindows or CropGeometry the planes were warped for."""
 
     def __init__(self, data, windows: IcnWindows):
         self.data, self.windows = data, windows
@@ -464,21 +597,25 @@ class WindowedPlanes:
         return self.windows.off
 
     def item(self, b):
-        x0, y0, w, h = (int(v) for v in self.windows.rect[b])
-        o = int(self.windows.off[b])
+        x0, y0, w, h, o = self.windows.window(b)
         return self.data[o:o + 5 * h * w * 3].view(5, h, w, 3)
 
 
-def get_icn_inputs_batch(planes, sketch_normals, sketch_masks, central_crops, icn_w=256, icn_h=256):
+def get_icn_inputs_batch(planes, sketch_normals, sketch_masks, central_crops, icn_w=256, icn_h=256, geometry=None):
     """`get_icn_inputs` for B vehicles at once.  planes (B,5,Hf,Wf,3) uint8 BGR (e.g. `warp_batch(...).warped` for whole
     frames, still on the device) -- or a WindowedPlanes (`warp_batch(..., window=icn_windows(sketch_masks, (Hf, Wf)))`), which
     holds only the pixels read here and gives the same result bit for bit --, sketch_normals (B,Hf,Wf,3) uint8 RGB, sketch_masks
     (B,Hf,Wf) bool / uint8 (non-zero = vehicle), central_crops (B,icn_h,icn_w,3) uint8 RGB; numpy or torch, host or device.
     Returns (gen_in (B,21,icn_h,icn_w) float32 CUDA tensor == the reference's tensors stacked, list of B crop_info dicts).
-    With WindowedPlanes, masks whose bounding boxes differ from those the windows were cut for raise ValueError."""
+    With WindowedPlanes, masks whose bounding boxes differ from those the windows were cut for raise ValueError.
+    geometry (crop_geometry of the sketch masks, optional; sketch_masks is then not read, pass None): the crops come from it -- no bbox
+    pass, no synchronisation -- and the call returns (gen_in, geometry).  planes are whole frames or warp_batch(..., window=geometry)'s
+    WindowedPlanes; an item with a non-zero status gets an all-zero gen_in row (its window, never written, is not read)."""
     if icn_w != icn_h:
         raise NotImplementedError("get_icn_inputs_batch: square ICN inputs only (the reference uses 256 x 256)")
     torch = _lib.require_cuda()
+    if geometry is not None:
+        return _icn_inputs_from_geometry(torch, planes, sketch_normals, central_crops, icn_h, geometry)
     windowed = isinstance(planes, WindowedPlanes)
     if windowed:
         pl = planes.data
@@ -513,6 +650,33 @@ def get_icn_inputs_batch(planes, sketch_normals, sketch_masks, central_crops, ic
                                           int(ek.numel()), _lib.ptr(bm), _lib.ptr(out), B, Hf, Wf, icn_h, _lib.stream_ptr(torch)), "fusg_pack_icn_inputs")
         out._keep = (pl, nm, ct, bbox)
     return out, [square_crop_info((Hf, Wf), bb[b]) for b in range(B)]
+
+
+def _icn_inputs_from_geometry(torch, planes, sketch_normals, central_crops, res, g):
+    B, (Hf, Wf) = len(g), g.frame_hw
+    if isinstance(planes, WindowedPlanes):
+        if planes.windows is not g:
+            raise ValueError("get_icn_inputs_batch: the planes were warped for other windows than the geometry's")
+        pl, win, win_off = planes.data, g.win, g.win_off
+    else:
+        pl = _dev(torch, planes, torch.uint8)
+        if tuple(pl.shape) != (B, 5, Hf, Wf, 3):
+            raise ValueError(f"get_icn_inputs_batch: planes must be {(B, 5, Hf, Wf, 3)} uint8 for this geometry")
+        # whole frames are windows too: item b's window is its frame at b * 5*Hf*Wf*3, empty where the geometry refused the item
+        win_off, win = _full_frame_rects(torch, B, Hf, Wf, pl.device)
+        win, win_off = win * (g.status == 0).to(torch.int32).view(B, 1), win_off * 15
+    dev = pl.device
+    nm = _dev(torch, sketch_normals, torch.uint8).to(dev)
+    ct = _dev(torch, central_crops, torch.uint8).to(dev)
+    if tuple(nm.shape) != (B, Hf, Wf, 3) or tuple(ct.shape) != (B, res, res, 3):
+        raise ValueError("get_icn_inputs_batch: sketch_normals (B,Hf,Wf,3), central_crops (B,res,res,3) expected")
+    gt, c, ek, ev, bm = _lab_tables(torch, dev)
+    out = torch.empty((B, 21, res, res), dtype=torch.float32, device=dev)
+    _lib.check(_lib.lib().fusg_pack_icn_inputs_window(_lib.ptr(pl), _lib.ptr(win), _lib.ptr(win_off), _lib.ptr(nm), _lib.ptr(ct), _lib.ptr(g.bbox),
+                                                      _lib.ptr(gt), _lib.ptr(c), _lib.ptr(ek), _lib.ptr(ev), int(ek.numel()), _lib.ptr(bm),
+                                                      _lib.ptr(out), B, Hf, Wf, res, _lib.stream_ptr(torch)), "fusg_pack_icn_inputs_window")
+    out._keep = (pl, nm, ct, win, win_off)
+    return out, g
 
 
 def get_icn_inputs(planes, sketch_normal, sketch_mask, central_crop, icn_w, icn_h):

@@ -32,8 +32,8 @@ class RefusedCrops(ValueError):
     """Raised when the kernels refused crops (plane_j == -2): a plane vertex or projected keypoint lies beyond
     2^20 pixels, where neither cv2's int32 polygon rasteriser nor the 16.16 edge arithmetic is defined."""
 
-    def __init__(self, indices):
-        super().__init__(f"fused warp refused {len(indices)} crop(s) (vertex magnitude > 2^20 px): {indices[:8]}")
+    def __init__(self, indices, reason="fused warp refused {n} crop(s) (vertex magnitude > 2^20 px)"):
+        super().__init__(f"{reason.format(n=len(indices))}: {indices[:8]}")
         self.indices = indices
 
 
@@ -63,7 +63,10 @@ def warp_batch(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, device=None, out=None
     window (frame_ops.IcnWindows, optional): write only each item's ICN crop window (`frame_ops.icn_windows` of the destination
     sketch masks): `warped` is then a frame_ops.WindowedPlanes whose item(b) equals the whole-frame warped[b] cropped to the window
     bit for bit (vis / plane_j / H12 unchanged), for any frame size.  Made for whole frames, where the ICN reads a small square of
-    each plane; get_icn_inputs_batch takes it in place of the (B,5,H,W,3) planes."""
+    each plane; get_icn_inputs_batch takes it in place of the (B,5,H,W,3) planes.
+    window may also be a frame_ops.CropGeometry built with a window_capacity: the windows then stay on the device, `warped` spans
+    capacity_bytes bytes, the kernel runs with max_win_h, and an item the geometry refused is refused here (plane_j == -2, none of
+    its bytes written) -- no host round trip, so the call can be captured in a CUDA graph."""
     torch = _lib.require_cuda()
     device = torch.device(device if device is not None else "cuda")
     src = _dev(torch, src, torch.uint8, src.shape, device)
@@ -100,6 +103,8 @@ def warp_batch(src, src_kp, dst_kp, K, E_src, E_dst, kp3d, device=None, out=None
     if window is not None:
         if len(window) != B or window.frame_hw != (H, W):
             raise ValueError(f"warp_batch: the windows are for {len(window)} items on {window.frame_hw} frames, the call has {B} on {(H, W)}")
+        if window.nbytes <= 0:
+            raise ValueError("warp_batch: the crop geometry was built without a window_capacity")
         win_rect, win_off = window.rect_dev.to(device), window.off_dev.to(device)
     if out is None:
         if window is None:

@@ -297,7 +297,7 @@ size_t fusg_paste_workspace_bytes(int F, int Hf, int Wf);
  * warp_learn/models.py:337-342); the mask of item b is the uint8 array masks + mask_off[b] of shape
  * (mask_rect[4b+3], mask_rect[4b+2]) placed at frame position (x, y) = (mask_rect[4b], mask_rect[4b+1]) -- a full-frame
  * dst_sketch_mask is rect (0, 0, Wf, Hf).  Later items win where masks overlap, as in the sequential reference.
- * frames [F,Hf,Wf,3] u8 is updated in place. */
+ * frames [F,Hf,Wf,3] u8 is updated in place; an item whose frame is outside [0, F) pastes nothing. */
 int fusg_paste_back(uint8_t *frames, const uint8_t *crops, const uint8_t *masks, const long long *mask_off, const int32_t *mask_rect,
                     const int32_t *info, void *workspace, size_t workspace_bytes, int B, int F, int Hf, int Wf, int S,
                     int max_mask_pixels, void *stream);
@@ -313,10 +313,24 @@ int fusg_mask_bbox(const uint8_t *masks, const long long *mask_off, const int32_
  *                           to_tensor(resize(square_crop(normal_src))[..., ::-1]));
  * y [B,3,res,res] f32 = to_tensor(resize(square_crop(normal_dst))[..., ::-1])
  * with square_crop = utils/crop_utils.py:4-52 on bbox[b], resize = cv2.resize(..., (res, res)), background = pixels whose
- * resized source normal is (0,0,0), to_tensor = utils/misc_utils.py:35-50.  frames [F,Hf,Wf,3] u8. */
+ * resized source normal is (0,0,0), to_tensor = utils/misc_utils.py:35-50.  frames [F,Hf,Wf,3] u8.  frame_idx[b] < 0 refuses item b:
+ * its x and y rows are zero. */
 int fusg_pack_vunet_inputs(const uint8_t *frames, const int32_t *frame_idx, const uint8_t *masks, const uint8_t *normal_src,
                            const uint8_t *normal_dst, const long long *off, const int32_t *rect, const int32_t *bbox, float *x, float *y,
                            int B, int Hf, int Wf, int res, void *stream);
+/* Crop geometry of B sketch masks from their fusg_mask_bbox output, for the kernels downstream to read from device memory (one
+ * launch, no host round trip, capturable in a graph):
+ *   info [B,9]: the fusg_paste_back info of square_crop (utils/crop_utils.py:4-52) on bbox[b], frame = frame_index[b] (NULL: 0) --
+ *     frame_ops.pack_crop_info(square_crop_info(...)) bit for bit;
+ *   win [B,4] (x0, y0, w, h): the frame window the ICN packing reads for that crop (frame_ops.icn_window_rect);
+ *   win_off [B]: byte offset of item b's five [h,w,3] planes, the exclusive scan of 16-byte-aligned blocks (frame_ops.window_layout);
+ *   status [B] i8: 0 ok; 1 empty mask (bbox x_max < 0); 2 the window does not fit: its block ends past window_capacity_bytes or
+ *     it is taller than max_win_h.  Offsets only grow, so the first block past the capacity refuses itself and every later item.
+ * An item with a non-zero status gets win (0, 0, 0, 0), which fusg_warp_fused_window refuses (writing none of its bytes) and
+ * fusg_pack_icn_inputs_window packs as a zero row; an empty mask gets info (frame, 0, ..., 0).  window_capacity_bytes 0: no
+ * windows (win / win_off may be NULL; written when given); a capacity needs win, win_off and max_win_h > 0. */
+int fusg_crop_geometry(const int32_t *bbox, const int32_t *frame_index, int B, int Hf, int Wf, long long window_capacity_bytes, int max_win_h,
+                       int32_t *info, int32_t *win, long long *win_off, int8_t *status, void *stream);
 /* ---- ICN input packing (SURVEY.md section 8f-1; warp_learn/models.py:323-366 get_icn_inputs) --------------------------------
  * Item b: planes [B,5,Hf,Wf,3] u8 (the warped planes, BGR -- fusg_warp_fused's `warped` for whole frames), normals [B,Hf,Wf,3] u8
  * (destination normal sketch, RGB), central [B,res,res,3] u8 (central crop, RGB), bbox[b] = bounding box of the sketch mask
@@ -332,7 +346,7 @@ int fusg_pack_icn_inputs(const uint8_t *planes, const uint8_t *normals, const ui
 /* The same packing with the warped planes as fusg_warp_fused_window writes them: item b's five planes are the frame window
  * win[b] = (x0, y0, w, h) at planes + win_off[b] (plane k = [h,w,3] u8 at byte k*h*w*3).  The window must hold the square crop of
  * bbox[b] clipped to the Hf x Wf frame (every pixel the crop reads); then out equals fusg_pack_icn_inputs on the whole-frame planes
- * bit for bit.  Every other argument as there. */
+ * bit for bit.  Every other argument as there.  An empty window (w or h < 1, fusg_crop_geometry's refusal) gives item b a zero row. */
 int fusg_pack_icn_inputs_window(const uint8_t *planes, const int32_t *win, const long long *win_off, const uint8_t *normals,
                                 const uint8_t *central, const int32_t *bbox, const uint16_t *gamma_tab, const uint16_t *cbrt_tab,
                                 const uint32_t *exc_keys, const uint16_t *exc_vals, int n_exc, const uint32_t *exc_bitmap, float *out,

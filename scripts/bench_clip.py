@@ -13,8 +13,11 @@ renderer).
 
 --icn-window runs the ICN branch in its windowed form instead: sketches -> icn_windows -> fused warp of only each item's ICN crop
 window, reading the one source frame through src_index (no N-fold copy of the frame) -> get_icn_inputs_batch from the windows.
-The JSON line carries the SHA-1 of both generators' composited frames, so that the two forms can be compared.
-usage: python scripts/bench_clip.py [--vehicles 30] [--steps 20] [--icn-window] [--out clip.json]"""
+--device-geometry computes the crop geometry of the destination masks once, on the device (frame_ops.crop_geometry: one bbox pass, no
+host round trip), and feeds it to the ICN packing, the y_tilde packing and both paste-backs, which then run no bbox pass of their own.
+The JSON line carries the SHA-1 of both generators' composited frames, so that the forms can be compared, and the batch size of every
+fusg_mask_bbox pass of the last clip.
+usage: python scripts/bench_clip.py [--vehicles 30] [--steps 20] [--icn-window | --device-geometry] [--out clip.json]"""
 import argparse
 import hashlib
 import json
@@ -32,7 +35,8 @@ from future_urban_scene_generation_b200.warp_learn import warp_batch
 from future_urban_scene_generation_b200.warp_learn.models import G_Resnet
 from future_urban_scene_generation_b200.warp_learn.planes_utils import to_image_batch
 from future_urban_scene_generation_b200.vunet.models import Vunet_fix_res
-from future_urban_scene_generation_b200.frame_ops import get_icn_inputs_batch, icn_windows, pack_vunet_inputs_batch, paste_back_batch
+from future_urban_scene_generation_b200.frame_ops import (PastePlan, crop_geometry, get_icn_inputs_batch, icn_windows, pack_vunet_inputs_batch,
+                                                         paste_back_batch, paste_back_packed)
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--vehicles", type=int, default=30)
@@ -40,8 +44,11 @@ ap.add_argument("--steps", type=int, default=20)
 ap.add_argument("--chunk", type=int, default=100)
 ap.add_argument("--reps", type=int, default=3)
 ap.add_argument("--icn-window", action="store_true", help="warp only the ICN crop windows (see the module docstring)")
+ap.add_argument("--device-geometry", action="store_true", help="one device-side crop geometry for the whole chain (module docstring)")
 ap.add_argument("--out", default=None)
 args = ap.parse_args()
+if args.icn_window and args.device_geometry:
+    ap.error("--icn-window and --device-geometry are separate forms")
 V, S, H, W = args.vehicles, args.steps, 1080, 1920
 N = V * S
 dev = torch.device("cuda")
@@ -69,6 +76,9 @@ meshes = [MeshOnDevice(*synth.make_car_mesh(v % 10)) for v in range(V)]
 vunet = Vunet_fix_res(Namespace(up_mode='subpixel', w_norm=True, drop_prob=0.2, vunet_256=True)).cuda().eval()
 icn = G_Resnet(21).cuda().eval()
 frames_dev = torch.from_numpy(frame).to(dev)
+mask_bbox_passes = []                                                  # batch size of every fusg_mask_bbox call
+_mask_bbox = _lib.lib().fusg_mask_bbox
+_lib.lib().fusg_mask_bbox = lambda *a: (mask_bbox_passes.append(int(a[4])), _mask_bbox(*a))[1]
 yy = torch.arange(H, device=dev, dtype=torch.float32).view(1, H, 1)
 xx = torch.arange(W, device=dev, dtype=torch.float32).view(1, 1, W)
 
@@ -91,7 +101,8 @@ def normals_for(masks, seed):
 
 def clip():
     ev = {k: (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for k in
-          ("kinematics", "warp", "sketches", "icn_inputs", "icn", "vunet_inputs", "vunet", "paste") + (("icn_windows",) if args.icn_window else ())}
+          ("kinematics", "warp", "sketches", "icn_inputs", "icn", "vunet_inputs", "vunet", "paste") + (("icn_windows",) if args.icn_window else ())
+          + (("crop_geometry",) if args.device_geometry else ())}
     # 1. kinematics
     ev["kinematics"][0].record()
     poses = [kinematics.trajectory_poses(c["meter_coords"]) for c in cases]
@@ -143,10 +154,17 @@ def clip():
         windows = icn_windows(dst_masks, (H, W))
         ev["icn_windows"][1].record()
         res = warp(windows)
+    if args.device_geometry:
+        ev["crop_geometry"][0].record()
+        geom = crop_geometry(dst_masks, (H, W), frame_index=torch.as_tensor(step_of_item, device=dev).to(torch.int32))
+        ev["crop_geometry"][1].record()
     central = torch.randint(0, 256, (N, 256, 256, 3), device=dev, dtype=torch.uint8)
     # 3. ICN inputs
     ev["icn_inputs"][0].record()
-    gen_in, crop_infos = get_icn_inputs_batch(res.warped, dst_normals, dst_masks, central)
+    if args.device_geometry:
+        gen_in, _ = get_icn_inputs_batch(res.warped, dst_normals, None, central, geometry=geom)
+    else:
+        gen_in, crop_infos = get_icn_inputs_batch(res.warped, dst_normals, dst_masks, central)
     ev["icn_inputs"][1].record()
     # 4. ICN
     ev["icn"][0].record()
@@ -155,7 +173,11 @@ def clip():
     # 5. VUNet: appearance once per vehicle, shape path per item
     ev["vunet_inputs"][0].record()
     x_src, _, _ = pack_vunet_inputs_batch(frames_dev.unsqueeze(0), [0] * V, ~src_masks, src_normals, src_normals)
-    _, y_all, _ = pack_vunet_inputs_batch(frames_dev.unsqueeze(0), [0] * N, ~dst_masks, dst_normals, dst_normals)
+    if args.device_geometry:
+        _, y_all, _ = pack_vunet_inputs_batch(frames_dev.unsqueeze(0), torch.zeros(N, dtype=torch.int32, device=dev), ~dst_masks, dst_normals,
+                                              dst_normals, geometry=geom)
+    else:
+        _, y_all, _ = pack_vunet_inputs_batch(frames_dev.unsqueeze(0), [0] * N, ~dst_masks, dst_normals, dst_normals)
     ev["vunet_inputs"][1].record()
     ev["vunet"][0].record()
     with torch.no_grad():
@@ -175,6 +197,14 @@ def clip():
     ev["paste"][0].record()
     frames_icn = frames_dev.unsqueeze(0).repeat(S, 1, 1, 1)
     frames_vun = frames_icn.clone()
+    if args.device_geometry:
+        # items stay in (vehicle, step) order: inside a frame that is vehicle order, so the same item wins where masks overlap
+        plan = PastePlan.from_geometry(geom, dst_masks)
+        paste_back_packed(frames_icn, to_image_batch(icn_img, from_LAB=True), plan)
+        paste_back_packed(frames_vun, to_image_batch(vun_img), plan)
+        ev["paste"][1].record()
+        torch.cuda.synchronize()
+        return {k: a.elapsed_time(b) for k, (a, b) in ev.items()}, res, frames_icn, frames_vun
     order = np.argsort(step_of_item, kind="stable")                    # vehicles in selection order inside every frame
     infos_l = [crop_infos[i] for i in order]
     fidx = [int(step_of_item[i]) for i in order]
@@ -191,6 +221,7 @@ clip()                                                                  # warm-u
 torch.cuda.synchronize()
 runs = []
 for _ in range(args.reps):                                              # host-side glue (CPU Sampler noise, Python) varies: report the best of a few
+    mask_bbox_passes.clear()
     n0 = _lib.kernel_launches()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
@@ -202,7 +233,7 @@ runs.sort(key=lambda r: r[0])
 _, total, stages, n_launch = runs[0]
 path_ms = total
 out = {"workload": f"BASELINE config 5: {V} vehicles x {S} future steps on {W}x{H} frames, {N} (vehicle, step) items, both generators, paste-back into {S} frames each",
-       "icn_window": args.icn_window, "items": N, "ms_total": total, "ms_path": path_ms, "items_per_s": N / path_ms * 1e3, "stages_ms": stages,
+       "icn_window": args.icn_window, "device_geometry": args.device_geometry, "items": N, "mask_bbox_passes": mask_bbox_passes, "ms_total": total, "ms_path": path_ms, "items_per_s": N / path_ms * 1e3, "stages_ms": stages,
        "gpu_launches": n_launch, "reps": args.reps, "ms_path_all_reps": [r[0] for r in runs],
        "refused_items": int((res.plane_j[:, 0] == -2).sum().item()),
        "items_with_out_of_frame_keypoints": int(((dst_kp_last < 0) | (dst_kp_last >= torch.tensor([W, H], device=dev))).any(-1).any(-1).sum().item()),

@@ -1,14 +1,18 @@
 """The warp + ICN-input stages of the whole-frame trajectory chain in its two forms, on one GPU:
 
-  full      fused warp of whole frames (B x 5 x H x W x 3 planes)     -> get_icn_inputs_batch(planes)
-  windowed  icn_windows(masks) -> fused warp of the ICN crop windows  -> get_icn_inputs_batch(WindowedPlanes)
+  full          fused warp of whole frames (B x 5 x H x W x 3 planes)     -> get_icn_inputs_batch(planes)
+  windowed      icn_windows(masks) -> fused warp of the ICN crop windows  -> get_icn_inputs_batch(WindowedPlanes)
+  device        crop_geometry(masks) (no host round trip) -> the same windowed warp -> get_icn_inputs_batch(geometry=)
+  device_graph  the three stages of `device`, each captured once in a CUDA graph and replayed
+
+The window capacity of the device forms is the exact size icn_windows reports for the same masks (a caller sizes it once per graph).
 
 Items are (vehicle, future step) pairs from the trajectory kinematics as in scripts/bench_clip.py (30 vehicles x 20 steps = 600
 items), on one source frame per vehicle read through src_index in both forms, so that only the output layout differs.  The two
 forms alternate in one process for --rounds rounds each; every stage is bracketed by CUDA events.  Reported per frame size: ms per
 stage (median and all rounds), bytes of planes written (from shapes: 5*w*h*3 per item against 5*H*W*3), the peak of
 torch.cuda.max_memory_allocated over one call of each form, the share of k_plane_masks in the warp call's kernel time (torch.profiler,
-a separate pass after the timed rounds), and that gen_in is byte-identical between the forms.  The device name and power limit
+a separate pass after the timed rounds) and the kernels of one crop_geometry call (the same way), and that gen_in is byte-identical between the forms.  The device name and power limit
 come from nvidia-smi in the same run.
 usage: python scripts/bench_icn_window.py [--vehicles 30] [--steps 20] [--rounds 5] [--sizes 720x1280,1080x1920] [--out FILE]"""
 import argparse
@@ -25,7 +29,7 @@ import torch
 
 from future_urban_scene_generation_b200 import synth, kinematics
 from future_urban_scene_generation_b200.warp_learn import warp_batch
-from future_urban_scene_generation_b200.frame_ops import get_icn_inputs_batch, icn_windows
+from future_urban_scene_generation_b200.frame_ops import crop_geometry, get_icn_inputs_batch, icn_windows
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--vehicles", type=int, default=30)
@@ -85,8 +89,60 @@ def scene(H, W):
                 central=central)
 
 
-def run(sc, windowed):
+FORMS = ("full", "windowed", "device", "device_graph")
+
+
+def device_stages(sc, cap):
+    """The three stages of the device form as closures, so that they can run eagerly or be captured one by one."""
+    st = {}
+    hw = tuple(sc["frames"].shape[1:3])
+
+    def geometry():
+        st["g"] = crop_geometry(sc["masks"], hw, window_capacity=cap)
+
+    def warp():
+        st["res"] = warp_batch(sc["frames"], *sc["warp_args"], kp3d_dst=sc["moved"], src_index=sc["idx"], window=st["g"])
+
+    def pack():
+        st["gen_in"], _ = get_icn_inputs_batch(st["res"].warped, sc["normals"], None, sc["central"], geometry=st["g"])
+    return st, (("crop_geometry", geometry), ("warp", warp), ("icn_pack", pack))
+
+
+def capture_device_graph(sc, cap):
+    """One CUDA graph per stage of the device form (one memory pool); returns (state, [(stage, graph)])."""
+    st, stages = device_stages(sc, cap)
+    s = torch.cuda.Stream()
+    s.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(s):                                  # warm-up on a side stream, as torch.cuda.graphs asks
+        for _, fn in stages:
+            fn()
+    torch.cuda.current_stream().wait_stream(s)
+    torch.cuda.synchronize()
+    pool, graphs = torch.cuda.graph_pool_handle(), []
+    for name, fn in stages:
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g, pool=pool):
+            fn()
+        graphs.append((name, g))
+    torch.cuda.synchronize()
+    return st, graphs
+
+
+def run(sc, form, cap=None, graph=None):
     """One pass of the stages; returns ({stage: ms}, gen_in, the warp result)."""
+    if form in ("device", "device_graph"):
+        if form == "device":
+            st, stages = device_stages(sc, cap)
+        else:
+            st, stages = graph[0], [(n, g.replay) for n, g in graph[1]]
+        ev = {n: (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for n, _ in stages}
+        for n, fn in stages:
+            ev[n][0].record()
+            fn()
+            ev[n][1].record()
+        torch.cuda.synchronize()
+        return {k: a.elapsed_time(b) for k, (a, b) in ev.items()}, st["gen_in"], st["res"]
+    windowed = form == "windowed"
     names = ("icn_windows", "warp", "icn_pack") if windowed else ("warp", "icn_pack")
     ev = {k: (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for k in names}
     window = None
@@ -102,6 +158,24 @@ def run(sc, windowed):
     ev["icn_pack"][1].record()
     torch.cuda.synchronize()
     return {k: a.elapsed_time(b) for k, (a, b) in ev.items()}, gen_in, res
+
+
+def kernel_times(fn):
+    """Per-kernel device time (us) of the libfusg kernels one call of fn launches (torch.profiler, CUDA activities)."""
+    from torch.profiler import profile, ProfilerActivity
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    per = {}
+    for e in prof.key_averages():
+        t = getattr(e, "device_time_total", None)
+        if t is None:
+            t = e.cuda_time_total
+        if t > 0:
+            k = e.key.split("(")[0].replace("void ", "")
+            per[k] = per.get(k, 0.0) + t
+    return per
 
 
 def plane_masks_share(sc, windowed):
@@ -130,28 +204,34 @@ for hw in args.sizes.split(","):
     H, W = (int(v) for v in hw.split("x"))
     sc = scene(H, W)
     N = sc["N"]
-    # warm-up of both forms (module load, allocator, Lab tables), then one call each under a fresh memory peak
-    peaks = {}
-    for windowed in (False, True):
-        run(sc, windowed)
+    w0 = icn_windows(sc["masks"], (H, W))
+    cap = (w0.nbytes, w0.max_h)
+    # warm-up of every form (module load, allocator, Lab tables), then one call each under a fresh memory peak
+    peaks, gens = {}, {}
+    graph = None
+    for form in FORMS:
+        if form == "device_graph":
+            graph = capture_device_graph(sc, cap)
+        run(sc, form, cap, graph)
         torch.cuda.synchronize()
         torch.cuda.reset_peak_memory_stats()
         base = torch.cuda.memory_allocated()
-        _, gi, res = run(sc, windowed)
-        peaks["windowed" if windowed else "full"] = torch.cuda.max_memory_allocated() - base
-        if windowed:
+        _, gi, res = run(sc, form, cap, graph)
+        peaks[form] = torch.cuda.max_memory_allocated() - base
+        if form == "windowed":
             rect = res.warped.rect
-            gen_win = gi
-        else:
-            gen_full = gi
+        if form.startswith("device"):
+            assert int(res.warped.windows.status.abs().sum()) == 0, "the device geometry refused items"
+        gens[form] = gi.clone() if form == "device_graph" else gi
         del res
-    assert torch.equal(gen_full.view(torch.int32), gen_win.view(torch.int32)), "gen_in differs between the forms"
-    del gen_full, gen_win
-    times = {"full": [], "windowed": []}
-    for _ in range(args.rounds):                               # alternate the forms: both see the same state of the shared machine
-        for windowed in (False, True):
-            st, gi, res = run(sc, windowed)
-            times["windowed" if windowed else "full"].append(st)
+    for form in FORMS[1:]:
+        assert torch.equal(gens["full"].view(torch.int32), gens[form].view(torch.int32)), f"gen_in differs between full and {form}"
+    del gens
+    times = {f: [] for f in FORMS}
+    for _ in range(args.rounds):                               # alternate the forms: all see the same state of the shared machine
+        for form in FORMS:
+            st, gi, res = run(sc, form, cap, graph)
+            times[form].append(st)
             del gi, res
     summary = {}
     for form, rounds in times.items():
@@ -165,13 +245,16 @@ for hw in args.sizes.split(","):
         "ms": summary,
         "planes_bytes_written": {"full": bytes_full, "windowed": bytes_win, "ratio_full_over_windowed": bytes_full / bytes_win},
         "window_px": {"mean_w": float(rect[:, 2].mean()), "mean_h": float(rect[:, 3].mean()), "max_h": int(rect[:, 3].max())},
+        "window_capacity": {"bytes": cap[0], "rows": cap[1]},
         "peak_memory_bytes": {**peaks, "ratio_full_over_windowed": peaks["full"] / peaks["windowed"]},
         "k_plane_masks": {"full": plane_masks_share(sc, False), "windowed": plane_masks_share(sc, True)},
+        "crop_geometry_kernels_us": kernel_times(lambda: crop_geometry(sc["masks"], (H, W), window_capacity=cap)),
         "gen_in_identical": True})
-    del sc
+    del sc, graph
     torch.cuda.empty_cache()
 result["note"] = ("ms per stage are CUDA-event brackets around the public calls, Python glue included; icn_windows synchronises (one "
-                  "device->host copy of the bboxes); peak memory is max_memory_allocated over one call of the form above what the inputs "
+                  "device->host copy of the bboxes), crop_geometry does not; device_graph replays one captured graph per stage, "
+                  "its peak memory is what a replay allocates beyond the graphs' pool; peak memory is max_memory_allocated over one call of the form above what the inputs "
                   "already held; data: synthetic")
 print(json.dumps(result))
 if args.out:
